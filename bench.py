@@ -2,6 +2,7 @@
 """bench.py -- batched NTT throughput on N B200s (BASELINE.json metric).
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference]
+                    [--dump-outputs DIR]
 
 A "step" is one pass of the hot path over one batch of synthetic input.  Workload
 (BASELINE.json configs[1]): 65,536 independent polynomials, N=4096, 32-bit prime
@@ -28,6 +29,14 @@ Numbers on the one JSON line rank 0 prints:
 
 --impl reference times only that CPU golden (all host threads) and prints the same
 line with "impl": "reference".
+
+--dump-outputs DIR writes, after the timed steps, what the last timed step returned: a fixed,
+seeded sample of DUMP_ROWS output polynomials (whole rows, spread over the ranks) as
+DIR/ntt_out.npy (DIR/ntt_out_rank<r>.npy on several GPUs), float64 (every residue < 2^31 is
+exact), 32 MiB in all.  The inputs are seeded, so two builds run with the same arguments can
+be compared output for output.  Compare dumps of the same arm only: the GPU arm draws its
+inputs on the device (torch.Generator seeded 0x5EED0001 + rank), --impl reference with numpy
+(default_rng(0x5EED0001)), so the two arms transform different polynomials.
 """
 from __future__ import annotations
 
@@ -53,6 +62,8 @@ METRIC = "batched NTT polys/sec (N=4096, 32-bit q)"
 BYTES_PER_POLY = 8 * N                 # algorithmic: 4 B read + 4 B written per coefficient
 BFLY_PER_POLY = (N // 2) * LOGN
 FALLBACK_HBM_GBS = 6650.0              # B200_PROFILING.md fallback
+DUMP_ROWS = 1024                       # --dump-outputs: 1024 x 4096 float64 = 32 MiB
+DUMP_SEED = 0x5EED00D0
 
 
 def workload_config(polys_per_gpu: int) -> dict:
@@ -81,6 +92,18 @@ def ncu_traffic_per_launch():
             return json.load(f).get("fused_gs4096_bytes_per_launch")
     except Exception:
         return None
+
+
+def dump_rows(batch: int, world: int) -> np.ndarray:
+    """Row indices of the --dump-outputs sample on each rank (the same on every run)."""
+    k = min(batch, max(1, DUMP_ROWS // world))
+    return np.sort(np.random.default_rng(DUMP_SEED).choice(batch, k, replace=False))
+
+
+def dump_outputs(out_dir: str, rank: int, world: int, sample: np.ndarray) -> None:
+    os.makedirs(out_dir, exist_ok=True)
+    name = "ntt_out" if world == 1 else f"ntt_out_rank{rank}"
+    np.save(os.path.join(out_dir, name + ".npy"), sample.astype(np.float64))
 
 
 class ClockSampler(threading.Thread):
@@ -210,12 +233,12 @@ def run_reference(args) -> None:
     rng = np.random.default_rng(0x5EED0001)
     a = rng.integers(0, Q, (sample, N), dtype=np.int32)
     work = a.copy()
-    # ~10 core-seconds per step: bound the run to a few minutes on small hosts
+    # ~10 core-seconds per step: the warm-up is bounded to ~20 s on small hosts
     t0 = time.perf_counter()
     fn(work, roots, Q, threads)
     per_step = time.perf_counter() - t0
     warmup = max(0, min(args.warmup, int(20.0 / per_step)) - 1)
-    steps = max(1, min(args.steps, int(120.0 / per_step)))
+    steps = args.steps
     for _ in range(warmup):
         np.copyto(work, a)
         fn(work, roots, Q, threads)
@@ -225,6 +248,8 @@ def run_reference(args) -> None:
         t0 = time.perf_counter()
         fn(work, roots, Q, threads)
         total += time.perf_counter() - t0
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, 0, 1, work[dump_rows(sample, 1)])
     value = sample * steps / total
     sample_txt = (f"{sample} polys/step x {steps} timed steps of the same workload "
                   f"(N={N}, q={Q}) on {threads} host threads, g++ -O2")
@@ -234,8 +259,7 @@ def run_reference(args) -> None:
         "ms_per_step": 1e3 * total / steps, "higher_is_better": True, "scaling": "weak",
         "vs_baseline": None, "dtype": "i32", "data": "synthetic",
         "config": workload_config(sample),
-        "note": "reference's own CPU golden ntt() (src/test.cpp:34-60); host only; "
-                f"{steps} of the requested {args.steps} steps timed (bounded to ~2 minutes)",
+        "note": f"CPU golden ntt() (src/test.cpp:34-60), kind {kind}; host only",
         "butterflies_per_s": value * BFLY_PER_POLY,
         "cpu_baseline": {"value": value, "unit": "polys/s", "cores": threads, "kind": kind,
                          "sample": sample_txt},
@@ -498,6 +522,9 @@ def run_ours(args) -> None:
     per_launch_ms = [ev[k].elapsed_time(ev[k + 1]) for k in range(args.steps)]
     total_ms_max = ctx.max_over_ranks(total_ms)
     value = world * batch * args.steps / (total_ms_max * 1e-3)
+    if args.dump_outputs:                      # d_out holds the last timed step's result
+        rows = torch.from_numpy(dump_rows(batch, world)).to(d_out.device)
+        dump_outputs(args.dump_outputs, rank, world, d_out[rows].cpu().numpy())
 
     # ---- end to end through the host-buffer entry point -----------------------------
     e2e_steps = 0 if args.no_e2e else max(3, min(args.steps, 10))
@@ -606,7 +633,11 @@ def main() -> None:
     ap.add_argument("--no-e2e", action="store_true", help="profiling runs: skip the host-buffer leg")
     ap.add_argument("--no-extras", action="store_true",
                     help="skip the polymul / cfg4 / four-step blocks (profiling runs)")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write a fixed sample of the last timed step's output to DIR/*.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     if args.warmup < 3 and args.impl == "ours":
         args.warmup = 3
     if args.impl == "reference":

@@ -1,5 +1,5 @@
 import os, sys, numpy as np, torch
-sys.path.insert(0, "/root/repo")
+sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.dirname(os.path.abspath(__file__)))))
 import ntt_aie_b200 as nt
 Q, n, batch = 469762049, 1 << 16, 2100
 roots = nt.make_roots(n, Q, 3)

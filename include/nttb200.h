@@ -21,6 +21,17 @@
  *   - device entry points are asynchronous on the given CUDA stream
  *     (cudaStream_t passed as void*, NULL = default stream); in == out (in place)
  *     is allowed; host entry points are synchronous;
+ *   - alignment: every device pointer need only be 4-byte aligned (views such as
+ *     t[1:] or one channel of a batch are fine).  16-byte alignment of all of a
+ *     call's buffers selects the fast kernels; any other pointer takes the
+ *     generic kernels (the stage passes; the word loop of pointwise / scale),
+ *     with the same results.  The N = 4096 golden kernel also
+ *     runs on an output that is only 4-byte aligned (not with
+ *     NTTB200_OUTPUT_BITREV).  Exceptions: the RNS entry points and
+ *     nttb200_gs_stage_range_scatter need 16-byte-aligned buffers and return
+ *     NTTB200_ERR_UNSUPPORTED otherwise (the scatter returns
+ *     NTTB200_ERR_INVALID_ARG for an unaligned peer buffer), except for d_c of
+ *     nttb200_rns_polymul_negacyclic, which needs 4-byte alignment only;
  *   - there is NO CPU fallback: every compute entry point fails with
  *     NTTB200_ERR_CUDA / NTTB200_ERR_NO_DEVICE when no B200 is usable.
  */
@@ -58,7 +69,10 @@ typedef enum nttb200_status {
 /* plan flags */
 #define NTTB200_ORDER_GOLDEN 0u     /* output in the CPU golden's order (src/test.cpp:34-60)    */
 #define NTTB200_ORDER_AIE_DEVICE 1u /* output permuted in 16 blocks of N/16 by ans_order, as the */
-                                    /* AIE device leaves it (src/test.cpp:69-71,212-219); N>=16  */
+                                    /* AIE device leaves it (src/test.cpp:69-71,212-219); N>=16. */
+                                    /* Applies to nttb200_gs_batch / gs_host at full depth only: */
+                                    /* a partial depth, ct_batch and gs_stage_range return the   */
+                                    /* unpermuted (golden) order on such a plan.                 */
 #define NTTB200_FORCE_GENERIC 2u    /* debugging: always take the generic stage-pass kernels     */
 
 #define NTTB200_REDUCE_INPUT 4u     /* nttb200_gs_batch / ct_batch accept ANY int32 words and reduce */

@@ -224,11 +224,18 @@ int launch_generic(nttb200_plan *p, const int32_t *d_in, int32_t *d_out, size_t 
     return NTTB200_OK;
 }
 
+// The uint4 loop of pointwise/scale needs every pointer 16-byte aligned; any other
+// 4-byte-aligned views (t[1:], one RNS channel, ...) take the scalar loop only.
+static bool vec_ok(const void *x, const void *y, const void *z) {
+    return !(((uintptr_t) x | (uintptr_t) y | (uintptr_t) z) & 15u);
+}
+
 int launch_pointwise(nttb200_plan *p, const int32_t *a, const int32_t *b, int32_t *c, size_t count,
                      cudaStream_t st) {
     if (count == 0) return NTTB200_OK;
-    size_t count4 = count / 4;
-    int grid = grid_for((count4 + 255) / 256 + 1, p->sm_count, 16);
+    const bool vec = vec_ok(a, b, c);
+    size_t count4 = vec ? count / 4 : 0;
+    int grid = grid_for(((vec ? count4 : count) + 255) / 256 + 1, p->sm_count, 16);
     pointwise_kernel<<<grid, 256, 0, st>>>(reinterpret_cast<const uint32_t *>(a),
                                            reinterpret_cast<const uint32_t *>(b),
                                            reinterpret_cast<uint32_t *>(c), count4, count, p->q,
@@ -241,8 +248,9 @@ int launch_pointwise(nttb200_plan *p, const int32_t *a, const int32_t *b, int32_
 int launch_scale(nttb200_plan *p, const int32_t *a, int32_t *c, size_t count, uint32_t s,
                  uint32_t s_shoup, cudaStream_t st) {
     if (count == 0) return NTTB200_OK;
-    size_t count4 = count / 4;
-    int grid = grid_for((count4 + 255) / 256 + 1, p->sm_count, 16);
+    const bool vec = vec_ok(a, a, c);
+    size_t count4 = vec ? count / 4 : 0;
+    int grid = grid_for(((vec ? count4 : count) + 255) / 256 + 1, p->sm_count, 16);
     scale_kernel<<<grid, 256, 0, st>>>(reinterpret_cast<const uint32_t *>(a),
                                        reinterpret_cast<uint32_t *>(c), count4, count, p->q, s,
                                        s_shoup);

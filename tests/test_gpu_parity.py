@@ -70,11 +70,15 @@ def test_stage_early_exit(lib, oracle_mod):
 
 
 @pytest.mark.parametrize("name", ["n4096_q29.npz", "n4096_p3329.npz"])
-@pytest.mark.parametrize("flags", [0, 2])
-def test_n4096_fixtures(lib, name, flags):
+@pytest.mark.parametrize("flags", [0, 1, 2, 3])
+def test_n4096_fixtures(lib, oracle_mod, name, flags):
+    """flags 1: the device-order variant of the fused kernel, 3: the generic passes' permuted
+    store."""
     g = load_golden(name)
-    out, _ = run_gs(lib, g["a"], g["roots"], int(g["p"]), flags=flags)
-    assert np.array_equal(out, g["out"])
+    out, path = run_gs(lib, g["a"], g["roots"], int(g["p"]), flags=flags)
+    want = oracle_mod.ans_order_permute(g["out"]) if flags & 1 else g["out"]
+    assert np.array_equal(out, want)
+    assert path == ("generic_stage_pass" if flags & 2 else "fused_gs4096_tma"), path
 
 
 def test_small_fixtures(lib):
@@ -214,12 +218,12 @@ def test_host_buffer_entry_point(lib, oracle_mod):
     n, p = 4096, Q29
     rng = np.random.default_rng(9)
     roots = lib.make_roots(n, p, 3)
-    batch = 1500      # > one 16 MiB staging chunk (1024 polys), not a multiple
+    batch = 2100      # > one 32 MiB staging chunk (2048 polys), not a multiple
     a = rng.integers(0, p, (batch, n), dtype=np.int32)
     out = np.empty_like(a)
     with lib.Plan(12, p, roots) as plan:
         plan.gs_host(a, out, batch)
-    idx = [0, 1, 1023, 1024, 1025, batch - 1] + rng.integers(0, batch, 26).tolist()
+    idx = [0, 1, 2047, 2048, 2049, batch - 1] + rng.integers(0, batch, 26).tolist()
     assert np.array_equal(out[idx], oracle_mod.ntt_gs(a[idx], roots, p))
     # the golden-signature wrapper
     g = load_golden("default_n2048_p3329.npz")

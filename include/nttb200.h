@@ -31,7 +31,7 @@
  *     nttb200_gs_stage_range_scatter need 16-byte-aligned buffers and return
  *     NTTB200_ERR_UNSUPPORTED otherwise (the scatter returns
  *     NTTB200_ERR_INVALID_ARG for an unaligned peer buffer), except for d_c of
- *     nttb200_rns_polymul_negacyclic, which needs 4-byte alignment only;
+ *     nttb200_rns_polymul_negacyclic at N = 4096, which needs 4-byte alignment only;
  *   - there is NO CPU fallback: every compute entry point fails with
  *     NTTB200_ERR_CUDA / NTTB200_ERR_NO_DEVICE when no B200 is usable.
  */
@@ -241,22 +241,45 @@ NTTB200_API int nttb200_polymul_negacyclic(nttb200_plan *fwd, nttb200_plan *inv,
 /* ---- RNS batches (new; SURVEY 8f.1) ------------------------------------------- */
 
 /* Polynomials in residue-number-system form: L channels ("limbs") modulo L different
- * primes, N = 4096, coefficients laid out [batch][L][4096]; channel l is transformed
- * modulo q[l] with its own table tables_host[l] (4096 words, the golden's table[h+i]
- * rule).  One launch serves all channels: the kernels pick twiddles AND modulus by
- * channel.  1 <= L <= 32. */
+ * primes, N = 2^logn with 12 <= logn <= 16 (N = 4096 .. 65536), coefficients laid out
+ * [batch][L][N]: channel l of polynomial b sits at (b*L + l)*N and is transformed modulo
+ * q[l] with its own table tables_host[l] (N words, the golden's table[h+i] rule).
+ * 1 <= L <= 32, 2 <= q[l] <= 2^30 (wider moduli give NTTB200_ERR_UNSUPPORTED), flags 0.
+ * N = 4096: one launch per transform serves all channels (the kernels pick twiddles AND
+ * modulus by channel).  N > 4096: two launches per transform serve all channels, a tile
+ * pass (stages 0..11) and a column pass (stages 12..logn-1).
+ * Argument errors are returned before any device is touched: logn outside [1, 27],
+ * limbs outside [1, 32], a null pointer or flags != 0 -> NTTB200_ERR_INVALID_ARG; another
+ * logn in [1, 27] -> NTTB200_ERR_UNSUPPORTED; q[l] outside [2, 2^31) -> NTTB200_ERR_MODULUS;
+ * tables_host[l][i] outside [0, q[l]) for some i >= 1 -> NTTB200_ERR_TABLE. */
 typedef struct nttb200_rns_plan nttb200_rns_plan;
+NTTB200_API int nttb200_rns_plan_create_logn(nttb200_rns_plan **plan, int device, uint32_t logn,
+                                             uint32_t limbs, const uint32_t *q,
+                                             const int32_t *const *tables_host, uint32_t flags);
+/* nttb200_rns_plan_create_logn with logn = 12 */
 NTTB200_API int nttb200_rns_plan_create(nttb200_rns_plan **plan, int device, uint32_t limbs,
                                         const uint32_t *q, const int32_t *const *tables_host,
                                         uint32_t flags);
+/* Same plan with every channel's table GENERATED ON THE DEVICE, as
+ * nttb200_plan_create_generated(.., logn, q[l], kind, bases[l], gen_logn = logn,
+ * block_mult = 1, ..) builds it: kind = NTTB200_GEN_BITREV with bases[l] = psi_l gives the
+ * forward table of the negacyclic product, psi_l^-1 the inverse one.  Same logn, limbs, q
+ * and flags rules; kind > NTTB200_GEN_BITREV or bases == NULL -> NTTB200_ERR_INVALID_ARG,
+ * bases[l] >= q[l] -> NTTB200_ERR_TABLE. */
+NTTB200_API int nttb200_rns_plan_create_generated(nttb200_rns_plan **plan, int device, uint32_t logn,
+                                                  uint32_t limbs, const uint32_t *q, uint32_t kind,
+                                                  const uint32_t *bases, uint32_t flags);
 NTTB200_API int nttb200_rns_plan_destroy(nttb200_rns_plan *plan);
-/* golden GS network / CT network on every channel of every polynomial */
+/* golden GS network / CT network on every channel of every polynomial; N from the plan.
+ * batch * L * N / 4096 must stay below 2^31 (else NTTB200_ERR_UNSUPPORTED). */
 NTTB200_API int nttb200_rns_gs_batch(nttb200_rns_plan *plan, const int32_t *d_in, int32_t *d_out,
                                      size_t batch, void *cuda_stream);
 NTTB200_API int nttb200_rns_ct_batch(nttb200_rns_plan *plan, const int32_t *d_in, int32_t *d_out,
                                      size_t batch, void *cuda_stream);
-/* c = a (*) b mod (x^4096 + 1, q[l]) on every channel; fwd holds psi_l^bitrev tables,
- * inv psi_l^-bitrev tables of the same primes */
+/* c = a (*) b mod (x^N + 1, q[l]) on every channel; fwd holds psi_l^bitrev tables,
+ * inv psi_l^-bitrev tables of the same primes and the same N (else NTTB200_ERR_INVALID_ARG).
+ * d_c may alias d_a or d_b.  At N = 4096 d_c needs 4-byte alignment only; at N > 4096 it
+ * must be 16-byte aligned like the operands (else NTTB200_ERR_UNSUPPORTED, nothing written). */
 NTTB200_API int nttb200_rns_polymul_negacyclic(nttb200_rns_plan *fwd, nttb200_rns_plan *inv,
                                                const int32_t *d_a, const int32_t *d_b, int32_t *d_c,
                                                size_t batch, void *cuda_stream);

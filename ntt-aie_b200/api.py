@@ -77,6 +77,11 @@ def load_library():
         "nttb200_polymul_negacyclic": (ctypes.c_int, [vp, vp, vp, vp, vp, sz, vp]),
         "nttb200_rns_plan_create": (ctypes.c_int, [ctypes.POINTER(vp), ctypes.c_int, u32,
                                                    ctypes.POINTER(u32), ctypes.POINTER(_i32p), u32]),
+        "nttb200_rns_plan_create_logn": (ctypes.c_int, [ctypes.POINTER(vp), ctypes.c_int, u32, u32,
+                                                        ctypes.POINTER(u32), ctypes.POINTER(_i32p), u32]),
+        "nttb200_rns_plan_create_generated": (ctypes.c_int, [ctypes.POINTER(vp), ctypes.c_int, u32, u32,
+                                                             ctypes.POINTER(u32), u32, ctypes.POINTER(u32),
+                                                             u32]),
         "nttb200_rns_plan_destroy": (ctypes.c_int, [vp]),
         "nttb200_rns_gs_batch": (ctypes.c_int, [vp, vp, vp, sz, vp]),
         "nttb200_rns_ct_batch": (ctypes.c_int, [vp, vp, vp, sz, vp]),
@@ -104,7 +109,8 @@ EXPORTED_SYMBOLS = (
     "nttb200_gs_batch", "nttb200_ct_batch", "nttb200_gs_stage_range",
     "nttb200_gs_host", "nttb200_gs_stage_range_scatter", "nttb200_host_alloc", "nttb200_host_free",
     "nttb200_pointwise", "nttb200_scale", "nttb200_polymul_negacyclic",
-    "nttb200_rns_plan_create", "nttb200_rns_plan_destroy", "nttb200_rns_gs_batch",
+    "nttb200_rns_plan_create", "nttb200_rns_plan_create_logn", "nttb200_rns_plan_create_generated",
+    "nttb200_rns_plan_destroy", "nttb200_rns_gs_batch",
     "nttb200_rns_ct_batch", "nttb200_rns_polymul_negacyclic",
     "nttb200_strerror", "nttb200_last_error", "nttb200_kernel_launches", "nttb200_plan_last_path",
     "nttb200_plan_logn", "nttb200_plan_modulus", "nttb200_version",
@@ -314,22 +320,44 @@ class Plan:
 
 
 class RnsPlan:
-    """N = 4096 polynomials in RNS form: L channels with their own primes and tables,
-    data laid out [batch][L][4096]; one launch per transform serves all channels."""
+    """Polynomials of N = 2^logn (4096..65536) in RNS form: L channels with their own primes
+    and tables, data laid out [batch][L][N]; one launch per pass serves all channels."""
 
-    def __init__(self, qs, tables, device: int = 0):
+    def __init__(self, qs, tables, device: int = 0, logn: int = 12):
         self._lib = load_library()
         self.limbs = len(qs)
+        n = 1 << logn
         tabs = [np.ascontiguousarray(t, dtype=np.int32) for t in tables]
-        if len(tabs) != self.limbs or any(t.size != 4096 for t in tabs):
-            raise ValueError("one 4096-word table per modulus")
+        if len(tabs) != self.limbs or any(t.size != n for t in tabs):
+            raise ValueError(f"one {n}-word table per modulus")
         qarr = (ctypes.c_uint32 * self.limbs)(*[int(q) for q in qs])
         parr = (_i32p * self.limbs)(*[t.ctypes.data_as(_i32p) for t in tabs])
         handle = ctypes.c_void_p()
-        _check(self._lib.nttb200_rns_plan_create(ctypes.byref(handle), device, self.limbs, qarr, parr,
-                                                 0), "rns_plan_create")
+        _check(self._lib.nttb200_rns_plan_create_logn(ctypes.byref(handle), device, logn, self.limbs,
+                                                      qarr, parr, 0), "rns_plan_create_logn")
         self._h = handle
         self.qs = [int(q) for q in qs]
+        self.logn, self.n, self.device = logn, n, device
+
+    @classmethod
+    def generated(cls, logn: int, qs, kind: int, bases, device: int = 0) -> "RnsPlan":
+        """Plan whose channel tables are generated ON THE DEVICE: channel l's table is the
+        one Plan.generated(logn, qs[l], kind, bases[l]) builds.  kind = GEN_BITREV with
+        bases[l] = psi_l gives the forward table, psi_l^-1 the inverse one."""
+        self = cls.__new__(cls)
+        self._lib = load_library()
+        self.limbs = len(qs)
+        if len(bases) != self.limbs:
+            raise ValueError("one base per modulus")
+        qarr = (ctypes.c_uint32 * self.limbs)(*[int(q) for q in qs])
+        barr = (ctypes.c_uint32 * self.limbs)(*[int(b) for b in bases])
+        handle = ctypes.c_void_p()
+        _check(self._lib.nttb200_rns_plan_create_generated(ctypes.byref(handle), device, logn, self.limbs,
+                                                           qarr, kind, barr, 0), "rns_plan_create_generated")
+        self._h = handle
+        self.qs = [int(q) for q in qs]
+        self.logn, self.n, self.device = logn, 1 << logn, device
+        return self
 
     def close(self) -> None:
         if getattr(self, "_h", None):

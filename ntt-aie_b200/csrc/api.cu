@@ -717,34 +717,54 @@ int nttb200_polymul_negacyclic(nttb200_plan *fwd, nttb200_plan *inv, const int32
 }
 
 /* --------------------------------------------------------------------- RNS */
-int nttb200_rns_plan_create(nttb200_rns_plan **out, int device, uint32_t limbs, const uint32_t *q,
-                            const int32_t *const *tables_host, uint32_t flags) {
+}  // extern "C"
+
+// Argument checks shared by the RNS constructors, all before any device is touched.
+// `tables` (host tables) or `bases` (device-generated tables) is non-null.
+static int rns_check_args(nttb200_rns_plan **out, uint32_t logn, uint32_t limbs, const uint32_t *q,
+                          const int32_t *const *tables, const uint32_t *bases, uint32_t flags) {
     if (!out) return NTTB200_ERR_INVALID_ARG;
     *out = nullptr;
-    if (!q || !tables_host || limbs < 1 || limbs > 32 || flags != 0) return NTTB200_ERR_INVALID_ARG;
-    nttb200_rns_plan *rp = new (std::nothrow) nttb200_rns_plan();
-    if (!rp) return NTTB200_ERR_ALLOC;
-    rp->device = device;
-    rp->limbs = limbs;
-    int rc = NTTB200_OK;
-    for (uint32_t l = 0; l < limbs && rc == NTTB200_OK; l++) {
-        nttb200_plan *sp = nullptr;
-        rc = nttb200_plan_create(&sp, device, 12, q[l], tables_host[l], 0);
-        if (rc == NTTB200_OK) {
-            rp->sub.push_back(sp);
-            if (!sp->d_tw_tile) rc = NTTB200_ERR_UNSUPPORTED;
+    if (!q || (!tables && !bases) || limbs < 1 || limbs > 32 || flags != 0) return NTTB200_ERR_INVALID_ARG;
+    if (logn < 1 || logn > NTTB200_MAX_LOGN) return NTTB200_ERR_INVALID_ARG;
+    if (logn < 12 || logn > 16) return NTTB200_ERR_UNSUPPORTED;
+    if (tables) {
+        for (uint32_t l = 0; l < limbs; l++) {
+            if (!tables[l]) return NTTB200_ERR_INVALID_ARG;
         }
     }
-    if (rc == NTTB200_OK) {
-        DeviceGuard guard(device);
-        rp->sm_count = rp->sub[0]->sm_count;
-        cudaError_t e = cudaMalloc(&rp->d_tw_tile, sizeof(uint4) * kRnsTwTile * limbs);
-        if (e != cudaSuccess) rc = cuda_fail(e, "cudaMalloc(rns tables)");
-        for (uint32_t l = 0; l < limbs && rc == NTTB200_OK; l++) {
-            e = cudaMemcpy(rp->d_tw_tile + (size_t) l * kRnsTwTile, rp->sub[l]->d_tw_tile,
-                           sizeof(uint4) * kRnsTwTile, cudaMemcpyDeviceToDevice);
-            if (e != cudaSuccess) rc = cuda_fail(e, "cudaMemcpy(rns tables)");
+    // the sub-plans' own checks, for every channel before the first one reaches the device
+    for (uint32_t l = 0; l < limbs; l++) {
+        if (q[l] < 2 || q[l] > 0x7fffffffu) return NTTB200_ERR_MODULUS;
+        if (bases && bases[l] >= q[l]) return NTTB200_ERR_TABLE;
+        for (uint32_t i = 1; tables && i < (1u << logn); i++) {
+            if (tables[l][i] < 0 || (uint32_t) tables[l][i] >= q[l]) return NTTB200_ERR_TABLE;
+        }
+    }
+    return NTTB200_OK;
+}
+
+// One sub-plan per channel exists: concatenate their tile tables ([L][G][32][65]), for
+// N > 4096 their (w, w') tables ([L][N]), and derive the per-channel constants.
+static int rns_plan_finish(nttb200_rns_plan *rp) {
+    const uint32_t limbs = rp->limbs;
+    for (nttb200_plan *sp : rp->sub) {
+        if (!sp->d_tw_tile) return NTTB200_ERR_UNSUPPORTED;   // q > 2^30: no tile kernels
+    }
+    DeviceGuard guard(rp->device);
+    rp->sm_count = rp->sub[0]->sm_count;
+    const size_t tile_words = (size_t) kRnsTwTile << (rp->logn - 12), n = (size_t) 1 << rp->logn;
+    NTTB200_CUDA(cudaMalloc(&rp->d_tw_tile, sizeof(uint4) * tile_words * limbs));
+    if (rp->logn > 12) NTTB200_CUDA(cudaMalloc(&rp->d_tw, sizeof(uint2) * n * limbs));
+    try {
+        for (uint32_t l = 0; l < limbs; l++) {
             const nttb200_plan *sp = rp->sub[l];
+            NTTB200_CUDA(cudaMemcpy(rp->d_tw_tile + l * tile_words, sp->d_tw_tile, sizeof(uint4) * tile_words,
+                                    cudaMemcpyDeviceToDevice));
+            if (rp->d_tw) {
+                NTTB200_CUDA(cudaMemcpy(rp->d_tw + l * n, sp->d_tw, sizeof(uint2) * n,
+                                        cudaMemcpyDeviceToDevice));
+            }
             uint4 pc = make_uint4(sp->q, 0, 0, 0);
             if (sp->q & 1u) {
                 pc.y = inv_mod_2_32(sp->q);
@@ -754,7 +774,34 @@ int nttb200_rns_plan_create(nttb200_rns_plan **out, int device, uint32_t limbs, 
             }
             rp->pos.push_back(pc);
         }
+    } catch (...) {
+        return NTTB200_ERR_ALLOC;
     }
+    return NTTB200_OK;
+}
+
+// make_sub(l, &sp) builds channel l's sub-plan (host table or device-generated)
+template <class MakeSub>
+static int rns_plan_build(nttb200_rns_plan **out, int device, uint32_t logn, uint32_t limbs,
+                          MakeSub make_sub) {
+    DeviceRestore restore;
+    nttb200_rns_plan *rp = new (std::nothrow) nttb200_rns_plan();
+    if (!rp) return NTTB200_ERR_ALLOC;
+    rp->device = device;
+    rp->logn = logn;
+    rp->limbs = limbs;
+    int rc = NTTB200_OK;
+    try {
+        rp->sub.reserve(limbs);
+    } catch (...) {
+        rc = NTTB200_ERR_ALLOC;
+    }
+    for (uint32_t l = 0; l < limbs && rc == NTTB200_OK; l++) {
+        nttb200_plan *sp = nullptr;
+        rc = make_sub(l, &sp);
+        if (rc == NTTB200_OK) rp->sub.push_back(sp);   // capacity reserved: does not throw
+    }
+    if (rc == NTTB200_OK) rc = rns_plan_finish(rp);
     if (rc != NTTB200_OK) {
         nttb200_rns_plan_destroy(rp);
         return rc;
@@ -763,11 +810,42 @@ int nttb200_rns_plan_create(nttb200_rns_plan **out, int device, uint32_t limbs, 
     return NTTB200_OK;
 }
 
+extern "C" {
+
+int nttb200_rns_plan_create_logn(nttb200_rns_plan **out, int device, uint32_t logn, uint32_t limbs,
+                                 const uint32_t *q, const int32_t *const *tables_host, uint32_t flags) {
+    if (out) *out = nullptr;
+    if (!tables_host) return NTTB200_ERR_INVALID_ARG;
+    int rc = rns_check_args(out, logn, limbs, q, tables_host, nullptr, flags);
+    if (rc != NTTB200_OK) return rc;
+    return rns_plan_build(out, device, logn, limbs, [&](uint32_t l, nttb200_plan **sp) {
+        return nttb200_plan_create(sp, device, logn, q[l], tables_host[l], 0);
+    });
+}
+
+int nttb200_rns_plan_create(nttb200_rns_plan **out, int device, uint32_t limbs, const uint32_t *q,
+                            const int32_t *const *tables_host, uint32_t flags) {
+    return nttb200_rns_plan_create_logn(out, device, 12, limbs, q, tables_host, flags);
+}
+
+int nttb200_rns_plan_create_generated(nttb200_rns_plan **out, int device, uint32_t logn, uint32_t limbs,
+                                      const uint32_t *q, uint32_t kind, const uint32_t *bases,
+                                      uint32_t flags) {
+    if (out) *out = nullptr;
+    if (!bases || kind > NTTB200_GEN_BITREV) return NTTB200_ERR_INVALID_ARG;
+    int rc = rns_check_args(out, logn, limbs, q, nullptr, bases, flags);
+    if (rc != NTTB200_OK) return rc;
+    return rns_plan_build(out, device, logn, limbs, [&](uint32_t l, nttb200_plan **sp) {
+        return nttb200_plan_create_generated(sp, device, logn, q[l], kind, bases[l], logn, 1, 0);
+    });
+}
+
 int nttb200_rns_plan_destroy(nttb200_rns_plan *rp) {
     if (!rp) return NTTB200_OK;
     {
         DeviceGuard guard(rp->device);
         if (rp->d_tw_tile) cudaFree(rp->d_tw_tile);
+        if (rp->d_tw) cudaFree(rp->d_tw);
     }
     for (nttb200_plan *sp : rp->sub) nttb200_plan_destroy(sp);
     delete rp;
@@ -778,8 +856,7 @@ static int rns_run(nttb200_rns_plan *rp, int kind, const int32_t *d_a, const int
                    int32_t *d_out, size_t batch, void *stream) {
     if (!rp || (batch && (!d_a || !d_out))) return NTTB200_ERR_INVALID_ARG;
     DeviceGuard guard(rp->device);
-    return rns_launch(rp->sm_count, kind, rp->d_tw_tile, rp->pos.data(), rp->limbs, d_a, d_b, d_out,
-                      batch, (cudaStream_t) stream);
+    return rns_launch(rp, kind, d_a, d_b, d_out, batch, (cudaStream_t) stream);
 }
 
 int nttb200_rns_gs_batch(nttb200_rns_plan *rp, const int32_t *d_in, int32_t *d_out, size_t batch,
@@ -795,25 +872,37 @@ int nttb200_rns_ct_batch(nttb200_rns_plan *rp, const int32_t *d_in, int32_t *d_o
 int nttb200_rns_polymul_negacyclic(nttb200_rns_plan *fwd, nttb200_rns_plan *inv, const int32_t *d_a,
                                    const int32_t *d_b, int32_t *d_c, size_t batch, void *stream) {
     if (!fwd || !inv || (batch && (!d_a || !d_b || !d_c))) return NTTB200_ERR_INVALID_ARG;
-    if (fwd->limbs != inv->limbs || fwd->device != inv->device) return NTTB200_ERR_INVALID_ARG;
+    if (fwd->limbs != inv->limbs || fwd->device != inv->device || fwd->logn != inv->logn) {
+        return NTTB200_ERR_INVALID_ARG;
+    }
     for (uint32_t l = 0; l < fwd->limbs; l++) {
         if (fwd->pos[l].x != inv->pos[l].x) return NTTB200_ERR_INVALID_ARG;
         if (!(fwd->pos[l].x & 1u)) return NTTB200_ERR_MODULUS;
     }
     if (batch == 0) return NTTB200_OK;
+    // N > 4096: the output is written by the tile pass's vector stores, so it must be aligned
+    // like the operands; checked here so that nothing runs on an unaligned request
+    if (fwd->logn > 12 && (((uintptr_t) d_a | (uintptr_t) d_b | (uintptr_t) d_c) & 15u)) {
+        return NTTB200_ERR_UNSUPPORTED;
+    }
     DeviceGuard guard(fwd->device);
     cudaStream_t st = (cudaStream_t) stream;
-    // one kernel per channel: both operands enter the SM once, the product leaves once
+    // N = 4096, one kernel per channel: both operands enter the SM once, the product leaves once
     // (12 N bytes per channel product instead of 28 N through the scratch buffers below)
     static const bool one_kernel = getenv("NTTB200_RNS_POLYMUL_3KERNEL") == nullptr;
-    if (one_kernel) {
+    if (one_kernel && fwd->logn == 12) {
         int rc1 = NTTB200_OK;
         for (uint32_t l = 0; l < fwd->limbs && rc1 == NTTB200_OK; l++) {
             rc1 = launch_polymul4096_strided(fwd->sub[l], inv->sub[l], d_a, d_b, d_c, batch, fwd->limbs, l, st);
         }
         if (rc1 != NTTB200_ERR_UNSUPPORTED) return rc1;   // nothing was launched when unsupported (l == 0)
     }
-    const size_t words = batch * fwd->limbs * 4096;
+    // CT(a), CT(b) into scratch (N > 4096: column pass + tile pass each); the DUAL tile pass
+    // multiplies them at load and scales by N^-1 at the store, then the GS column pass
+    if (batch > 0xffffffffull || ((uint64_t) batch * fwd->limbs << (fwd->logn - 12)) > 0x7fffffffull) {
+        return NTTB200_ERR_UNSUPPORTED;   // the tile kernels count tiles in 31 bits
+    }
+    const size_t words = (batch * fwd->limbs) << fwd->logn;
     int32_t *tmp = nullptr;
     {
         int rca = scratch_alloc_async((void **) &tmp, sizeof(int32_t) * words * 2, st);

@@ -24,7 +24,8 @@
 //   tile_ct_kernel / tile_ct_db_kernel  the forward (Cooley-Tukey) tile pass, output through
 //                                     a TMA store; MULT fuses a pointwise product
 //   tile_gs_kernel<DUAL>              pointwise product at load + N^-1 at the store
-//   template flag RNS                 tile position = residue channel with its own modulus
+//   template mode RNS                 tile position -> residue channel with its own modulus
+//                                     (column_kernel<.., RNS>: polynomial -> channel)
 //   column_kernel<.., SCATTER>        the multi-GPU exchange as NVLink peer stores
 #include <stdlib.h>
 
@@ -34,14 +35,26 @@
 
 namespace nttb200 {
 
-// RNS: tile position c = residue-channel index, each with its own modulus:
-// pos[c] = (q_c, q_c^-1 mod 2^32, scale_c, scale_c's Shoup companion).  Passed as a kernel
+// RNS: residue channel l has its own modulus:
+// pos[l] = (q_l, q_l^-1 mod 2^32, scale_l, scale_l's Shoup companion).  Passed as a kernel
 // parameter so that the (warp-uniform) lookup is a uniform constant-bank load and the
 // modulus stays in uniform registers, as in the single-modulus kernels.
+// A tile kernel's RNS template mode says which channel tile position c belongs to:
+//   kRnsTile: c itself (N = 4096, one tile per channel);
+//   kRnsSpan: c >> log_g (N = 4096 * 2^log_g, the G tiles of a channel are adjacent positions).
+// The two are separate instantiations so that the N = 4096 kernels carry no shift.
 constexpr int kM_MaxChannels = 32;
+constexpr int kRnsOff = 0, kRnsTile = 1, kRnsSpan = 2;
 struct RnsConsts {
     uint4 pos[kM_MaxChannels];
+    uint32_t log_g;   // kRnsSpan: log2 of the tiles per channel
+    uint32_t limbs;   // column pass: polynomial P = b*L + l is channel P mod L
 };
+
+template <int RNS>
+__device__ __forceinline__ uint4 rns_channel(const RnsConsts &rns, uint32_t c) {
+    return rns.pos[RNS == kRnsSpan ? c >> rns.log_g : c];
+}
 
 // DUAL = false: plain golden stages 0..11 of every tile.
 // DUAL = true : the tile's input is the pointwise product of two buffers (second pair
@@ -55,7 +68,7 @@ struct RnsConsts {
 //     at position changes, the table of the segment's position is staged between two
 //     __syncthreads (batched large-N and RNS workloads, where a segment is long).
 // L4: 4q-lazy butterflies (q < 2^29, single modulus); the tile's output is canonical either way.
-template <bool DUAL, bool RNS, int TWMODE = 0, bool L4 = false>
+template <bool DUAL, int RNS, int TWMODE = 0, bool L4 = false>
 __global__ void __launch_bounds__(kM_Threads, 1)
 tile_gs_kernel(const __grid_constant__ CUtensorMap map_lo, const __grid_constant__ CUtensorMap map_hi,
                const __grid_constant__ CUtensorMap map_b_lo,
@@ -140,7 +153,7 @@ tile_gs_kernel(const __grid_constant__ CUtensorMap map_lo, const __grid_constant
         uint32_t v[64];
         const uint4 *tw = prm.tw_tile + (size_t) c_cur * kM_TwTile;
         if (RNS) {
-            const uint4 pc = rns.pos[c_cur];
+            const uint4 pc = rns_channel<RNS>(rns, c_cur);
             q = pc.x;
             two_q = 2u * pc.x;
             qinv = pc.y;
@@ -412,7 +425,7 @@ poly_gs_kernel(const __grid_constant__ CUtensorMap map_lo, const __grid_constant
 // STAGED (not with SMEM_TW / MULT): an 8 KiB staging slot per team takes the output in two
 // halves (see tile_ct_h_kernel below), so the tile buffer receives the prefetch of the team's next
 // tile as soon as the rows are in registers instead of after the store has drained.
-template <bool RNS, bool SMEM_TW = false, bool MULT = false, bool STAGED = false, bool L4 = false>
+template <int RNS, bool SMEM_TW = false, bool MULT = false, bool STAGED = false, bool L4 = false>
 __global__ void __launch_bounds__(kM_Threads, 1)
 tile_ct_kernel(const __grid_constant__ CUtensorMap map_lo, const __grid_constant__ CUtensorMap map_hi,
                const __grid_constant__ CUtensorMap out_lo, const __grid_constant__ CUtensorMap out_hi,
@@ -479,7 +492,7 @@ tile_ct_kernel(const __grid_constant__ CUtensorMap map_lo, const __grid_constant
         uint32_t v[64];
         const uint4 *tw = prm.tw_tile + (size_t) c_cur * kM_TwTile;
         if (RNS) {
-            const uint4 pc = rns.pos[c_cur];
+            const uint4 pc = rns_channel<RNS>(rns, c_cur);
             q = pc.x;
             two_q = 2u * pc.x;
         }
@@ -1149,13 +1162,19 @@ template <> struct VecT<1> { using type = uint32_t; };
 template <> struct VecT<2> { using type = uint2; };
 template <> struct VecT<4> { using type = uint4; };
 
-template <int K, int VC, bool CT, bool SCATTER>
+// RNS: polynomial P of the pass is b*L + l of a [batch][L][N] layout, so it runs modulo
+// q_l = rns.pos[P mod L].x with twiddles tw + l*N ([L][N] tables).  The channel is
+// warp-uniform as long as a warp stays inside one polynomial (s0 = 12: 1024 threads each).
+template <int K, int VC, bool CT, bool SCATTER, bool RNS = false>
 __global__ void __launch_bounds__(256)
 column_kernel(const uint32_t *__restrict__ in, uint32_t *__restrict__ out,
-              const uint2 *__restrict__ tw, const ColParams p, const ScatterParams sp) {
+              const uint2 *__restrict__ tw, const ColParams p, const ScatterParams sp,
+              const __grid_constant__ RnsConsts rns) {
     constexpr int R = 1 << K;
     using V = typename VecT<VC>::type;
-    const uint32_t q = p.q, two_q = 2u * p.q, zero = p.zero;
+    static_assert(!(RNS && SCATTER), "the scatter serves one single-modulus vector");
+    uint32_t q = p.q, two_q = 2u * p.q;
+    const uint32_t zero = p.zero;
     const uint32_t n = 1u << p.logn;
     const uint32_t cg_bits = p.s0 - (VC == 4 ? 2 : VC == 2 ? 1 : 0);   // column groups per row
     const uint32_t high_bits = p.logn - p.s0 - K;
@@ -1166,6 +1185,13 @@ column_kernel(const uint32_t *__restrict__ in, uint32_t *__restrict__ out,
         const uint32_t high = (uint32_t) (rest & ((1ull << high_bits) - 1));
         const uint64_t poly = rest >> high_bits;
         const size_t base = poly * n + ((size_t) high << (p.s0 + K)) + (size_t) cg * VC;
+        const uint2 *twp = tw;
+        if (RNS) {   // the host keeps batch * L below 2^31
+            const uint32_t l = (uint32_t) poly % rns.limbs;
+            q = rns.pos[l].x;
+            two_q = 2u * q;
+            twp = tw + ((size_t) l << p.logn);
+        }
         uint32_t v[R][VC];
 #pragma unroll
         for (int r = 0; r < R; r++) {
@@ -1178,7 +1204,7 @@ column_kernel(const uint32_t *__restrict__ in, uint32_t *__restrict__ out,
         for (int mm = 0; mm < K; mm++) {
             const int m = CT ? K - 1 - mm : mm;  // CT: largest stride first
             const uint32_t s = p.s0 + m;
-            const uint2 *tws = tw + (n >> (s + 1)) + ((size_t) high << (K - m - 1));
+            const uint2 *tws = twp + (n >> (s + 1)) + ((size_t) high << (K - m - 1));
 #pragma unroll
             for (int b = 0; b < (R >> (m + 1)); b++) {
                 const uint2 w = __ldg(tws + b);
@@ -1250,6 +1276,12 @@ int multi_set_attrs() {
     NTTB200_CUDA(cudaFuncSetAttribute(tile_gs_kernel<true, false, 2>, attr, kM_SmemBytesTw));
     NTTB200_CUDA(cudaFuncSetAttribute(tile_gs_kernel<false, true, 2>, attr, kM_SmemBytesTw));
     NTTB200_CUDA(cudaFuncSetAttribute(tile_gs_kernel<true, true, 2>, attr, kM_SmemBytesTw));
+    NTTB200_CUDA(cudaFuncSetAttribute(tile_gs_kernel<false, kRnsSpan>, attr, kM_SmemBytes));
+    NTTB200_CUDA(cudaFuncSetAttribute(tile_gs_kernel<true, kRnsSpan>, attr, kM_SmemBytes));
+    NTTB200_CUDA(cudaFuncSetAttribute(tile_gs_kernel<false, kRnsSpan, 2>, attr, kM_SmemBytesTw));
+    NTTB200_CUDA(cudaFuncSetAttribute(tile_gs_kernel<true, kRnsSpan, 2>, attr, kM_SmemBytesTw));
+    NTTB200_CUDA(cudaFuncSetAttribute(tile_ct_kernel<kRnsSpan>, attr, kM_SmemBytes));
+    NTTB200_CUDA(cudaFuncSetAttribute(tile_ct_kernel<kRnsSpan, false, false, true>, attr, kM_SmemBytesStaged));
     NTTB200_CUDA(cudaFuncSetAttribute(tile_gs_kernel<true, false, 1>, attr, kM_SmemBytesTw));
     NTTB200_CUDA(cudaFuncSetAttribute(tile_gs_kernel<false, false, 0, true>, attr, kM_SmemBytes));
     NTTB200_CUDA(cudaFuncSetAttribute(tile_gs_kernel<true, false, 0, true>, attr, kM_SmemBytes));
@@ -1308,28 +1340,30 @@ void multi_release(nttb200_plan *p) {
     p->d_tw_tile = nullptr;
 }
 
+// rns != nullptr: batch counts the polynomials of all channels (b*L + l), tw is [L][N]
 template <int K, int VC, bool CT>
-static int launch_column(nttb200_plan *p, const int32_t *in, int32_t *out, size_t batch, int s0,
-                         cudaStream_t st, const ScatterParams *scatter = nullptr) {
+static int launch_column(uint32_t logn, uint32_t q, const uint2 *tw, int sm_count, const int32_t *in,
+                         int32_t *out, size_t batch, int s0, cudaStream_t st,
+                         const ScatterParams *scatter = nullptr, const RnsConsts *rns = nullptr) {
     ColParams cp;
-    cp.logn = p->logn;
+    cp.logn = logn;
     cp.s0 = (uint32_t) s0;
-    cp.q = p->q;
+    cp.q = q;
     cp.zero = 0;
-    cp.threads = ((uint64_t) batch << p->logn) >> (K + (VC == 4 ? 2 : VC == 2 ? 1 : 0));
+    cp.threads = ((uint64_t) batch << logn) >> (K + (VC == 4 ? 2 : VC == 2 ? 1 : 0));
     if (cp.threads == 0) return NTTB200_OK;
     uint64_t blocks = (cp.threads + 255) / 256;
-    uint64_t cap = (uint64_t) p->sm_count * 64;
+    uint64_t cap = (uint64_t) sm_count * 64;
     int grid = (int) (blocks < cap ? blocks : cap);
-    if (scatter) {
-        column_kernel<K, VC, CT, true><<<grid, 256, 0, st>>>(reinterpret_cast<const uint32_t *>(in),
-                                                             reinterpret_cast<uint32_t *>(out),
-                                                             p->d_tw, cp, *scatter);
+    const uint32_t *src = reinterpret_cast<const uint32_t *>(in);
+    uint32_t *dst = reinterpret_cast<uint32_t *>(out);
+    ScatterParams none{};
+    if (rns) {
+        column_kernel<K, VC, CT, false, true><<<grid, 256, 0, st>>>(src, dst, tw, cp, none, *rns);
+    } else if (scatter) {
+        column_kernel<K, VC, CT, true><<<grid, 256, 0, st>>>(src, dst, tw, cp, *scatter, kNoRns);
     } else {
-        ScatterParams none{};
-        column_kernel<K, VC, CT, false><<<grid, 256, 0, st>>>(reinterpret_cast<const uint32_t *>(in),
-                                                              reinterpret_cast<uint32_t *>(out),
-                                                              p->d_tw, cp, none);
+        column_kernel<K, VC, CT, false><<<grid, 256, 0, st>>>(src, dst, tw, cp, none, kNoRns);
     }
     g_launches.fetch_add(1, std::memory_order_relaxed);
     NTTB200_CUDA(cudaGetLastError());
@@ -1342,13 +1376,33 @@ static int column_pass_t(nttb200_plan *p, const int32_t *in, int32_t *out, size_
                          int k, cudaStream_t st, const ScatterParams *sc = nullptr) {
     if (s0 < 2 || k < 1 || k > 6 || s0 + k > (int) p->logn) return NTTB200_ERR_UNSUPPORTED;
     if (((uintptr_t) in & 15u) || ((uintptr_t) out & 15u)) return NTTB200_ERR_UNSUPPORTED;
+    const uint32_t ln = p->logn, q = p->q;
+    const uint2 *tw = p->d_tw;
+    const int sm = p->sm_count;
     switch (k) {
-        case 1: return launch_column<1, 4, CT>(p, in, out, batch, s0, st, sc);
-        case 2: return launch_column<2, 4, CT>(p, in, out, batch, s0, st, sc);
-        case 3: return launch_column<3, 4, CT>(p, in, out, batch, s0, st, sc);
-        case 4: return launch_column<4, 4, CT>(p, in, out, batch, s0, st, sc);
-        case 5: return launch_column<5, 2, CT>(p, in, out, batch, s0, st, sc);
-        default: return launch_column<6, 1, CT>(p, in, out, batch, s0, st, sc);
+        case 1: return launch_column<1, 4, CT>(ln, q, tw, sm, in, out, batch, s0, st, sc);
+        case 2: return launch_column<2, 4, CT>(ln, q, tw, sm, in, out, batch, s0, st, sc);
+        case 3: return launch_column<3, 4, CT>(ln, q, tw, sm, in, out, batch, s0, st, sc);
+        case 4: return launch_column<4, 4, CT>(ln, q, tw, sm, in, out, batch, s0, st, sc);
+        case 5: return launch_column<5, 2, CT>(ln, q, tw, sm, in, out, batch, s0, st, sc);
+        default: return launch_column<6, 1, CT>(ln, q, tw, sm, in, out, batch, s0, st, sc);
+    }
+}
+
+// RNS, N = 2^13..2^16: the cross-tile stages 12..logn-1 of every channel of `polys`
+// = batch * L polynomials as one column pass of K = logn - 12 stages
+template <bool CT>
+static int rns_column_pass(const nttb200_rns_plan *rp, const RnsConsts &rc, const int32_t *in,
+                           int32_t *out, size_t polys, cudaStream_t st) {
+    const uint32_t ln = rp->logn;
+    const uint2 *tw = rp->d_tw;
+    const int sm = rp->sm_count;
+    switch (ln - 12) {
+        case 1: return launch_column<1, 4, CT>(ln, 0, tw, sm, in, out, polys, 12, st, nullptr, &rc);
+        case 2: return launch_column<2, 4, CT>(ln, 0, tw, sm, in, out, polys, 12, st, nullptr, &rc);
+        case 3: return launch_column<3, 4, CT>(ln, 0, tw, sm, in, out, polys, 12, st, nullptr, &rc);
+        case 4: return launch_column<4, 4, CT>(ln, 0, tw, sm, in, out, polys, 12, st, nullptr, &rc);
+        default: return NTTB200_ERR_UNSUPPORTED;
     }
 }
 
@@ -1760,13 +1814,47 @@ int launch_multi_ct_mul(nttb200_plan *p, const int32_t *d_in, const int32_t *d_m
 }
 
 // ------------------------------------------------------------------------- RNS
-// N = 4096, L residue channels: coefficients [batch][L][4096]; channel l is transformed
-// modulo q_l with its own table.  The tile kernels already pick their twiddles by tile
-// position; here the position is the channel and also selects the modulus.
-int rns_launch(int sm_count, int kind, const uint4 *d_tw_tile, const uint4 *h_pos, uint32_t limbs,
-               const int32_t *d_a, const int32_t *d_b, int32_t *d_out, size_t batch,
-               cudaStream_t st) {
-    const uint64_t tiles = (uint64_t) batch * limbs;
+// L residue channels: coefficients [batch][L][N]; channel l is transformed modulo q_l with
+// its own table.  The tile kernels already pick their twiddles by tile position; with
+// G = N/4096 tiles per channel, position c of the position-major order is tile c mod G of
+// channel c >> log2 G, and the concatenated [L][G][32][65] table is indexed by c as for one
+// modulus.  N > 4096 adds the cross-tile stages as one RNS column pass.
+template <int RNS>
+static void rns_tile_launch(int kind, int grid, bool seg, const CUtensorMap &a_lo, const CUtensorMap &a_hi,
+                            const CUtensorMap &b_lo, const CUtensorMap &b_hi, const TileParams &tp,
+                            const RnsConsts &rc, cudaStream_t st) {
+    if (kind == 0) {         // GS
+        if (seg) {
+            tile_gs_kernel<false, RNS, 2><<<grid, kM_Threads, kM_SmemBytesTw, st>>>(a_lo, a_hi, a_lo,
+                                                                                   a_hi, tp, rc);
+        } else {
+            tile_gs_kernel<false, RNS><<<grid, kM_Threads, kM_SmemBytes, st>>>(a_lo, a_hi, a_lo, a_hi,
+                                                                               tp, rc);
+        }
+    } else if (kind == 1) {  // CT (b_lo / b_hi: output tensor maps)
+        if (ct_staged()) {
+            tile_ct_kernel<RNS, false, false, true><<<grid, kM_Threads, kM_SmemBytesStaged, st>>>(
+                a_lo, a_hi, b_lo, b_hi, tp, rc, a_lo, a_hi);
+        } else {
+            tile_ct_kernel<RNS><<<grid, kM_Threads, kM_SmemBytes, st>>>(a_lo, a_hi, b_lo, b_hi, tp, rc, a_lo,
+                                                                        a_hi);
+        }
+    } else {                 // GS of the pointwise product, scaled
+        if (seg) {
+            tile_gs_kernel<true, RNS, 2><<<grid, kM_Threads, kM_SmemBytesTw, st>>>(a_lo, a_hi, b_lo,
+                                                                                  b_hi, tp, rc);
+        } else {
+            tile_gs_kernel<true, RNS><<<grid, kM_Threads, kM_SmemBytes, st>>>(a_lo, a_hi, b_lo, b_hi,
+                                                                              tp, rc);
+        }
+    }
+}
+
+// kind 0: GS, 1: CT, 2: GS of the pointwise product d_a (*) d_b, scaled by N^-1
+int rns_launch(const nttb200_rns_plan *rp, int kind, const int32_t *d_a, const int32_t *d_b,
+               int32_t *d_out, size_t batch, cudaStream_t st) {
+    const uint32_t limbs = rp->limbs, log_g = rp->logn - 12;
+    const uint64_t tiles = ((uint64_t) batch * limbs) << log_g;
     if (tiles == 0) return NTTB200_OK;
     if (limbs > (uint32_t) kM_MaxChannels) return NTTB200_ERR_UNSUPPORTED;
     if (tiles > 0x7fffffffull || batch > 0xffffffffull || ((uintptr_t) d_a & 15u) ||
@@ -1774,49 +1862,45 @@ int rns_launch(int sm_count, int kind, const uint4 *d_tw_tile, const uint4 *h_po
         return NTTB200_ERR_UNSUPPORTED;
     }
     RnsConsts rc{};
-    for (uint32_t l = 0; l < limbs; l++) rc.pos[l] = h_pos[l];
+    for (uint32_t l = 0; l < limbs; l++) rc.pos[l] = rp->pos[l];
+    rc.log_g = log_g;
+    rc.limbs = limbs;
     TileParams tp;
     tp.out = reinterpret_cast<uint32_t *>(d_out);
-    tp.tw_tile = d_tw_tile;
+    tp.tw_tile = rp->d_tw_tile;
     tp.batch = (uint32_t) batch;
-    tp.chunks = limbs;
+    tp.chunks = limbs << log_g;
     tp.q = 0;
     tp.zero = 0;
     tp.qinv = tp.scale = tp.scale_shoup = 0;
     tp.four_q = 0;   // RNS primes sit just below 2^30: classic butterflies
     uint64_t ctas = (tiles + kM_Teams - 1) / kM_Teams;
-    int grid = (int) (ctas < (uint64_t) sm_count ? ctas : (uint64_t) sm_count);
+    int grid = (int) (ctas < (uint64_t) rp->sm_count ? ctas : (uint64_t) rp->sm_count);
+    const size_t polys = batch * limbs;
+    // CT: the cross-tile stages (largest strides) come first, then the tile pass in place
+    const int32_t *src = d_a;
+    if (kind == 1 && log_g) {
+        int rc1 = rns_column_pass<true>(rp, rc, d_a, d_out, polys, st);
+        if (rc1 != NTTB200_OK) return rc1;
+        src = d_out;
+    }
     CUtensorMap a_lo, a_hi, b_lo, b_hi;
-    if (tile_maps(&a_lo, &a_hi, d_a, (size_t) tiles) != NTTB200_OK) return NTTB200_ERR_CUDA;
-    if (kind == 0) {         // GS
-        if (seg_tables(batch)) {
-            tile_gs_kernel<false, true, 2><<<grid, kM_Threads, kM_SmemBytesTw, st>>>(a_lo, a_hi, a_lo,
-                                                                                    a_hi, tp, rc);
-        } else {
-            tile_gs_kernel<false, true><<<grid, kM_Threads, kM_SmemBytes, st>>>(a_lo, a_hi, a_lo, a_hi,
-                                                                                tp, rc);
-        }
-    } else if (kind == 1) {  // CT (output tensor maps on d_out)
-        if (tile_maps(&b_lo, &b_hi, d_out, (size_t) tiles) != NTTB200_OK) return NTTB200_ERR_CUDA;
-        if (ct_staged()) {
-            tile_ct_kernel<true, false, false, true><<<grid, kM_Threads, kM_SmemBytesStaged, st>>>(
-                a_lo, a_hi, b_lo, b_hi, tp, rc, a_lo, a_hi);
-        } else {
-            tile_ct_kernel<true><<<grid, kM_Threads, kM_SmemBytes, st>>>(a_lo, a_hi, b_lo, b_hi, tp, rc, a_lo,
-                                                                         a_hi);
-        }
-    } else {                 // GS of the pointwise product, scaled
-        if (tile_maps(&b_lo, &b_hi, d_b, (size_t) tiles) != NTTB200_OK) return NTTB200_ERR_CUDA;
-        if (seg_tables(batch)) {
-            tile_gs_kernel<true, true, 2><<<grid, kM_Threads, kM_SmemBytesTw, st>>>(a_lo, a_hi, b_lo,
-                                                                                   b_hi, tp, rc);
-        } else {
-            tile_gs_kernel<true, true><<<grid, kM_Threads, kM_SmemBytes, st>>>(a_lo, a_hi, b_lo, b_hi,
-                                                                               tp, rc);
-        }
+    if (tile_maps(&a_lo, &a_hi, src, (size_t) tiles) != NTTB200_OK) return NTTB200_ERR_CUDA;
+    if (kind != 0 && tile_maps(&b_lo, &b_hi, kind == 1 ? d_out : d_b, (size_t) tiles) != NTTB200_OK) {
+        return NTTB200_ERR_CUDA;
+    }
+    if (kind == 0) {
+        b_lo = a_lo;
+        b_hi = a_hi;
+    }
+    if (log_g == 0) {
+        rns_tile_launch<kRnsTile>(kind, grid, seg_tables(batch), a_lo, a_hi, b_lo, b_hi, tp, rc, st);
+    } else {
+        rns_tile_launch<kRnsSpan>(kind, grid, seg_tables(batch), a_lo, a_hi, b_lo, b_hi, tp, rc, st);
     }
     g_launches.fetch_add(1, std::memory_order_relaxed);
     NTTB200_CUDA(cudaGetLastError());
+    if (kind != 1 && log_g) return rns_column_pass<false>(rp, rc, d_out, d_out, polys, st);
     return NTTB200_OK;
 }
 

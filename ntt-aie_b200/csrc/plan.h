@@ -63,13 +63,15 @@ struct nttb200_plan {
     bool host_ready = false;
 };
 
-// N = 4096, L residue channels with their own moduli and tables (SURVEY 8f.1)
+// N = 2^12..2^16, L residue channels with their own moduli and tables (SURVEY 8f.1)
 struct nttb200_rns_plan {
     int device = 0;
+    uint32_t logn = 12;
     uint32_t limbs = 0;
     int sm_count = 148;
     std::vector<nttb200_plan *> sub;   // one validated single-modulus plan per channel
-    uint4 *d_tw_tile = nullptr;        // [limbs][32][65]
+    uint4 *d_tw_tile = nullptr;        // [limbs][N/4096][32][65]
+    uint2 *d_tw = nullptr;             // [limbs][N] (w, w') of the column pass (N > 4096 only)
     std::vector<uint4> pos;            // (q, q^-1 mod 2^32, N^-1*2^32 mod q, its Shoup companion)
 };
 
@@ -172,16 +174,15 @@ int launch_column_pass(nttb200_plan *p, const int32_t *in, int32_t *out, size_t 
                        cudaStream_t st);
 int launch_gs_range_scatter(nttb200_plan *p, int32_t *d_buf, int sb, int se, void *const *peers,
                             int world, int rank, cudaStream_t st);
-int rns_launch(int sm_count, int kind, const uint4 *d_tw_tile, const uint4 *h_pos, uint32_t limbs,
-               const int32_t *d_a, const int32_t *d_b, int32_t *d_out, size_t batch,
-               cudaStream_t st);
+int rns_launch(const nttb200_rns_plan *rp, int kind, const int32_t *d_a, const int32_t *d_b,
+               int32_t *d_out, size_t batch, cudaStream_t st);
 // q^-1 mod 2^32 for odd q (Montgomery products): Newton iteration, 3 correct bits doubling per step
 inline uint32_t inv_mod_2_32(uint32_t q) {
     uint32_t x = q;
     for (int i = 0; i < 5; i++) x *= 2u - q * x;
     return x;
 }
-constexpr int kRnsTwTile = 32 * 65;  // uint4s per channel in d_tw_tile (kernels_multi.cu)
+constexpr int kRnsTwTile = 32 * 65;  // uint4s per tile position in d_tw_tile (kernels_multi.cu)
 int launch_multi_ct(nttb200_plan *p, const int32_t *d_in, int32_t *d_out, size_t batch,
                     cudaStream_t st);
 int launch_multi_ct_mul(nttb200_plan *p, const int32_t *d_in, const int32_t *d_mul, int32_t *d_out,

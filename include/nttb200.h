@@ -284,6 +284,48 @@ NTTB200_API int nttb200_rns_polymul_negacyclic(nttb200_rns_plan *fwd, nttb200_rn
                                                const int32_t *d_a, const int32_t *d_b, int32_t *d_c,
                                                size_t batch, void *cuda_stream);
 
+/* ---- RNS evaluation-domain arithmetic (new) ------------------------------------
+ * Operators on polynomials kept in the NTT domain, so that a whole computation runs as
+ * nttb200_rns_ct_batch -> (pointwise / scale / dot)* -> nttb200_rns_gs_scaled_batch on one
+ * plan, one launch per operation for all channels.  Shared rules:
+ *   - data is [batch][L][N] on the plan's L primes and N; inputs canonical (in [0, q[l])),
+ *     outputs canonical;
+ *   - argument errors are returned before anything is launched: a null plan, a null pointer
+ *     with batch > 0 or an option out of range -> NTTB200_ERR_INVALID_ARG; batch == 0 ->
+ *     NTTB200_OK with nothing launched;
+ *   - a disallowed overlap of the output with an input -> NTTB200_ERR_INVALID_ARG, a buffer that
+ *     is not 16-byte aligned -> NTTB200_ERR_UNSUPPORTED; nothing is written in either case;
+ *   - indexing is 64-bit: pointwise, scale and dot have no 2^31-word limit. */
+#define NTTB200_RNS_ADD 0u
+#define NTTB200_RNS_SUB 1u
+#define NTTB200_RNS_MUL 2u
+/* c[b][l] = a[b][l] op b'[l] mod q[l], elementwise (op: NTTB200_RNS_ADD / SUB / MUL, else
+ * INVALID_ARG); b' = d_b[b] if b_batch == batch, d_b[0] (one [L][N] operand broadcast over the
+ * batch) if b_batch == 1, another b_batch -> INVALID_ARG.  d_c may equal d_a, or d_b when
+ * b_batch == batch; any other overlap -> INVALID_ARG. */
+NTTB200_API int nttb200_rns_pointwise(nttb200_rns_plan *plan, uint32_t op, const int32_t *d_a,
+                                      const int32_t *d_b, int32_t *d_c, size_t batch, size_t b_batch,
+                                      void *cuda_stream);
+/* c[b][l] = a[b][l] * scalars[l] mod q[l]; scalars: L words on the HOST, scalars[l] < q[l]
+ * (a null scalars or a larger word -> INVALID_ARG, also for batch == 0).  In place (d_c == d_a)
+ * allowed; any other overlap -> INVALID_ARG. */
+NTTB200_API int nttb200_rns_scale(nttb200_rns_plan *plan, const int32_t *d_a, int32_t *d_c, size_t batch,
+                                  const uint32_t *scalars, void *cuda_stream);
+/* c[b][l] = (accumulate ? c[b][l] : 0) + sum_{k < terms} a[k][b][l] * w[k][b'][l] mod q[l]:
+ * the inner product of key switching.  d_a: [terms][batch][L][N]; d_w: [terms][w_batch][L][N]
+ * with w_batch == batch (b' = b) or w_batch == 1 (b' = 0: one key shared by the whole batch),
+ * another w_batch -> INVALID_ARG; 1 <= terms <= 64 (else INVALID_ARG).  The products are summed
+ * exactly in 64 bits and reduced every 16 terms.  d_c must not overlap d_a or d_w (INVALID_ARG). */
+NTTB200_API int nttb200_rns_dot(nttb200_rns_plan *plan, const int32_t *d_a, const int32_t *d_w,
+                                int32_t *d_c, uint32_t terms, size_t batch, size_t w_batch,
+                                int accumulate, void *cuda_stream);
+/* The GS network of nttb200_rns_gs_batch on every channel with every output multiplied by
+ * N^-1 mod q[l]: the inverse NTT of a plan holding psi_l^-bitrev tables, in the same passes
+ * (the scaling rides on the tile pass's store).  In place allowed.  An even q[l] (no N^-1) ->
+ * NTTB200_ERR_MODULUS; batch * L * N / 4096 must stay below 2^31 (else UNSUPPORTED). */
+NTTB200_API int nttb200_rns_gs_scaled_batch(nttb200_rns_plan *plan, const int32_t *d_in, int32_t *d_out,
+                                            size_t batch, void *cuda_stream);
+
 /* ---- introspection ---------------------------------------------------------- */
 NTTB200_API const char *nttb200_strerror(int status);
 /* text of the last CUDA error seen by the calling thread ("" if none) */

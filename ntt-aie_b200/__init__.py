@@ -15,6 +15,10 @@ from .api import (  # noqa: F401
     HostBuffer,
     RnsPlan,
     rns_polymul_negacyclic,
+    rns_dot,
+    RNS_ADD,
+    RNS_SUB,
+    RNS_MUL,
     ORDER_AIE_DEVICE,
     ORDER_GOLDEN,
     FORCE_GENERIC,

@@ -20,6 +20,9 @@ INPUT_BITREV = 8
 OUTPUT_BITREV = 16
 GEN_POWERS = 0
 GEN_BITREV = 1
+RNS_ADD = 0
+RNS_SUB = 1
+RNS_MUL = 2
 
 _lib = None
 _i32p = ctypes.POINTER(ctypes.c_int32)
@@ -86,6 +89,10 @@ def load_library():
         "nttb200_rns_gs_batch": (ctypes.c_int, [vp, vp, vp, sz, vp]),
         "nttb200_rns_ct_batch": (ctypes.c_int, [vp, vp, vp, sz, vp]),
         "nttb200_rns_polymul_negacyclic": (ctypes.c_int, [vp, vp, vp, vp, vp, sz, vp]),
+        "nttb200_rns_pointwise": (ctypes.c_int, [vp, u32, vp, vp, vp, sz, sz, vp]),
+        "nttb200_rns_scale": (ctypes.c_int, [vp, vp, vp, sz, ctypes.POINTER(u32), vp]),
+        "nttb200_rns_dot": (ctypes.c_int, [vp, vp, vp, vp, u32, sz, sz, ctypes.c_int, vp]),
+        "nttb200_rns_gs_scaled_batch": (ctypes.c_int, [vp, vp, vp, sz, vp]),
         "nttb200_strerror": (ctypes.c_char_p, [ctypes.c_int]),
         "nttb200_last_error": (ctypes.c_char_p, []),
         "nttb200_kernel_launches": (ctypes.c_uint64, []),
@@ -112,6 +119,7 @@ EXPORTED_SYMBOLS = (
     "nttb200_rns_plan_create", "nttb200_rns_plan_create_logn", "nttb200_rns_plan_create_generated",
     "nttb200_rns_plan_destroy", "nttb200_rns_gs_batch",
     "nttb200_rns_ct_batch", "nttb200_rns_polymul_negacyclic",
+    "nttb200_rns_pointwise", "nttb200_rns_scale", "nttb200_rns_dot", "nttb200_rns_gs_scaled_batch",
     "nttb200_strerror", "nttb200_last_error", "nttb200_kernel_launches", "nttb200_plan_last_path",
     "nttb200_plan_logn", "nttb200_plan_modulus", "nttb200_version",
 )
@@ -384,11 +392,42 @@ class RnsPlan:
         _check(self._lib.nttb200_rns_ct_batch(self._h, _addr(d_in), _addr(d_out), batch,
                                               _stream(stream)), "rns_ct_batch")
 
+    def gs_scaled(self, d_in, d_out, batch: int, stream=None) -> None:
+        """GS on every channel with every output times N^-1 mod q_l: the inverse NTT of a plan
+        holding psi_l^-bitrev tables."""
+        _check(self._lib.nttb200_rns_gs_scaled_batch(self._h, _addr(d_in), _addr(d_out), batch,
+                                                     _stream(stream)), "rns_gs_scaled_batch")
+
+    def pointwise(self, op: int, d_a, d_b, d_c, batch: int, b_batch: Optional[int] = None,
+                  stream=None) -> None:
+        """c = a op b per channel (op: RNS_ADD / RNS_SUB / RNS_MUL).  b_batch = 1 broadcasts one
+        [L][N] operand over the batch; None means b_batch = batch."""
+        _check(self._lib.nttb200_rns_pointwise(self._h, op, _addr(d_a), _addr(d_b), _addr(d_c), batch,
+                                               batch if b_batch is None else b_batch, _stream(stream)),
+               "rns_pointwise")
+
+    def scale(self, d_a, d_c, batch: int, scalars, stream=None) -> None:
+        """c[b][l] = a[b][l] * scalars[l] mod q_l (one host scalar per channel)."""
+        if len(scalars) != self.limbs:
+            raise ValueError("one scalar per modulus")
+        arr = (ctypes.c_uint32 * self.limbs)(*[int(s) for s in scalars])
+        _check(self._lib.nttb200_rns_scale(self._h, _addr(d_a), _addr(d_c), batch, arr, _stream(stream)),
+               "rns_scale")
+
 
 def rns_polymul_negacyclic(fwd: RnsPlan, inv: RnsPlan, d_a, d_b, d_c, batch: int, stream=None) -> None:
     _check(fwd._lib.nttb200_rns_polymul_negacyclic(fwd._h, inv._h, _addr(d_a), _addr(d_b),
                                                    _addr(d_c), batch, _stream(stream)),
            "rns_polymul_negacyclic")
+
+
+def rns_dot(plan: RnsPlan, d_a, d_w, d_c, terms: int, batch: int, w_batch: Optional[int] = None,
+            accumulate: bool = False, stream=None) -> None:
+    """c = (c if accumulate else 0) + sum_k a[k] * w[k] per channel.  d_a: [terms][batch][L][N],
+    d_w: [terms][w_batch][L][N] with w_batch = batch (None) or 1 (one key for the batch)."""
+    _check(plan._lib.nttb200_rns_dot(plan._h, _addr(d_a), _addr(d_w), _addr(d_c), terms, batch,
+                                     batch if w_batch is None else w_batch, 1 if accumulate else 0,
+                                     _stream(stream)), "rns_dot")
 
 
 def polymul_negacyclic(fwd: Plan, inv: Plan, d_a, d_b, d_c, batch: int, stream=None) -> None:

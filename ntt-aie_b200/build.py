@@ -23,7 +23,8 @@ NVCC_FLAGS = ["-O3", "-std=c++17", "-lineinfo", "-Xcompiler", "-fPIC,-fvisibilit
               "--use_fast_math", "-Xptxas", "-v"] + ARCH + os.environ.get("NTTB200_NVCC_EXTRA", "").split()
 
 SOURCES = ["api.cu", "kernels_generic.cu", "kernels_fused.cu", "kernels_multi.cu",
-           "kernels_small.cu", "tables.cu", "kernels_polymul.cu", "kernels_poly.cu", "kernels_tilecol.cu"]
+           "kernels_small.cu", "tables.cu", "kernels_polymul.cu", "kernels_poly.cu", "kernels_tilecol.cu",
+           "kernels_rns_eval.cu"]
 HEADERS = ["plan.h", "modarith.cuh", "fused_common.cuh", "tile_common.cuh", os.path.join(ROOT, "include", "nttb200.h")]
 
 

@@ -765,14 +765,16 @@ static int rns_plan_finish(nttb200_rns_plan *rp) {
                 NTTB200_CUDA(cudaMemcpy(rp->d_tw + l * n, sp->d_tw, sizeof(uint2) * n,
                                         cudaMemcpyDeviceToDevice));
             }
-            uint4 pc = make_uint4(sp->q, 0, 0, 0);
+            uint4 pc = make_uint4(sp->q, 0, 0, 0), ps = pc;
             if (sp->q & 1u) {
                 pc.y = inv_mod_2_32(sp->q);
                 uint64_t sc = ((uint64_t) sp->n_inv << 32) % sp->q;
                 pc.z = (uint32_t) sc;
                 pc.w = (uint32_t) ((sc << 32) / sp->q);
+                ps = make_uint4(sp->q, pc.y, sp->n_inv, sp->n_inv_shoup);
             }
             rp->pos.push_back(pc);
+            rp->pos_scaled.push_back(ps);
         }
     } catch (...) {
         return NTTB200_ERR_ALLOC;
@@ -914,6 +916,90 @@ int nttb200_rns_polymul_negacyclic(nttb200_rns_plan *fwd, nttb200_rns_plan *inv,
     cudaError_t e = cudaFreeAsync(tmp, st);
     if (rc == NTTB200_OK && e != cudaSuccess) rc = cuda_fail(e, "cudaFreeAsync");
     return rc;
+}
+
+int nttb200_rns_gs_scaled_batch(nttb200_rns_plan *rp, const int32_t *d_in, int32_t *d_out, size_t batch,
+                                void *stream) {
+    if (!rp || (batch && (!d_in || !d_out))) return NTTB200_ERR_INVALID_ARG;
+    for (uint32_t l = 0; l < rp->limbs; l++) {
+        if (!(rp->pos[l].x & 1u)) return NTTB200_ERR_MODULUS;   // N^-1 must exist
+    }
+    return rns_run(rp, 3, d_in, nullptr, d_out, batch, stream);
+}
+
+}  // extern "C"
+
+// Evaluation-domain operators: [lo, hi) byte ranges of the buffers, for the aliasing rules
+struct ByteRange {
+    uintptr_t lo, hi;
+    bool overlaps(const ByteRange &o) const { return lo < o.hi && o.lo < hi; }
+};
+
+static ByteRange byte_range(const void *p, uint64_t words) {
+    return {(uintptr_t) p, (uintptr_t) p + words * sizeof(int32_t)};
+}
+
+static bool aligned16(const void *a, const void *b, const void *c) {
+    return !(((uintptr_t) a | (uintptr_t) b | (uintptr_t) c) & 15u);
+}
+
+// words of `polys` polynomials of the plan, or 0 when the byte count would not fit 62 bits
+static uint64_t rns_words(const nttb200_rns_plan *rp, uint64_t polys) {
+    const uint64_t per = (uint64_t) rp->limbs << rp->logn;
+    return polys > ((uint64_t) 1 << 60) / per ? 0 : polys * per;
+}
+
+extern "C" {
+
+int nttb200_rns_pointwise(nttb200_rns_plan *rp, uint32_t op, const int32_t *d_a, const int32_t *d_b,
+                          int32_t *d_c, size_t batch, size_t b_batch, void *stream) {
+    if (!rp || (batch && (!d_a || !d_b || !d_c))) return NTTB200_ERR_INVALID_ARG;
+    if (op > NTTB200_RNS_MUL || (b_batch != batch && b_batch != 1)) return NTTB200_ERR_INVALID_ARG;
+    if (batch == 0) return NTTB200_OK;
+    const uint64_t words = rns_words(rp, batch);
+    if (!words) return NTTB200_ERR_UNSUPPORTED;
+    const bool bcast = b_batch != batch;   // b_batch == 1 < batch
+    const ByteRange a = byte_range(d_a, words), c = byte_range(d_c, words);
+    const ByteRange b = byte_range(d_b, bcast ? words / batch : words);
+    if ((c.overlaps(a) && d_c != d_a) || (c.overlaps(b) && (d_c != d_b || bcast))) {
+        return NTTB200_ERR_INVALID_ARG;
+    }
+    if (!aligned16(d_a, d_b, d_c)) return NTTB200_ERR_UNSUPPORTED;
+    DeviceGuard guard(rp->device);
+    return launch_rns_stream(rp, op, d_a, d_b, d_c, batch, bcast, nullptr, (cudaStream_t) stream);
+}
+
+int nttb200_rns_scale(nttb200_rns_plan *rp, const int32_t *d_a, int32_t *d_c, size_t batch,
+                      const uint32_t *scalars, void *stream) {
+    if (!rp || !scalars || (batch && (!d_a || !d_c))) return NTTB200_ERR_INVALID_ARG;
+    for (uint32_t l = 0; l < rp->limbs; l++) {
+        if (scalars[l] >= rp->pos[l].x) return NTTB200_ERR_INVALID_ARG;
+    }
+    if (batch == 0) return NTTB200_OK;
+    const uint64_t words = rns_words(rp, batch);
+    if (!words) return NTTB200_ERR_UNSUPPORTED;
+    if (d_c != d_a && byte_range(d_c, words).overlaps(byte_range(d_a, words))) return NTTB200_ERR_INVALID_ARG;
+    if (!aligned16(d_a, d_a, d_c)) return NTTB200_ERR_UNSUPPORTED;
+    DeviceGuard guard(rp->device);
+    return launch_rns_stream(rp, 3, d_a, nullptr, d_c, batch, false, scalars, (cudaStream_t) stream);
+}
+
+int nttb200_rns_dot(nttb200_rns_plan *rp, const int32_t *d_a, const int32_t *d_w, int32_t *d_c, uint32_t terms,
+                    size_t batch, size_t w_batch, int accumulate, void *stream) {
+    if (!rp || (batch && (!d_a || !d_w || !d_c))) return NTTB200_ERR_INVALID_ARG;
+    if (terms < 1 || terms > 64 || (w_batch != batch && w_batch != 1)) return NTTB200_ERR_INVALID_ARG;
+    if (batch == 0) return NTTB200_OK;
+    const uint64_t words = rns_words(rp, batch), a_words = rns_words(rp, (uint64_t) terms * batch);
+    if (!words || !a_words) return NTTB200_ERR_UNSUPPORTED;
+    const bool w_shared = w_batch != batch;   // w_batch == 1 < batch
+    const ByteRange c = byte_range(d_c, words);
+    if (c.overlaps(byte_range(d_a, a_words)) ||
+        c.overlaps(byte_range(d_w, w_shared ? a_words / batch : a_words))) {
+        return NTTB200_ERR_INVALID_ARG;
+    }
+    if (!aligned16(d_a, d_w, d_c)) return NTTB200_ERR_UNSUPPORTED;
+    DeviceGuard guard(rp->device);
+    return launch_rns_dot(rp, d_a, d_w, d_c, terms, batch, w_shared, accumulate != 0, (cudaStream_t) stream);
 }
 
 /* ---------------------------------------------------------- introspection */

@@ -68,7 +68,9 @@ __device__ __forceinline__ uint4 rns_channel(const RnsConsts &rns, uint32_t c) {
 //     at position changes, the table of the segment's position is staged between two
 //     __syncthreads (batched large-N and RNS workloads, where a segment is long).
 // L4: 4q-lazy butterflies (q < 2^29, single modulus); the tile's output is canonical either way.
-template <bool DUAL, int RNS, int TWMODE = 0, bool L4 = false>
+// SCALED: plain GS load, every output multiplied by `scale` (Shoup, as DUAL's store) -- with
+//   scale = N^-1 mod q the inverse NTT of a psi^-bitrev table in the same passes.
+template <bool DUAL, int RNS, int TWMODE = 0, bool L4 = false, bool SCALED = false>
 __global__ void __launch_bounds__(kM_Threads, 1)
 tile_gs_kernel(const __grid_constant__ CUtensorMap map_lo, const __grid_constant__ CUtensorMap map_hi,
                const __grid_constant__ CUtensorMap map_b_lo,
@@ -87,6 +89,7 @@ tile_gs_kernel(const __grid_constant__ CUtensorMap map_lo, const __grid_constant
     uint32_t qinv = prm.qinv, scale = prm.scale, scale_shoup = prm.scale_shoup;
     const uint32_t zero = prm.zero, four_q = prm.four_q;
     static_assert(!L4 || !RNS, "the channels of an RNS batch sit just below 2^30");
+    static_assert(!(DUAL && SCALED) && !(L4 && SCALED), "SCALED is the plain-load form of DUAL's store");
 
     const uint32_t tws = bar_base + 64;
     if (TWMODE == 1) {
@@ -238,7 +241,7 @@ tile_gs_kernel(const __grid_constant__ CUtensorMap map_lo, const __grid_constant
 #pragma unroll
         for (int i = 0; i < 64; i++) {
             uint32_t r = v[i];
-            if (DUAL) {
+            if (DUAL || SCALED) {
                 r = shoup_mul_lazy(r, scale, scale_shoup, q);   // any word in, [0, 2q) out
             } else if (L4 && !(i & 32)) {
                 r = min(r - two_q, r);                          // a sum of the last stage: below 4q
@@ -1280,6 +1283,10 @@ int multi_set_attrs() {
     NTTB200_CUDA(cudaFuncSetAttribute(tile_gs_kernel<true, kRnsSpan>, attr, kM_SmemBytes));
     NTTB200_CUDA(cudaFuncSetAttribute(tile_gs_kernel<false, kRnsSpan, 2>, attr, kM_SmemBytesTw));
     NTTB200_CUDA(cudaFuncSetAttribute(tile_gs_kernel<true, kRnsSpan, 2>, attr, kM_SmemBytesTw));
+    NTTB200_CUDA(cudaFuncSetAttribute(tile_gs_kernel<false, kRnsTile, 0, false, true>, attr, kM_SmemBytes));
+    NTTB200_CUDA(cudaFuncSetAttribute(tile_gs_kernel<false, kRnsSpan, 0, false, true>, attr, kM_SmemBytes));
+    NTTB200_CUDA(cudaFuncSetAttribute(tile_gs_kernel<false, kRnsTile, 2, false, true>, attr, kM_SmemBytesTw));
+    NTTB200_CUDA(cudaFuncSetAttribute(tile_gs_kernel<false, kRnsSpan, 2, false, true>, attr, kM_SmemBytesTw));
     NTTB200_CUDA(cudaFuncSetAttribute(tile_ct_kernel<kRnsSpan>, attr, kM_SmemBytes));
     NTTB200_CUDA(cudaFuncSetAttribute(tile_ct_kernel<kRnsSpan, false, false, true>, attr, kM_SmemBytesStaged));
     NTTB200_CUDA(cudaFuncSetAttribute(tile_gs_kernel<true, false, 1>, attr, kM_SmemBytesTw));
@@ -1839,7 +1846,7 @@ static void rns_tile_launch(int kind, int grid, bool seg, const CUtensorMap &a_l
             tile_ct_kernel<RNS><<<grid, kM_Threads, kM_SmemBytes, st>>>(a_lo, a_hi, b_lo, b_hi, tp, rc, a_lo,
                                                                         a_hi);
         }
-    } else {                 // GS of the pointwise product, scaled
+    } else if (kind == 2) {  // GS of the pointwise product, scaled
         if (seg) {
             tile_gs_kernel<true, RNS, 2><<<grid, kM_Threads, kM_SmemBytesTw, st>>>(a_lo, a_hi, b_lo,
                                                                                   b_hi, tp, rc);
@@ -1847,10 +1854,19 @@ static void rns_tile_launch(int kind, int grid, bool seg, const CUtensorMap &a_l
             tile_gs_kernel<true, RNS><<<grid, kM_Threads, kM_SmemBytes, st>>>(a_lo, a_hi, b_lo, b_hi,
                                                                               tp, rc);
         }
+    } else {                 // GS, every output times N^-1
+        if (seg) {
+            tile_gs_kernel<false, RNS, 2, false, true><<<grid, kM_Threads, kM_SmemBytesTw, st>>>(
+                a_lo, a_hi, a_lo, a_hi, tp, rc);
+        } else {
+            tile_gs_kernel<false, RNS, 0, false, true><<<grid, kM_Threads, kM_SmemBytes, st>>>(
+                a_lo, a_hi, a_lo, a_hi, tp, rc);
+        }
     }
 }
 
-// kind 0: GS, 1: CT, 2: GS of the pointwise product d_a (*) d_b, scaled by N^-1
+// kind 0: GS, 1: CT, 2: GS of the pointwise product d_a (*) d_b, scaled by N^-1,
+// 3: GS scaled by N^-1
 int rns_launch(const nttb200_rns_plan *rp, int kind, const int32_t *d_a, const int32_t *d_b,
                int32_t *d_out, size_t batch, cudaStream_t st) {
     const uint32_t limbs = rp->limbs, log_g = rp->logn - 12;
@@ -1862,7 +1878,7 @@ int rns_launch(const nttb200_rns_plan *rp, int kind, const int32_t *d_a, const i
         return NTTB200_ERR_UNSUPPORTED;
     }
     RnsConsts rc{};
-    for (uint32_t l = 0; l < limbs; l++) rc.pos[l] = rp->pos[l];
+    for (uint32_t l = 0; l < limbs; l++) rc.pos[l] = kind == 3 ? rp->pos_scaled[l] : rp->pos[l];
     rc.log_g = log_g;
     rc.limbs = limbs;
     TileParams tp;
@@ -1886,10 +1902,11 @@ int rns_launch(const nttb200_rns_plan *rp, int kind, const int32_t *d_a, const i
     }
     CUtensorMap a_lo, a_hi, b_lo, b_hi;
     if (tile_maps(&a_lo, &a_hi, src, (size_t) tiles) != NTTB200_OK) return NTTB200_ERR_CUDA;
-    if (kind != 0 && tile_maps(&b_lo, &b_hi, kind == 1 ? d_out : d_b, (size_t) tiles) != NTTB200_OK) {
+    if ((kind == 1 || kind == 2) &&
+        tile_maps(&b_lo, &b_hi, kind == 1 ? d_out : d_b, (size_t) tiles) != NTTB200_OK) {
         return NTTB200_ERR_CUDA;
     }
-    if (kind == 0) {
+    if (kind == 0 || kind == 3) {
         b_lo = a_lo;
         b_hi = a_hi;
     }

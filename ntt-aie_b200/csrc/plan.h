@@ -73,6 +73,7 @@ struct nttb200_rns_plan {
     uint4 *d_tw_tile = nullptr;        // [limbs][N/4096][32][65]
     uint2 *d_tw = nullptr;             // [limbs][N] (w, w') of the column pass (N > 4096 only)
     std::vector<uint4> pos;            // (q, q^-1 mod 2^32, N^-1*2^32 mod q, its Shoup companion)
+    std::vector<uint4> pos_scaled;     // (q, q^-1 mod 2^32, N^-1 mod q, its Shoup companion)
 };
 
 namespace nttb200 {
@@ -176,6 +177,12 @@ int launch_gs_range_scatter(nttb200_plan *p, int32_t *d_buf, int sb, int se, voi
                             int world, int rank, cudaStream_t st);
 int rns_launch(const nttb200_rns_plan *rp, int kind, const int32_t *d_a, const int32_t *d_b,
                int32_t *d_out, size_t batch, cudaStream_t st);
+// evaluation-domain operators on RNS batches (kernels_rns_eval.cu); the caller has checked the
+// arguments, the aliasing and the 16-byte alignment
+int launch_rns_stream(const nttb200_rns_plan *rp, uint32_t op, const int32_t *a, const int32_t *b, int32_t *c,
+                      size_t batch, bool bcast, const uint32_t *scalars, cudaStream_t st);
+int launch_rns_dot(const nttb200_rns_plan *rp, const int32_t *a, const int32_t *w, int32_t *c, uint32_t terms,
+                   size_t batch, bool w_shared, bool accumulate, cudaStream_t st);
 // q^-1 mod 2^32 for odd q (Montgomery products): Newton iteration, 3 correct bits doubling per step
 inline uint32_t inv_mod_2_32(uint32_t q) {
     uint32_t x = q;

@@ -326,6 +326,59 @@ NTTB200_API int nttb200_rns_dot(nttb200_rns_plan *plan, const int32_t *d_a, cons
 NTTB200_API int nttb200_rns_gs_scaled_batch(nttb200_rns_plan *plan, const int32_t *d_in, int32_t *d_out,
                                             size_t batch, void *cuda_stream);
 
+/* ---- RNS basis conversion (new) -------------------------------------------------
+ * Moves coefficient-domain values from the primes of one plan to those of another: the step
+ * under CKKS rescale, the BGV-style modulus drop and the ModUp / ModDown of hybrid key
+ * switching.  A conversion object is built from a source plan `from` (S channels, moduli b_i,
+ * product B) and a target plan `to` (T channels, moduli c_j, product C).
+ * nttb200_rns_conv_create: both plans on the same device with the same logn, flags 0 (else, or
+ * a null pointer, NTTB200_ERR_INVALID_ARG); the S + T moduli pairwise coprime (else
+ * NTTB200_ERR_MODULUS; the moduli need not be prime).  These are checked before any device is
+ * touched.  The object copies the moduli, N, the device and every constant it needs: the plans
+ * may be destroyed after this call.
+ * Shared rules of the two operations (those of the evaluation-domain operators): inputs
+ * canonical, outputs canonical; a null conv, a null pointer with batch > 0, an unknown flag or
+ * a bad stride -> NTTB200_ERR_INVALID_ARG; batch == 0 -> NTTB200_OK with nothing launched; a
+ * disallowed overlap of output and input -> NTTB200_ERR_INVALID_ARG; a buffer that is not
+ * 16-byte aligned -> NTTB200_ERR_UNSUPPORTED (nothing is written in either case); indexing is
+ * 64-bit, with no 2^31-word limit. */
+typedef struct nttb200_rns_conv nttb200_rns_conv;
+NTTB200_API int nttb200_rns_conv_create(nttb200_rns_conv **conv, const nttb200_rns_plan *from,
+                                        const nttb200_rns_plan *to, uint32_t flags);
+NTTB200_API int nttb200_rns_conv_destroy(nttb200_rns_conv *conv);
+
+/* Fast (approximate) base conversion, coefficient domain, for ModUp:
+ *   out[b][j] = sum_i [in[b][i] * (B/b_i)^-1]_{b_i} * (B/b_i)  mod c_j.
+ * Contract: with x in [0, B) the CRT value of the S input residues and y_i the bracket above,
+ * sum_i y_i * (B/b_i) = x + alpha*B with 0 <= alpha < S, and out[b][j] is that sum mod c_j
+ * (exact, alpha = 0, when S = 1).  in_stride / out_stride: words between consecutive
+ * polynomials; 0 means dense (S*N, T*N), otherwise a multiple of N and at least S*N (T*N), else
+ * INVALID_ARG.  So a digit (a channel range of a [batch][L][N] ciphertext) can be read, and the
+ * result written into the P channels of a [batch][L+K][N] buffer, without copies.  The output
+ * must not share a word with any input row (INVALID_ARG): with equal strides the views are
+ * compared row by row, so the P channels of the buffer whose Q channels are read may be
+ * written; with different strides the whole extents must be disjoint. */
+NTTB200_API int nttb200_rns_base_convert(nttb200_rns_conv *conv, const int32_t *d_in, size_t in_stride,
+                                         int32_t *d_out, size_t out_stride, size_t batch,
+                                         void *cuda_stream);
+
+/* Division by B with the source channels dropped, for rescale / modulus drop and ModDown.
+ * d_in: [batch][T+S][N], the T target channels first, then the S source channels;
+ * d_out: [batch][T][N]:
+ *   out[b][j] = ((x_C,j + h_C,j) - sum_i y'_i * (B/b_i)) * B^-1  mod c_j,
+ *   y'_i = (x_B,i + h_B,i) * (B/b_i)^-1  mod b_i,
+ * h = floor(B/2) with NTTB200_RNS_ROUND, h = 0 without (other flags -> INVALID_ARG).
+ * Contract: with X in [0, C*B) the CRT value of all T + S input channels and X' = (X + h) mod CB,
+ * out = (floor(X'/B) - alpha) mod c_j with alpha in [0, S) the overshoot of converting X' mod B.
+ * With S = 1, alpha = 0 and the result is exact: floor((X + floor(B/2))/B) = round(X/B) for
+ * X < CB - floor(B/2) with ROUND, floor(X/B) without.  from = {q_L-1}, to = {q_0..q_L-2}: the
+ * natural [batch][L][N] ciphertext is the input (CKKS rescale); from = P, to = Q: ModDown of a
+ * [batch][L+K][N] key-switching result.  The output must not overlap the input (INVALID_ARG;
+ * in place is not possible: at batch > 1 output row b lands on input row b-1's source channels). */
+#define NTTB200_RNS_ROUND 1u
+NTTB200_API int nttb200_rns_mod_down(nttb200_rns_conv *conv, const int32_t *d_in, int32_t *d_out,
+                                     size_t batch, uint32_t flags, void *cuda_stream);
+
 /* ---- introspection ---------------------------------------------------------- */
 NTTB200_API const char *nttb200_strerror(int status);
 /* text of the last CUDA error seen by the calling thread ("" if none) */

@@ -14,11 +14,13 @@ from .api import (  # noqa: F401
     Plan,
     HostBuffer,
     RnsPlan,
+    RnsConv,
     rns_polymul_negacyclic,
     rns_dot,
     RNS_ADD,
     RNS_SUB,
     RNS_MUL,
+    RNS_ROUND,
     ORDER_AIE_DEVICE,
     ORDER_GOLDEN,
     FORCE_GENERIC,

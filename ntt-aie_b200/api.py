@@ -23,6 +23,7 @@ GEN_BITREV = 1
 RNS_ADD = 0
 RNS_SUB = 1
 RNS_MUL = 2
+RNS_ROUND = 1
 
 _lib = None
 _i32p = ctypes.POINTER(ctypes.c_int32)
@@ -93,6 +94,10 @@ def load_library():
         "nttb200_rns_scale": (ctypes.c_int, [vp, vp, vp, sz, ctypes.POINTER(u32), vp]),
         "nttb200_rns_dot": (ctypes.c_int, [vp, vp, vp, vp, u32, sz, sz, ctypes.c_int, vp]),
         "nttb200_rns_gs_scaled_batch": (ctypes.c_int, [vp, vp, vp, sz, vp]),
+        "nttb200_rns_conv_create": (ctypes.c_int, [ctypes.POINTER(vp), vp, vp, u32]),
+        "nttb200_rns_conv_destroy": (ctypes.c_int, [vp]),
+        "nttb200_rns_base_convert": (ctypes.c_int, [vp, vp, sz, vp, sz, sz, vp]),
+        "nttb200_rns_mod_down": (ctypes.c_int, [vp, vp, vp, sz, u32, vp]),
         "nttb200_strerror": (ctypes.c_char_p, [ctypes.c_int]),
         "nttb200_last_error": (ctypes.c_char_p, []),
         "nttb200_kernel_launches": (ctypes.c_uint64, []),
@@ -120,6 +125,7 @@ EXPORTED_SYMBOLS = (
     "nttb200_rns_plan_destroy", "nttb200_rns_gs_batch",
     "nttb200_rns_ct_batch", "nttb200_rns_polymul_negacyclic",
     "nttb200_rns_pointwise", "nttb200_rns_scale", "nttb200_rns_dot", "nttb200_rns_gs_scaled_batch",
+    "nttb200_rns_conv_create", "nttb200_rns_conv_destroy", "nttb200_rns_base_convert", "nttb200_rns_mod_down",
     "nttb200_strerror", "nttb200_last_error", "nttb200_kernel_launches", "nttb200_plan_last_path",
     "nttb200_plan_logn", "nttb200_plan_modulus", "nttb200_version",
 )
@@ -413,6 +419,50 @@ class RnsPlan:
         arr = (ctypes.c_uint32 * self.limbs)(*[int(s) for s in scalars])
         _check(self._lib.nttb200_rns_scale(self._h, _addr(d_a), _addr(d_c), batch, arr, _stream(stream)),
                "rns_scale")
+
+
+class RnsConv:
+    """Basis conversion from the primes of `src` (S channels, product B) to those of `dst`
+    (T channels), coefficient domain.  The object copies what it needs: the plans may be closed
+    afterwards.  See nttb200_rns_conv_create for the rules."""
+
+    def __init__(self, src: RnsPlan, dst: RnsPlan):
+        self._lib = load_library()
+        handle = ctypes.c_void_p()
+        _check(self._lib.nttb200_rns_conv_create(ctypes.byref(handle), src._h, dst._h, 0), "rns_conv_create")
+        self._h = handle
+        self.src_qs, self.dst_qs = list(src.qs), list(dst.qs)
+        self.logn, self.n = src.logn, src.n
+
+    def close(self) -> None:
+        if getattr(self, "_h", None):
+            self._lib.nttb200_rns_conv_destroy(self._h)
+            self._h = None
+
+    def __del__(self):
+        try:
+            self.close()
+        except Exception:
+            pass
+
+    def __enter__(self):
+        return self
+
+    def __exit__(self, *exc):
+        self.close()
+
+    def convert(self, d_in, d_out, batch: int, in_stride: int = 0, out_stride: int = 0, stream=None) -> None:
+        """Fast base conversion (ModUp): out[b][j] = sum_i [in[b][i] (B/b_i)^-1]_{b_i} (B/b_i) mod c_j,
+        i.e. (x + alpha B) mod c_j with 0 <= alpha < S.  Strides in words between polynomials
+        (0: dense S*N / T*N)."""
+        _check(self._lib.nttb200_rns_base_convert(self._h, _addr(d_in), in_stride, _addr(d_out), out_stride,
+                                                  batch, _stream(stream)), "rns_base_convert")
+
+    def mod_down(self, d_in, d_out, batch: int, round: bool = False, stream=None) -> None:
+        """Divide by B and drop the source channels: d_in [batch][T+S][N] (target channels
+        first), d_out [batch][T][N]; floor((X + (floor(B/2) if round else 0)) / B) - alpha."""
+        _check(self._lib.nttb200_rns_mod_down(self._h, _addr(d_in), _addr(d_out), batch,
+                                              RNS_ROUND if round else 0, _stream(stream)), "rns_mod_down")
 
 
 def rns_polymul_negacyclic(fwd: RnsPlan, inv: RnsPlan, d_a, d_b, d_c, batch: int, stream=None) -> None:

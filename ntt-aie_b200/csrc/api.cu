@@ -1002,6 +1002,95 @@ int nttb200_rns_dot(nttb200_rns_plan *rp, const int32_t *d_a, const int32_t *d_w
     return launch_rns_dot(rp, d_a, d_w, d_c, terms, batch, w_shared, accumulate != 0, (cudaStream_t) stream);
 }
 
+/* ------------------------------------------------------- RNS basis conversion */
+int nttb200_rns_conv_create(nttb200_rns_conv **conv, const nttb200_rns_plan *from, const nttb200_rns_plan *to,
+                            uint32_t flags) {
+    if (!conv) return NTTB200_ERR_INVALID_ARG;
+    *conv = nullptr;
+    if (!from || !to || flags != 0) return NTTB200_ERR_INVALID_ARG;
+    if (from->device != to->device || from->logn != to->logn) return NTTB200_ERR_INVALID_ARG;
+    nttb200_rns_conv *cv = new (std::nothrow) nttb200_rns_conv();
+    if (!cv) return NTTB200_ERR_ALLOC;
+    cv->device = from->device;
+    cv->logn = from->logn;
+    cv->src = from->limbs;
+    cv->dst = to->limbs;
+    cv->sm_count = from->sm_count;
+    uint32_t b[kConvMaxChannels], c[kConvMaxChannels];
+    for (uint32_t i = 0; i < cv->src; i++) b[i] = from->pos[i].x;
+    for (uint32_t j = 0; j < cv->dst; j++) c[j] = to->pos[j].x;
+    int rc;
+    try {
+        rc = rns_conv_prepare(cv, b, c);
+    } catch (...) {
+        rc = NTTB200_ERR_ALLOC;
+    }
+    if (rc != NTTB200_OK) {
+        delete cv;
+        return rc;
+    }
+    *conv = cv;
+    return NTTB200_OK;
+}
+
+int nttb200_rns_conv_destroy(nttb200_rns_conv *conv) {
+    delete conv;
+    return NTTB200_OK;
+}
+
+}  // extern "C"
+
+// Word offsets of the rows of an equal-stride pair of views overlap: input row b holds
+// [I + b P, I + b P + SA), output row b' holds [O + b' P, O + b' P + TA) (bytes, P > 0, every
+// row shorter than P).  They share a byte iff some k = b' - b in (-batch, batch) has
+// I - O - TA < k P < I - O + SA.
+static bool rows_overlap(uintptr_t in, uint64_t sa, uintptr_t out, uint64_t ta, uint64_t period, uint64_t batch) {
+    const int64_t d = (int64_t) (in - out), p = (int64_t) period, lo = d - (int64_t) ta;
+    int64_t k = (lo >= 0 ? lo / p : -((-lo + p - 1) / p)) + 1;   // floor(lo / p) + 1: least k with k P > lo
+    if (k < 1 - (int64_t) batch) k = 1 - (int64_t) batch;
+    return k <= (int64_t) batch - 1 && k * p < d + (int64_t) sa;
+}
+
+extern "C" {
+
+int nttb200_rns_base_convert(nttb200_rns_conv *conv, const int32_t *d_in, size_t in_stride, int32_t *d_out,
+                             size_t out_stride, size_t batch, void *stream) {
+    if (!conv || (batch && (!d_in || !d_out))) return NTTB200_ERR_INVALID_ARG;
+    const uint64_t n = (uint64_t) 1 << conv->logn;
+    const uint64_t s_words = conv->src * n, t_words = conv->dst * n;
+    const uint64_t is = in_stride ? in_stride : s_words, os = out_stride ? out_stride : t_words;
+    if (is % n || is < s_words || os % n || os < t_words) return NTTB200_ERR_INVALID_ARG;
+    if (batch == 0) return NTTB200_OK;
+    // extents, or 0 when the byte count would not fit 62 bits
+    const uint64_t lim = (uint64_t) 1 << 60;
+    if (is > lim || os > lim || batch - 1 > (lim - s_words) / is || batch - 1 > (lim - t_words) / os) {
+        return NTTB200_ERR_UNSUPPORTED;
+    }
+    const uintptr_t in = (uintptr_t) d_in, out = (uintptr_t) d_out;
+    const bool overlap = is == os ? rows_overlap(in, 4 * s_words, out, 4 * t_words, 4 * is, batch)
+                                  : byte_range(d_in, (batch - 1) * is + s_words)
+                                        .overlaps(byte_range(d_out, (batch - 1) * os + t_words));
+    if (overlap) return NTTB200_ERR_INVALID_ARG;
+    if (!aligned16(d_in, d_in, d_out)) return NTTB200_ERR_UNSUPPORTED;
+    DeviceGuard guard(conv->device);
+    return launch_rns_conv(conv, d_in, nullptr, is, d_out, os, batch, false, false, (cudaStream_t) stream);
+}
+
+int nttb200_rns_mod_down(nttb200_rns_conv *conv, const int32_t *d_in, int32_t *d_out, size_t batch, uint32_t flags,
+                         void *stream) {
+    if (!conv || (batch && (!d_in || !d_out))) return NTTB200_ERR_INVALID_ARG;
+    if (flags & ~NTTB200_RNS_ROUND) return NTTB200_ERR_INVALID_ARG;
+    if (batch == 0) return NTTB200_OK;
+    const uint64_t n = (uint64_t) 1 << conv->logn;
+    const uint64_t row = (conv->src + conv->dst) * n, t_words = conv->dst * n;
+    if (batch > ((uint64_t) 1 << 60) / row) return NTTB200_ERR_UNSUPPORTED;
+    if (byte_range(d_in, batch * row).overlaps(byte_range(d_out, batch * t_words))) return NTTB200_ERR_INVALID_ARG;
+    if (!aligned16(d_in, d_in, d_out)) return NTTB200_ERR_UNSUPPORTED;
+    DeviceGuard guard(conv->device);
+    return launch_rns_conv(conv, d_in + t_words, d_in, row, d_out, t_words, batch, true,
+                           (flags & NTTB200_RNS_ROUND) != 0, (cudaStream_t) stream);
+}
+
 /* ---------------------------------------------------------- introspection */
 const char *nttb200_strerror(int status) {
     switch (status) {

@@ -38,14 +38,6 @@ struct RnsEvalConsts {
     uint32_t sp[kE_MaxChannels];
 };
 
-// t mod q for any t < 2^64, q <= 2^30, mu = floor(2^64 / q):
-// t/q - 1 < t*mu/2^64 <= t/q, so qhat = floor(t*mu/2^64) is floor(t/q) or one less and the
-// remainder t - qhat*q lies in [0, 2q) (computed mod 2^32, where it fits).
-__device__ __forceinline__ uint32_t reduce64(uint64_t t, uint32_t q, uint64_t mu) {
-    const uint64_t qhat = __umul64hi(t, mu);
-    return csub((uint32_t) t - (uint32_t) qhat * q, q);
-}
-
 template <int OP>
 __device__ __forceinline__ uint32_t stream_op(uint32_t a, uint32_t b, uint32_t q, uint64_t mu, uint32_t s,
                                               uint32_t sp) {

@@ -41,6 +41,14 @@ __device__ __forceinline__ uint32_t shoup_mul(uint32_t x, uint32_t w, uint32_t w
     return csub(shoup_mul_lazy(x, w, wp, q), q);
 }
 
+// t mod q for any t < 2^64, q <= 2^30, mu = floor(2^64 / q):
+// t/q - 1 < t*mu/2^64 <= t/q, so qhat = floor(t*mu/2^64) is floor(t/q) or one less and the
+// remainder t - qhat*q lies in [0, 2q) (computed mod 2^32, where it fits).
+__device__ __forceinline__ uint32_t reduce64(uint64_t t, uint32_t q, uint64_t mu) {
+    const uint64_t qhat = __umul64hi(t, mu);
+    return csub((uint32_t) t - (uint32_t) qhat * q, q);
+}
+
 // General a*b mod q for two data operands (pointwise product): 64-bit product
 // and a Barrett quotient estimate.  mu = floor(2^62 / q); for a,b < q <= 2^30 the
 // product t < 2^60 and qhat = floor(t*mu / 2^62) is floor(t/q) or one less, so

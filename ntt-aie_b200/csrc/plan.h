@@ -78,6 +78,37 @@ struct nttb200_rns_plan {
 
 namespace nttb200 {
 
+constexpr int kConvMaxChannels = 32;
+
+// Constants of one basis conversion (source moduli b_i, product B; target moduli c_j), passed
+// to the kernel as one __grid_constant__ parameter block (5376 bytes).
+struct RnsConvConsts {
+    uint32_t m[kConvMaxChannels][kConvMaxChannels];   // [j][i] = (B / b_i) mod c_j
+    uint64_t mu[kConvMaxChannels];     // floor(2^64 / c_j) for reduce64
+    uint32_t c[kConvMaxChannels];      // c_j
+    uint32_t hc[kConvMaxChannels];     // floor(B/2) mod c_j (0 when not rounding)
+    uint32_t binv[kConvMaxChannels];   // B^-1 mod c_j
+    uint32_t binvp[kConvMaxChannels];  // its Shoup companion
+    uint32_t b[kConvMaxChannels];      // b_i
+    uint32_t hb[kConvMaxChannels];     // floor(B/2) mod b_i (0 when not rounding)
+    uint32_t w[kConvMaxChannels];      // (B / b_i)^-1 mod b_i
+    uint32_t wp[kConvMaxChannels];     // its Shoup companion
+};
+
+}  // namespace nttb200
+
+// Self-contained: copies what it needs from the two plans, which may be destroyed afterwards.
+struct nttb200_rns_conv {
+    int device = 0;
+    uint32_t logn = 12;
+    uint32_t src = 0;                  // S
+    uint32_t dst = 0;                  // T
+    int sm_count = 148;
+    nttb200::RnsConvConsts k{};        // hc / hb hold floor(B/2); zeroed per call without rounding
+};
+
+namespace nttb200 {
+
 extern std::atomic<uint64_t> g_launches;
 
 // error plumbing (api.cu)
@@ -183,6 +214,14 @@ int launch_rns_stream(const nttb200_rns_plan *rp, uint32_t op, const int32_t *a,
                       size_t batch, bool bcast, const uint32_t *scalars, cudaStream_t st);
 int launch_rns_dot(const nttb200_rns_plan *rp, const int32_t *a, const int32_t *w, int32_t *c, uint32_t terms,
                    size_t batch, bool w_shared, bool accumulate, cudaStream_t st);
+// basis conversion (kernels_rns_conv.cu).  rns_conv_prepare fills cv->k from the moduli
+// (host only; NTTB200_ERR_MODULUS when two of them share a factor).  launch_rns_conv: the
+// caller has checked the arguments, the overlap and the 16-byte alignment; src rows (S
+// channels) at src + b * src_stride, target input rows (mod_down only) at tin + b * src_stride,
+// output rows (T channels) at out + b * out_stride.
+int rns_conv_prepare(nttb200_rns_conv *cv, const uint32_t *b, const uint32_t *c);
+int launch_rns_conv(const nttb200_rns_conv *cv, const int32_t *src, const int32_t *tin, uint64_t src_stride,
+                    int32_t *out, uint64_t out_stride, size_t batch, bool down, bool round, cudaStream_t st);
 // q^-1 mod 2^32 for odd q (Montgomery products): Newton iteration, 3 correct bits doubling per step
 inline uint32_t inv_mod_2_32(uint32_t q) {
     uint32_t x = q;

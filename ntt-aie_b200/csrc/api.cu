@@ -7,7 +7,6 @@
 // nttb200_gs_batch / nttb200_gs_host.  There is no CPU compute path in here:
 // without a usable CUDA device every compute entry point returns an error.
 #include <stdio.h>
-#include <stdlib.h>
 #include <string.h>
 
 #include <new>
@@ -530,16 +529,13 @@ static void host_release(nttb200_plan *p) {
     p->host_ready = false;
 }
 
+// staging buffers of 32 MiB each: deep enough to hide the PCIe latency, small enough that the
+// first kernel starts early (measured: 46.2 GB/s each way at 32 MiB vs 44.7 at 16)
+constexpr size_t kHostChunkMB = 32;
+
 static int host_prepare(nttb200_plan *p) {
     if (p->host_ready) return NTTB200_OK;
-    // staging buffers of 32 MiB each: deep enough to hide the PCIe latency,
-    // small enough that the first kernel starts early
-    static const long chunk_mb = []() {
-        const char *e = getenv("NTTB200_HOST_CHUNK_MB");
-        long v = e ? atol(e) : 32L;  // measured: 46.2 GB/s each way at 32 MiB vs 44.7 at 16
-        return v < 1 ? 1L : v;
-    }();
-    size_t polys = ((size_t) chunk_mb << 20) / (sizeof(int32_t) * p->n);
+    size_t polys = (kHostChunkMB << 20) / (sizeof(int32_t) * p->n);
     if (polys < 1) polys = 1;
     for (int k = 0; k < kHostStreams; k++) {
         cudaError_t e = cudaStreamCreateWithFlags(&p->hstream[k], cudaStreamNonBlocking);
@@ -649,17 +645,17 @@ int nttb200_polymul_negacyclic(nttb200_plan *fwd, nttb200_plan *inv, const int32
     cudaStream_t st = (cudaStream_t) stream;
     const size_t words = batch * fwd->n;
     if (fwd->logn == 12 && !((fwd->flags | inv->flags) & NTTB200_FORCE_GENERIC)) {
-        // N = 4096: one kernel per product, operands and result cross HBM once (12 N bytes)
-        static const bool one_kernel = getenv("NTTB200_POLYMUL_3KERNEL") == nullptr;
-        if (one_kernel) {
-            int rc = launch_polymul4096(fwd, inv, d_a, d_b, d_c, batch, st);
-            if (rc != NTTB200_ERR_UNSUPPORTED) return rc;
-        }
+        // N = 4096: one kernel per product, operands and result cross HBM once (12 N bytes).
+        // It declines (launching nothing) on operands that are not 16-byte aligned, a d_c that
+        // is not 4-byte aligned or 2^31 tiles; the transform kernels would decline as well, so
+        // the generic pipeline below serves these calls.
+        int rc = launch_polymul4096(fwd, inv, d_a, d_b, d_c, batch, st);
+        if (rc != NTTB200_ERR_UNSUPPORTED) return rc;
     }
     // scratch for NTT(b) (and NTT(a) when the output aliases b)
     int32_t *tmp = nullptr;
-    const bool fast = !((fwd->flags | inv->flags) & NTTB200_FORCE_GENERIC) && fwd->d_tw_tile &&
-                      inv->d_tw_tile;
+    const bool fast = fwd->logn > 12 && !((fwd->flags | inv->flags) & NTTB200_FORCE_GENERIC) &&
+                      fwd->d_tw_tile && inv->d_tw_tile;
     if (fast) {
         // NTT(a), NTT(b) into scratch; pointwise product, inverse transform and the
         // N^-1 scaling in one pass over them
@@ -668,15 +664,8 @@ int nttb200_polymul_negacyclic(nttb200_plan *fwd, nttb200_plan *inv, const int32
             if (rca != NTTB200_OK) return rca;
         }
         int rc = launch_multi_ct(fwd, d_a, tmp, batch, st);
-        if (rc == NTTB200_OK && fwd->logn == 12 && inv->d_tw_r1 && !getenv("NTTB200_POLYMUL_DUAL")) {
-            // N = 4096: the pointwise product rides on the second forward transform (its
-            // operand load hides behind the row stages), the N^-1 on the inverse's store
-            rc = launch_multi_ct_mul(fwd, d_b, tmp, tmp + words, batch, st);
-            if (rc == NTTB200_OK) rc = launch_fused_gs_scaled(inv, tmp + words, d_c, batch, st);
-        } else {
-            if (rc == NTTB200_OK) rc = launch_multi_ct(fwd, d_b, tmp + words, batch, st);
-            if (rc == NTTB200_OK) rc = launch_multi_gs_dual(inv, tmp, tmp + words, d_c, batch, st);
-        }
+        if (rc == NTTB200_OK) rc = launch_multi_ct(fwd, d_b, tmp + words, batch, st);
+        if (rc == NTTB200_OK) rc = launch_multi_gs_dual(inv, tmp, tmp + words, d_c, batch, st);
         cudaError_t e = cudaFreeAsync(tmp, st);
         if (rc != NTTB200_ERR_UNSUPPORTED) {
             if (rc == NTTB200_OK && e != cudaSuccess) rc = cuda_fail(e, "cudaFreeAsync");
@@ -890,16 +879,17 @@ int nttb200_rns_polymul_negacyclic(nttb200_rns_plan *fwd, nttb200_rns_plan *inv,
     DeviceGuard guard(fwd->device);
     cudaStream_t st = (cudaStream_t) stream;
     // N = 4096, one kernel per channel: both operands enter the SM once, the product leaves once
-    // (12 N bytes per channel product instead of 28 N through the scratch buffers below)
-    static const bool one_kernel = getenv("NTTB200_RNS_POLYMUL_3KERNEL") == nullptr;
-    if (one_kernel && fwd->logn == 12) {
-        int rc1 = NTTB200_OK;
-        for (uint32_t l = 0; l < fwd->limbs && rc1 == NTTB200_OK; l++) {
-            rc1 = launch_polymul4096_strided(fwd->sub[l], inv->sub[l], d_a, d_b, d_c, batch, fwd->limbs, l, st);
+    // (12 N bytes per channel product instead of 28 N through the scratch buffers below).  It
+    // declines for the first channel already (launching nothing) where the transform kernels
+    // would decline as well: unaligned buffers, 2^31 tiles.
+    if (fwd->logn == 12) {
+        int rc = NTTB200_OK;
+        for (uint32_t l = 0; l < fwd->limbs && rc == NTTB200_OK; l++) {
+            rc = launch_polymul4096_strided(fwd->sub[l], inv->sub[l], d_a, d_b, d_c, batch, fwd->limbs, l, st);
         }
-        if (rc1 != NTTB200_ERR_UNSUPPORTED) return rc1;   // nothing was launched when unsupported (l == 0)
+        return rc;
     }
-    // CT(a), CT(b) into scratch (N > 4096: column pass + tile pass each); the DUAL tile pass
+    // N > 4096: CT(a), CT(b) into scratch (column pass + tile pass each); the DUAL tile pass
     // multiplies them at load and scales by N^-1 at the store, then the GS column pass
     if (batch > 0xffffffffull || ((uint64_t) batch * fwd->limbs << (fwd->logn - 12)) > 0x7fffffffull) {
         return NTTB200_ERR_UNSUPPORTED;   // the tile kernels count tiles in 31 bits

@@ -26,7 +26,6 @@
 // src/aie2.py:161-317; the twiddle index rule is the golden's table[h+i]
 // (src/test.cpp:45).
 #include <cuda.h>
-#include <stdlib.h>
 
 #include <vector>
 
@@ -146,8 +145,6 @@ struct FusedParams {
     uint32_t zero;        // always 0 (see gs_bfly)
     uint32_t four_q;      // 4q as an opaque value (computed in the kernel it is folded into LEA + VIMNMX)
     uint32_t permute;     // ans_order on store (reference src/test.cpp:69-71,212-219)
-    uint32_t scale;       // SCALE: every output times this constant (Shoup pair) -- the
-    uint32_t scale_shoup; // N^-1 of an inverse transform, fused into the store
 };
 
 // IN_BR / OUT_BR: layout adapters fused into the load and the store (SURVEY 8f.2): the input
@@ -160,7 +157,7 @@ struct FusedParams {
 // (Measured and kept out of this kernel: round-1 twiddles in tensor memory instead of the
 // 32 KiB shared-memory table, 0.471 against 0.462 ms; CTA-wide instead of team barriers,
 // 0.516 ms.)
-template <bool PERMUTE, bool SCALE = false, bool IN_BR = false, bool OUT_BR = false, bool L4 = false>
+template <bool PERMUTE, bool IN_BR = false, bool OUT_BR = false, bool L4 = false>
 __global__ void __launch_bounds__(kF_Threads, 1)
 fused_gs4096_kernel(const __grid_constant__ CUtensorMap map_lo,
                     const __grid_constant__ CUtensorMap map_hi,
@@ -298,12 +295,7 @@ fused_gs4096_kernel(const __grid_constant__ CUtensorMap map_lo,
                 blk = ((blk & 0x5) << 1) | ((blk & 0xA) >> 1);
                 row = (blk << 2) | (i & 3);
             }
-            if (SCALE) {
-                uint32_t r = shoup_mul_lazy(v[i], prm.scale, prm.scale_shoup, q);
-                dst[row * 64] = min(r - q, r);
-            } else {
-                dst[row * 64] = v[i];
-            }
+            dst[row * 64] = v[i];
         }
     }
 }
@@ -395,15 +387,13 @@ int fused_prepare(nttb200_plan *p) {
                                       cudaFuncAttributeMaxDynamicSharedMemorySize, kF_SmemBytes));
     NTTB200_CUDA(cudaFuncSetAttribute(fused_gs4096_kernel<true>,
                                       cudaFuncAttributeMaxDynamicSharedMemorySize, kF_SmemBytes));
-    NTTB200_CUDA(cudaFuncSetAttribute(fused_gs4096_kernel<false, false, false, false, true>,
-                                      cudaFuncAttributeMaxDynamicSharedMemorySize, kF_SmemBytes));
-    NTTB200_CUDA(cudaFuncSetAttribute(fused_gs4096_kernel<false, true>,
-                                      cudaFuncAttributeMaxDynamicSharedMemorySize, kF_SmemBytes));
-    NTTB200_CUDA(cudaFuncSetAttribute(fused_gs4096_kernel<false, false, true, false>,
-                                      cudaFuncAttributeMaxDynamicSharedMemorySize, kF_SmemBytes));
     NTTB200_CUDA(cudaFuncSetAttribute(fused_gs4096_kernel<false, false, false, true>,
                                       cudaFuncAttributeMaxDynamicSharedMemorySize, kF_SmemBytes));
-    NTTB200_CUDA(cudaFuncSetAttribute(fused_gs4096_kernel<false, false, true, true>,
+    NTTB200_CUDA(cudaFuncSetAttribute(fused_gs4096_kernel<false, true, false>,
+                                      cudaFuncAttributeMaxDynamicSharedMemorySize, kF_SmemBytes));
+    NTTB200_CUDA(cudaFuncSetAttribute(fused_gs4096_kernel<false, false, true>,
+                                      cudaFuncAttributeMaxDynamicSharedMemorySize, kF_SmemBytes));
+    NTTB200_CUDA(cudaFuncSetAttribute(fused_gs4096_kernel<false, true, true>,
                                       cudaFuncAttributeMaxDynamicSharedMemorySize, kF_SmemBytes));
     return NTTB200_OK;
 }
@@ -414,36 +404,22 @@ void fused_release(nttb200_plan *p) {
 }
 
 static int launch_fused_impl(nttb200_plan *p, const int32_t *d_in, int32_t *d_out, size_t batch,
-                             bool permute_out, bool scaled, cudaStream_t st, bool in_br = false,
-                             bool out_br = false);
-
-bool l4_enabled() {
-    static const bool on = getenv("NTTB200_NO_L4") == nullptr;
-    return on;
-}
+                             bool permute_out, cudaStream_t st, bool in_br = false, bool out_br = false);
 
 int launch_fused_gs(nttb200_plan *p, const int32_t *d_in, int32_t *d_out, size_t batch,
                     bool permute_out, cudaStream_t st) {
-    return launch_fused_impl(p, d_in, d_out, batch, permute_out, false, st);
+    return launch_fused_impl(p, d_in, d_out, batch, permute_out, st);
 }
 
 // golden network with the bit-reversal adapters fused into the load and/or the store
 int launch_fused_gs_bitrev(nttb200_plan *p, const int32_t *d_in, int32_t *d_out, size_t batch,
                            bool in_br, bool out_br, cudaStream_t st) {
     if (out_br && ((uintptr_t) d_out & 15u)) return NTTB200_ERR_UNSUPPORTED;
-    return launch_fused_impl(p, d_in, d_out, batch, false, false, st, in_br, out_br);
-}
-
-// golden network followed by a multiplication of every output by N^-1 * 2^32 mod q: the
-// inverse transform of a Montgomery-form pointwise product (nttb200_polymul_negacyclic)
-int launch_fused_gs_scaled(nttb200_plan *p, const int32_t *d_in, int32_t *d_out, size_t batch,
-                           cudaStream_t st) {
-    if (!(p->q & 1u)) return NTTB200_ERR_UNSUPPORTED;
-    return launch_fused_impl(p, d_in, d_out, batch, false, true, st);
+    return launch_fused_impl(p, d_in, d_out, batch, false, st, in_br, out_br);
 }
 
 static int launch_fused_impl(nttb200_plan *p, const int32_t *d_in, int32_t *d_out, size_t batch,
-                             bool permute_out, bool scaled, cudaStream_t st, bool in_br, bool out_br) {
+                             bool permute_out, cudaStream_t st, bool in_br, bool out_br) {
     if (p->logn != 12 || !p->d_tw_r1) return NTTB200_ERR_UNSUPPORTED;
     if (batch == 0) return NTTB200_OK;
     if (batch > 0x7fffffffull || ((uintptr_t) d_in & 15u) || ((uintptr_t) d_out & 3u)) {
@@ -461,31 +437,22 @@ static int launch_fused_impl(nttb200_plan *p, const int32_t *d_in, int32_t *d_ou
     prm.zero = 0;
     prm.four_q = 4u * p->q;   // only used when 8q fits a word
     prm.permute = permute_out;
-    prm.scale = prm.scale_shoup = 0;
-    if (scaled) {
-        uint64_t sc = ((uint64_t) p->n_inv << 32) % p->q;
-        prm.scale = (uint32_t) sc;
-        prm.scale_shoup = (uint32_t) ((sc << 32) / p->q);
-    }
     int grid = (int) (batch < (uint64_t) p->sm_count ? batch : (uint64_t) p->sm_count);
-    if (scaled) {
-        fused_gs4096_kernel<false, true><<<grid, kF_Threads, kF_SmemBytes, st>>>(map_lo, map_hi,
-                                                                                 p->uni_gs, prm);
-    } else if (permute_out) {
+    if (permute_out) {
         fused_gs4096_kernel<true><<<grid, kF_Threads, kF_SmemBytes, st>>>(map_lo, map_hi, p->uni_gs,
                                                                           prm);
     } else if (in_br && out_br) {
-        fused_gs4096_kernel<false, false, true, true><<<grid, kF_Threads, kF_SmemBytes, st>>>(
+        fused_gs4096_kernel<false, true, true><<<grid, kF_Threads, kF_SmemBytes, st>>>(
             map_lo, map_hi, p->uni_gs, prm);
     } else if (in_br) {
-        fused_gs4096_kernel<false, false, true, false><<<grid, kF_Threads, kF_SmemBytes, st>>>(
+        fused_gs4096_kernel<false, true, false><<<grid, kF_Threads, kF_SmemBytes, st>>>(
             map_lo, map_hi, p->uni_gs, prm);
     } else if (out_br) {
-        fused_gs4096_kernel<false, false, false, true><<<grid, kF_Threads, kF_SmemBytes, st>>>(
+        fused_gs4096_kernel<false, false, true><<<grid, kF_Threads, kF_SmemBytes, st>>>(
             map_lo, map_hi, p->uni_gs, prm);
     } else if (use_l4(p)) {
         // 8q fits a word: the 4q-lazy butterflies (fused_common.cuh, gs_bfly_l4)
-        fused_gs4096_kernel<false, false, false, false, true><<<grid, kF_Threads, kF_SmemBytes, st>>>(
+        fused_gs4096_kernel<false, false, false, true><<<grid, kF_Threads, kF_SmemBytes, st>>>(
             map_lo, map_hi, p->uni_gs, prm);
     } else {
         fused_gs4096_kernel<false><<<grid, kF_Threads, kF_SmemBytes, st>>>(map_lo, map_hi,
@@ -493,8 +460,7 @@ static int launch_fused_impl(nttb200_plan *p, const int32_t *d_in, int32_t *d_ou
     }
     g_launches.fetch_add(1, std::memory_order_relaxed);
     NTTB200_CUDA(cudaGetLastError());
-    p->last_path = scaled ? "fused_gs4096_tma_scaled"
-                          : (in_br || out_br) ? "fused_gs4096_tma_bitrev" : "fused_gs4096_tma";
+    p->last_path = (in_br || out_br) ? "fused_gs4096_tma_bitrev" : "fused_gs4096_tma";
     return NTTB200_OK;
 }
 

@@ -18,17 +18,12 @@
 // stages (src/aie2.py:178-295, src/aie_core.cc:161-187).
 //
 // Also in this file (all built from the same team/tile machinery):
-//   poly_gs_kernel / poly_ct_kernel   N = 2^13..2^15 in ONE pass: the tiles of a polynomial
-//                                     on G teams of one CTA, cross-tile stages in a third
-//                                     register round through the tile buffers
-//   tile_ct_kernel / tile_ct_db_kernel  the forward (Cooley-Tukey) tile pass, output through
-//                                     a TMA store; MULT fuses a pointwise product
+//   tile_ct_kernel / tile_ct_h_kernel the forward (Cooley-Tukey) tile pass, output through
+//                                     a TMA store
 //   tile_gs_kernel<DUAL>              pointwise product at load + N^-1 at the store
 //   template mode RNS                 tile position -> residue channel with its own modulus
 //                                     (column_kernel<.., RNS>: polynomial -> channel)
 //   column_kernel<.., SCATTER>        the multi-GPU exchange as NVLink peer stores
-#include <stdlib.h>
-
 #include <vector>
 
 #include "tile_common.cuh"
@@ -63,7 +58,6 @@ __device__ __forceinline__ uint4 rns_channel(const RnsConsts &rns, uint32_t c) {
 //   negacyclic product).  The network is linear, so scaling here instead of after the
 //   last column pass gives the same residues.
 // TWMODE: where the twiddles come from.  0 = global memory (LDG; any workload),
-// 1 = one shared-memory table for the whole launch (every tile at position 0: N = 4096),
 // 2 = shared-memory table per SEGMENT: the CTA's range of position-major tiles is cut
 //     at position changes, the table of the segment's position is staged between two
 //     __syncthreads (batched large-N and RNS workloads, where a segment is long).
@@ -92,12 +86,6 @@ tile_gs_kernel(const __grid_constant__ CUtensorMap map_lo, const __grid_constant
     static_assert(!(DUAL && SCALED) && !(L4 && SCALED), "SCALED is the plain-load form of DUAL's store");
 
     const uint32_t tws = bar_base + 64;
-    if (TWMODE == 1) {
-        for (int i = tid; i < kM_TwTile; i += kM_Threads) {
-            uint4 x = __ldg(prm.tw_tile + i);
-            sts128(tws + i * 16, x.x, x.y, x.z, x.w);
-        }
-    }
     if (tid < kM_Teams) mbar_init(bar_base + tid * 8, 1);
     asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
     __syncthreads();
@@ -252,188 +240,17 @@ tile_gs_kernel(const __grid_constant__ CUtensorMap map_lo, const __grid_constant
     }  // segments
 }
 
-// N = 2^13 .. 2^15 in ONE pass: the G = N/4096 tiles of a polynomial are taken by G
-// teams of the same CTA at the same time.  Each team runs the two register rounds of
-// its tile (stages 0-11) exactly as above; then a third round exchanges through the G
-// tile buffers (every thread keeps 64/G register rows of ALL G tiles) and runs the
-// last log2 G stages -- the cross-tile stages -- in registers, so no second HBM pass
-// is needed.  Successor of the reference's cross-tile ntt_1stage calls
-// (src/aie_core.cc:161-187, src/aie2.py:184-295) with a group barrier in the role of
-// the lock fifos (src/aie2.py:128-154).
-template <int LOGG, bool DUAL>
-__global__ void __launch_bounds__(kM_Threads, 1)
-poly_gs_kernel(const __grid_constant__ CUtensorMap map_lo, const __grid_constant__ CUtensorMap map_hi,
-               const __grid_constant__ CUtensorMap map_b_lo,
-               const __grid_constant__ CUtensorMap map_b_hi, const TileParams prm,
-               const uint2 *__restrict__ tw_flat) {
-    constexpr int G = 1 << LOGG;           // tiles = teams per polynomial
-    constexpr int kGroups = kM_Teams / G;  // polynomials in flight per CTA
-    constexpr int kSlice = 64 / G;         // register rows a thread keeps in round 3
-    extern __shared__ uint8_t smem_raw[];
-    const uint32_t data_base = (smem_u32(smem_raw) + 1023u) & ~1023u;
-    const uint32_t bar_base = data_base + kM_Teams * kF_PolyBytes;
-    const int tid = threadIdx.x;
-    const int team = __shfl_sync(0xffffffffu, tid >> 6, 0);  // warp-uniform for the compiler
-    const int j = tid & 63;
-    const int grp = team >> LOGG, t = team & (G - 1);
-    const uint32_t q = prm.q, two_q = 2u * prm.q, zero = prm.zero;
-
-    if (tid < kM_Teams) mbar_init(bar_base + tid * 8, 1);
-    asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
-    __syncthreads();
-
-    const uint32_t buf = data_base + team * kF_PolyBytes;
-    const uint32_t gbuf = data_base + (grp << LOGG) * kF_PolyBytes;
-    const uint32_t bar = bar_base + team * 8;
-    const uint32_t stride = gridDim.x * kGroups;
-    uint32_t poly = blockIdx.x * kGroups + grp;
-    uint32_t parity = 0;
-    if (j == 0 && poly < prm.batch) {
-        mbar_expect_tx(bar, kF_PolyBytes);
-        tma_load_3d(buf, &map_lo, bar, 0, 0, (int) (poly * G + t));
-        tma_load_3d(buf + kF_PolyBytes / 2, &map_hi, bar, 0, 0, (int) (poly * G + t));
-    }
-    const uint32_t r1_row = buf + j * 128;
-    const uint32_t r1_xor = (j & 7) << 4;
-    const uint32_t r2_col = buf + (j >> 5) * (kF_PolyBytes / 2) + (j & 3) * 4;
-    const uint32_t r2_chunk = ((j & 31) >> 2) << 4;
-    const uint4 *tw = prm.tw_tile + (size_t) t * kM_TwTile;
-    auto group_sync = [&]() {
-        asm volatile("bar.sync %0, %1;" ::"r"(9 + grp), "n"(G * 64) : "memory");
-    };
-
-    for (; poly < prm.batch; poly += stride) {
-        uint32_t v[64];
-        const int tile = (int) (poly * G + t);
-        mbar_wait(bar, parity);
-        parity ^= 1;
-#pragma unroll
-        for (int c = 0; c < 16; c++) {
-            uint4 x = lds128(r1_row + (c >> 3) * (kF_PolyBytes / 2) + (((c & 7) << 4) ^ r1_xor));
-            v[4 * c + 0] = x.x;
-            v[4 * c + 1] = x.y;
-            v[4 * c + 2] = x.z;
-            v[4 * c + 3] = x.w;
-        }
-        if (DUAL) {
-            team_sync(team);
-            if (j == 0) {
-                mbar_expect_tx(bar, kF_PolyBytes);
-                tma_load_3d(buf, &map_b_lo, bar, 0, 0, tile);
-                tma_load_3d(buf + kF_PolyBytes / 2, &map_b_hi, bar, 0, 0, tile);
-            }
-            mbar_wait(bar, parity);
-            parity ^= 1;
-#pragma unroll
-            for (int c = 0; c < 16; c++) {
-                uint4 x = lds128(r1_row + (c >> 3) * (kF_PolyBytes / 2) + (((c & 7) << 4) ^ r1_xor));
-                const uint32_t bb[4] = {x.x, x.y, x.z, x.w};
-#pragma unroll
-                for (int e = 0; e < 4; e++) {
-                    uint64_t prod = (uint64_t) v[4 * c + e] * bb[e];
-                    uint32_t m = (uint32_t) prod * prm.qinv;
-                    v[4 * c + e] = (uint32_t) (prod >> 32) - __umulhi(m, q) + q;
-                }
-            }
-        }
-        const uint4 *tw1 = tw + j;
-        gs_stage_g<0, DUAL>(v, tw1, q, two_q, zero);
-        gs_stage_g<1, true>(v, tw1, q, two_q, zero);
-        gs_stage_g<2, true>(v, tw1, q, two_q, zero);
-        gs_stage_g<3, true>(v, tw1, q, two_q, zero);
-        gs_stage_g<4, true>(v, tw1, q, two_q, zero);
-        gs_stage_g<5, true>(v, tw1, q, two_q, zero);
-#pragma unroll
-        for (int c = 0; c < 16; c++) {
-            sts128(r1_row + (c >> 3) * (kF_PolyBytes / 2) + (((c & 7) << 4) ^ r1_xor), v[4 * c],
-                   v[4 * c + 1], v[4 * c + 2], v[4 * c + 3]);
-        }
-        team_sync(team);
-#pragma unroll
-        for (int i = 0; i < 64; i++) {
-            v[i] = lds32(r2_col + i * 128 + (r2_chunk ^ ((i & 7) << 4)));
-        }
-        team_sync(team);
-        const uint4 *tw2 = tw + 64;
-        gs_stage_g<0, true>(v, tw2, q, two_q, zero);
-        gs_stage_g<1, true>(v, tw2, q, two_q, zero);
-        gs_stage_g<2, true>(v, tw2, q, two_q, zero);
-        gs_stage_g<3, true>(v, tw2, q, two_q, zero);
-        gs_stage_g<4, true>(v, tw2, q, two_q, zero);
-        gs_stage_g<5, true>(v, tw2, q, two_q, zero);
-
-        // ---- round 3: register i is a[t*4096 + j + 64 i].  Park it at [i][j] of this
-        // team's buffer, then collect rows t*kSlice .. +kSlice-1 of ALL G tiles.
-#pragma unroll
-        for (int i = 0; i < 64; i++) {
-            asm volatile("st.shared.u32 [%0], %1;" ::"r"(buf + (i * 64 + j) * 4), "r"(v[i]) : "memory");
-        }
-        group_sync();
-        uint32_t w[64];
-#pragma unroll
-        for (int tt = 0; tt < G; tt++) {
-#pragma unroll
-            for (int ii = 0; ii < kSlice; ii++) {
-                w[tt * kSlice + ii] =
-                    lds32(gbuf + tt * kF_PolyBytes + (((t * kSlice + ii) * 64 + j) << 2));
-            }
-        }
-        fence_proxy_async();
-        group_sync();
-        // ---- every buffer of the group is free: prefetch this team's next tile
-        const uint32_t next = poly + stride;
-        if (j == 0 && next < prm.batch) {
-            mbar_expect_tx(bar, kF_PolyBytes);
-            tma_load_3d(buf, &map_lo, bar, 0, 0, (int) (next * G + t));
-            tma_load_3d(buf + kF_PolyBytes / 2, &map_hi, bar, 0, 0, (int) (next * G + t));
-        }
-        // ---- stages 12 .. 12+LOGG-1 pair tiles tt and tt + 2^m; twiddle
-        //      table[(G >> (m+1)) + (tt >> (m+1))], the same for every thread
-#pragma unroll
-        for (int m = 0; m < LOGG; m++) {
-#pragma unroll
-            for (int b2 = 0; b2 < (G >> (m + 1)); b2++) {
-                const uint2 tq = __ldg(tw_flat + (G >> (m + 1)) + b2);
-#pragma unroll
-                for (int e = 0; e < (1 << m); e++) {
-                    const int t0 = (b2 << (m + 1)) + e;
-#pragma unroll
-                    for (int ii = 0; ii < kSlice; ii++) {
-                        gs_bfly<true>(w[t0 * kSlice + ii], w[(t0 + (1 << m)) * kSlice + ii], tq.x, tq.y,
-                                      q, two_q, zero);
-                    }
-                }
-            }
-        }
-        uint32_t *dst = prm.out + ((size_t) poly << (12 + LOGG)) + j + 64 * (t * kSlice);
-#pragma unroll
-        for (int tt = 0; tt < G; tt++) {
-#pragma unroll
-            for (int ii = 0; ii < kSlice; ii++) {
-                uint32_t r = w[tt * kSlice + ii];
-                if (DUAL) r = shoup_mul_lazy(r, prm.scale, prm.scale_shoup, q);
-                dst[tt * 4096 + ii * 64] = min(r - q, r);
-            }
-        }
-    }
-}
-
 // Forward partner: CT stages 11..0 of every tile (stride 2048 -> 1).  Columns first
 // (uniform twiddles), exchange, rows (thread-private twiddles); the rows go back to the
 // team's buffer and leave through a TMA store.
-// MULT: the transformed tile is multiplied point by point with the same tile of a third
-// buffer (an already transformed operand) before it is stored -- a Montgomery product
-// x*y*2^-32, canonical.  That operand's TMA load is issued as soon as the rows are in
-// registers and lands behind the six row stages, so it costs no waiting.
-// STAGED (not with SMEM_TW / MULT): an 8 KiB staging slot per team takes the output in two
-// halves (see tile_ct_h_kernel below), so the tile buffer receives the prefetch of the team's next
-// tile as soon as the rows are in registers instead of after the store has drained.
-template <int RNS, bool SMEM_TW = false, bool MULT = false, bool STAGED = false, bool L4 = false>
+// An 8 KiB staging slot per team takes the output in two halves (see tile_ct_h_kernel below),
+// so the tile buffer receives the prefetch of the team's next tile as soon as the rows are in
+// registers instead of after the store has drained.
+template <int RNS, bool L4 = false>
 __global__ void __launch_bounds__(kM_Threads, 1)
 tile_ct_kernel(const __grid_constant__ CUtensorMap map_lo, const __grid_constant__ CUtensorMap map_hi,
                const __grid_constant__ CUtensorMap out_lo, const __grid_constant__ CUtensorMap out_hi,
-               const TileParams prm, const __grid_constant__ RnsConsts rns,
-               const __grid_constant__ CUtensorMap mul_lo, const __grid_constant__ CUtensorMap mul_hi) {
+               const TileParams prm, const __grid_constant__ RnsConsts rns) {
     extern __shared__ uint8_t smem_raw[];
     const uint32_t data_base = (smem_u32(smem_raw) + 1023u) & ~1023u;
     const uint32_t bar_base = data_base + kM_Teams * kF_PolyBytes;
@@ -446,20 +263,12 @@ tile_ct_kernel(const __grid_constant__ CUtensorMap map_lo, const __grid_constant
     uint32_t q = prm.q, two_q = 2u * prm.q;
     const uint32_t zero = prm.zero;
 
-    const uint32_t tws = bar_base + 64;
-    static_assert(!STAGED || (!SMEM_TW && !MULT), "the staged variant has no table / product form");
-    static_assert(!L4 || (STAGED && !RNS), "4q-lazy only in the staged single-modulus form");
+    static_assert(!L4 || !RNS, "4q-lazy only in the single-modulus form");
     const uint32_t four_q = prm.four_q;
     constexpr int kBCol = ct_l4_out_n(1, 6), kB4 = ct_l4_out(kBCol), kB3 = ct_l4_out(kB4), kB2 = ct_l4_out(kB3),
                   kB1 = ct_l4_out(kB2), kB0 = ct_l4_out(kB1), kBRow = ct_l4_out(kB0);
     const uint32_t stg = ((bar_base + 64 + 1023u) & ~1023u) + team * (kF_PolyBytes / 2);
     const uint32_t st_row = stg + j * 128;
-    if (SMEM_TW) {
-        for (int i = tid; i < kM_TwTile; i += kM_Threads) {
-            uint4 x = __ldg(prm.tw_tile + i);
-            sts128(tws + i * 16, x.x, x.y, x.z, x.w);
-        }
-    }
     if (tid < kM_Teams) mbar_init(bar_base + tid * 8, 1);
     asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
     __syncthreads();
@@ -508,8 +317,6 @@ tile_ct_kernel(const __grid_constant__ CUtensorMap map_lo, const __grid_constant
         }
         if (L4) {
             ct_round_l4<1>(v, TwGlobal{tw + 64}, q, two_q, four_q, zero);
-        } else if (SMEM_TW) {
-            ct_round<false>(v, TwShared{tws + 64 * 16}, q, two_q, zero);
         } else {
             ct_round<false>(v, TwGlobal{tw + 64}, q, two_q, zero);
         }
@@ -529,300 +336,72 @@ tile_ct_kernel(const __grid_constant__ CUtensorMap map_lo, const __grid_constant
             v[4 * c + 2] = t.z;
             v[4 * c + 3] = t.w;
         }
-        if (MULT) {
-            // the buffer is idle during the row stages: fetch the other operand's tile
-            fence_proxy_async();
-            team_sync(team);
-            if (j == 0) {
-                mbar_expect_tx(bar, kF_PolyBytes);
-                tma_load_3d(buf, &mul_lo, bar, 0, 0, (int) tile_cur);
-                tma_load_3d(buf + kF_PolyBytes / 2, &mul_hi, bar, 0, 0, (int) tile_cur);
-            }
-        }
-        if constexpr (STAGED) {
-            // ---- the tile buffer is free: prefetch the team's next tile; the staging slot is free
-            // once the previous tile's right half has been read by its store
-            fence_proxy_async();
-            if (j == 0) asm volatile("cp.async.bulk.wait_group.read 0;" ::: "memory");
-            team_sync(team);
-            const uint32_t next = u + kM_Teams;
-            uint32_t tile_next = 0;
-            if (next < u_end) tile_next = tile_of(next, c_cur);
-            if (j == 0 && next < u_end) {
-                mbar_expect_tx(bar, kF_PolyBytes);
-                tma_load_3d(buf, &map_lo, bar, 0, 0, (int) tile_next);
-                tma_load_3d(buf + kF_PolyBytes / 2, &map_hi, bar, 0, 0, (int) tile_next);
-            }
-            // ---- rows: stage 5 pairs the halves, stages 4..0 run per half
-            const TwGlobal twr{tw + j};
-            if (L4) {
-                ct_stage_l4<5, kBCol>(v, twr, q, two_q, four_q, zero);
-            } else {
-                ct_stage_t<5, true>(v, twr, q, two_q, zero);
-            }
-#pragma unroll
-            for (int h = 0; h < 2; h++) {
-                if (h == 0) {
-                    ct_half_stage<4, 0, (L4 ? kB4 : -1)>(v, twr, q, two_q, four_q, zero);
-                    ct_half_stage<3, 0, (L4 ? kB3 : -1)>(v, twr, q, two_q, four_q, zero);
-                    ct_half_stage<2, 0, (L4 ? kB2 : -1)>(v, twr, q, two_q, four_q, zero);
-                    ct_half_stage<1, 0, (L4 ? kB1 : -1)>(v, twr, q, two_q, four_q, zero);
-                    ct_half_stage<0, 0, (L4 ? kB0 : -1)>(v, twr, q, two_q, four_q, zero);
-                } else {
-                    ct_half_stage<4, 1, (L4 ? kB4 : -1)>(v, twr, q, two_q, four_q, zero);
-                    ct_half_stage<3, 1, (L4 ? kB3 : -1)>(v, twr, q, two_q, four_q, zero);
-                    ct_half_stage<2, 1, (L4 ? kB2 : -1)>(v, twr, q, two_q, four_q, zero);
-                    ct_half_stage<1, 1, (L4 ? kB1 : -1)>(v, twr, q, two_q, four_q, zero);
-                    ct_half_stage<0, 1, (L4 ? kB0 : -1)>(v, twr, q, two_q, four_q, zero);
-                    if (j == 0) asm volatile("cp.async.bulk.wait_group.read 0;" ::: "memory");
-                    team_sync(team);
-                }
-#pragma unroll
-                for (int c = 0; c < 8; c++) {
-                    uint32_t o[4];
-#pragma unroll
-                    for (int e = 0; e < 4; e++) {
-                        uint32_t r = v[32 * h + 4 * c + e];
-                        if (L4) {
-                            o[e] = canon_l4(kBRow, r, q, two_q, four_q);
-                        } else {
-                            r = min(r - two_q, r);
-                            o[e] = min(r - q, r);
-                        }
-                    }
-                    sts128(st_row + ((c << 4) ^ r1_xor), o[0], o[1], o[2], o[3]);
-                }
-                fence_proxy_async();
-                team_sync(team);
-                if (j == 0) {
-                    tma_store_3d(h == 0 ? &out_lo : &out_hi, stg, 0, 0, (int) tile_cur);
-                    asm volatile("cp.async.bulk.commit_group;" ::: "memory");
-                }
-            }
-            tile_cur = tile_next;
-            continue;
-        }
-        // ---- rows: stages 5..0
-        if (SMEM_TW) {
-            ct_round<true>(v, TwShared{tws + j * 16}, q, two_q, zero);
-        } else {
-            ct_round<true>(v, TwGlobal{tw + j}, q, two_q, zero);
-        }
-        if (MULT) {
-            mbar_wait(bar, parity);
-            parity ^= 1;
-        }
-        // ---- canonical rows back to the buffer, TMA store, then the next load
-#pragma unroll
-        for (int c = 0; c < 16; c++) {
-            uint32_t o[4];
-            uint4 other = make_uint4(0, 0, 0, 0);
-            if (MULT) {
-                other = lds128(r1_row + (c >> 3) * (kF_PolyBytes / 2) + (((c & 7) << 4) ^ r1_xor));
-            }
-            const uint32_t ob[4] = {other.x, other.y, other.z, other.w};
-#pragma unroll
-            for (int e = 0; e < 4; e++) {
-                uint32_t r = v[4 * c + e];
-                r = min(r - two_q, r);
-                if (MULT) {
-                    // r in [0, 2q), other operand canonical: x*y*2^-32 in (0, 2q)
-                    uint64_t prod = (uint64_t) r * ob[e];
-                    uint32_t m = (uint32_t) prod * prm.qinv;
-                    r = (uint32_t) (prod >> 32) - __umulhi(m, q) + q;
-                }
-                o[e] = min(r - q, r);
-            }
-            sts128(r1_row + (c >> 3) * (kF_PolyBytes / 2) + (((c & 7) << 4) ^ r1_xor), o[0], o[1],
-                   o[2], o[3]);
-        }
+        // ---- the tile buffer is free: prefetch the team's next tile; the staging slot is free
+        // once the previous tile's right half has been read by its store
         fence_proxy_async();
+        if (j == 0) asm volatile("cp.async.bulk.wait_group.read 0;" ::: "memory");
         team_sync(team);
         const uint32_t next = u + kM_Teams;
         uint32_t tile_next = 0;
         if (next < u_end) tile_next = tile_of(next, c_cur);
-        if (j == 0) {
-            tma_store_3d(&out_lo, buf, 0, 0, (int) tile_cur);
-            tma_store_3d(&out_hi, buf + kF_PolyBytes / 2, 0, 0, (int) tile_cur);
-            tma_store_commit_and_wait_read();
-            if (next < u_end) {
-                mbar_expect_tx(bar, kF_PolyBytes);
-                tma_load_3d(buf, &map_lo, bar, 0, 0, (int) tile_next);
-                tma_load_3d(buf + kF_PolyBytes / 2, &map_hi, bar, 0, 0, (int) tile_next);
+        if (j == 0 && next < u_end) {
+            mbar_expect_tx(bar, kF_PolyBytes);
+            tma_load_3d(buf, &map_lo, bar, 0, 0, (int) tile_next);
+            tma_load_3d(buf + kF_PolyBytes / 2, &map_hi, bar, 0, 0, (int) tile_next);
+        }
+        // ---- rows: stage 5 pairs the halves, stages 4..0 run per half
+        const TwGlobal twr{tw + j};
+        if (L4) {
+            ct_stage_l4<5, kBCol>(v, twr, q, two_q, four_q, zero);
+        } else {
+            ct_stage_t<5, true>(v, twr, q, two_q, zero);
+        }
+#pragma unroll
+        for (int h = 0; h < 2; h++) {
+            if (h == 0) {
+                ct_half_stage<4, 0, (L4 ? kB4 : -1)>(v, twr, q, two_q, four_q, zero);
+                ct_half_stage<3, 0, (L4 ? kB3 : -1)>(v, twr, q, two_q, four_q, zero);
+                ct_half_stage<2, 0, (L4 ? kB2 : -1)>(v, twr, q, two_q, four_q, zero);
+                ct_half_stage<1, 0, (L4 ? kB1 : -1)>(v, twr, q, two_q, four_q, zero);
+                ct_half_stage<0, 0, (L4 ? kB0 : -1)>(v, twr, q, two_q, four_q, zero);
+            } else {
+                ct_half_stage<4, 1, (L4 ? kB4 : -1)>(v, twr, q, two_q, four_q, zero);
+                ct_half_stage<3, 1, (L4 ? kB3 : -1)>(v, twr, q, two_q, four_q, zero);
+                ct_half_stage<2, 1, (L4 ? kB2 : -1)>(v, twr, q, two_q, four_q, zero);
+                ct_half_stage<1, 1, (L4 ? kB1 : -1)>(v, twr, q, two_q, four_q, zero);
+                ct_half_stage<0, 1, (L4 ? kB0 : -1)>(v, twr, q, two_q, four_q, zero);
+                if (j == 0) asm volatile("cp.async.bulk.wait_group.read 0;" ::: "memory");
+                team_sync(team);
+            }
+#pragma unroll
+            for (int c = 0; c < 8; c++) {
+                uint32_t o[4];
+#pragma unroll
+                for (int e = 0; e < 4; e++) {
+                    uint32_t r = v[32 * h + 4 * c + e];
+                    if (L4) {
+                        o[e] = canon_l4(kBRow, r, q, two_q, four_q);
+                    } else {
+                        r = min(r - two_q, r);
+                        o[e] = min(r - q, r);
+                    }
+                }
+                sts128(st_row + ((c << 4) ^ r1_xor), o[0], o[1], o[2], o[3]);
+            }
+            fence_proxy_async();
+            team_sync(team);
+            if (j == 0) {
+                tma_store_3d(h == 0 ? &out_lo : &out_hi, stg, 0, 0, (int) tile_cur);
+                asm volatile("cp.async.bulk.commit_group;" ::: "memory");
             }
         }
         tile_cur = tile_next;
     }
-    if (STAGED && j == 0) asm volatile("cp.async.bulk.wait_group.read 0;" ::: "memory");
-    // every store was followed by wait_group.read, so shared memory is no longer in
-    // use when the CTA exits; the writes themselves complete before the grid does.
-    // (A trailing divergent wait here also stops ptxas from keeping q/2q in uniform
-    // registers -- measured in the SASS.)
-}
-
-// N = 4096 forward transform with TWO buffers per team (6 teams per CTA): the output of
-// tile k leaves buffer k&1 through a TMA store while tile k+1 is already being worked
-// on in the other buffer and tile k+2's load is queued behind the store -- the dead
-// time of tile_ct_kernel (store drain + load latency after every tile) disappears.
-constexpr int kD_Teams = 6;
-constexpr int kD_Threads = kD_Teams * kF_Team;
-constexpr int kD_SmemBytes = kD_Teams * 2 * kF_PolyBytes + kM_TwTile * 16 + 128 + 1024;
-
-template <bool MULT, bool L4 = false>
-__global__ void __launch_bounds__(kD_Threads, 1)
-tile_ct_db_kernel(const __grid_constant__ CUtensorMap map_lo, const __grid_constant__ CUtensorMap map_hi,
-                  const __grid_constant__ CUtensorMap out_lo, const __grid_constant__ CUtensorMap out_hi,
-                  const __grid_constant__ CUtensorMap mul_lo, const __grid_constant__ CUtensorMap mul_hi,
-                  const __grid_constant__ UniformTw uni, const TileParams prm) {
-    extern __shared__ uint8_t smem_raw[];
-    const uint32_t data_base = (smem_u32(smem_raw) + 1023u) & ~1023u;
-    const uint32_t bar_base = data_base + kD_Teams * 2 * kF_PolyBytes;   // 2 mbarriers per team
-    const uint32_t tws = bar_base + 128;
-    const int tid = threadIdx.x;
-    const int team = __shfl_sync(0xffffffffu, tid >> 6, 0);
-    const int j = tid & 63;
-    const uint32_t q = prm.q, two_q = 2u * prm.q, four_q = prm.four_q, zero = prm.zero;
-
-    for (int i = tid; i < kM_TwTile; i += kD_Threads) {
-        uint4 x = __ldg(prm.tw_tile + i);
-        sts128(tws + i * 16, x.x, x.y, x.z, x.w);
-    }
-    if (tid < kD_Teams * 2) mbar_init(bar_base + tid * 8, 1);
-    asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
-    __syncthreads();
-
-    const uint32_t total = prm.batch;  // chunks == 1
-    const uint32_t stride = gridDim.x * kD_Teams;
-    uint32_t tile = blockIdx.x * kD_Teams + team;
-    const uint32_t buf0 = data_base + team * 2 * kF_PolyBytes;
-    const uint32_t bar0 = bar_base + team * 16;
-    uint32_t parity0 = 0, parity1 = 0;
-    if (j == 0 && tile < total) {
-        mbar_expect_tx(bar0, kF_PolyBytes);
-        tma_load_3d(buf0, &map_lo, bar0, 0, 0, (int) tile);
-        tma_load_3d(buf0 + kF_PolyBytes / 2, &map_hi, bar0, 0, 0, (int) tile);
-    }
-    const uint32_t r1_off = j * 128;
-    const uint32_t r1_xor = (j & 7) << 4;
-    const uint32_t r2_off = (j >> 5) * (kF_PolyBytes / 2) + (j & 3) * 4;
-    const uint32_t r2_chunk = ((j & 31) >> 2) << 4;
-
-    for (uint32_t k = 0; tile < total; tile += stride, k++) {
-        const uint32_t cur = k & 1;
-        const uint32_t buf = buf0 + cur * kF_PolyBytes;
-        const uint32_t bar = bar0 + cur * 8;
-        const uint32_t next = tile + stride;
-        if (j == 0) {
-            // the other buffer held the previous tile's output: once the TMA store has
-            // read it, queue the next tile's load there
-            asm volatile("cp.async.bulk.wait_group.read 0;" ::: "memory");
-            if (next < total) {
-                const uint32_t nbuf = buf0 + (cur ^ 1) * kF_PolyBytes, nbar = bar0 + (cur ^ 1) * 8;
-                mbar_expect_tx(nbar, kF_PolyBytes);
-                tma_load_3d(nbuf, &map_lo, nbar, 0, 0, (int) next);
-                tma_load_3d(nbuf + kF_PolyBytes / 2, &map_hi, nbar, 0, 0, (int) next);
-            }
-        }
-        uint32_t v[64];
-        if (cur == 0) {
-            mbar_wait(bar, parity0);
-            parity0 ^= 1;
-        } else {
-            mbar_wait(bar, parity1);
-            parity1 ^= 1;
-        }
-        const uint32_t r2_col = buf + r2_off, r1_row = buf + r1_off;
-#pragma unroll
-        for (int i = 0; i < 64; i++) {
-            v[i] = lds32(r2_col + i * 128 + (r2_chunk ^ ((i & 7) << 4)));
-        }
-        // stages 11..6: twiddles table[1..63] from the constant bank
-        constexpr int kBCol = ct_l4_out_n(1, 6), kBRow = ct_l4_out_n(kBCol, 6);   // L4 bounds
-        if (L4) {
-            ct_round_uniform_l4<1>(v, uni, q, two_q, four_q, zero);
-        } else {
-            ct_stage_uniform<5, false>(v, uni, q, two_q, zero);
-            ct_stage_uniform<4, true>(v, uni, q, two_q, zero);
-            ct_stage_uniform<3, true>(v, uni, q, two_q, zero);
-            ct_stage_uniform<2, true>(v, uni, q, two_q, zero);
-            ct_stage_uniform<1, true>(v, uni, q, two_q, zero);
-            ct_stage_uniform<0, true>(v, uni, q, two_q, zero);
-        }
-#pragma unroll
-        for (int i = 0; i < 64; i++) {
-            asm volatile("st.shared.u32 [%0], %1;" ::"r"(r2_col + i * 128 + (r2_chunk ^ ((i & 7) << 4))),
-                         "r"(v[i])
-                         : "memory");
-        }
-        team_sync(team);
-#pragma unroll
-        for (int c = 0; c < 16; c++) {
-            uint4 t = lds128(r1_row + (c >> 3) * (kF_PolyBytes / 2) + (((c & 7) << 4) ^ r1_xor));
-            v[4 * c + 0] = t.x;
-            v[4 * c + 1] = t.y;
-            v[4 * c + 2] = t.z;
-            v[4 * c + 3] = t.w;
-        }
-        if (MULT) {
-            fence_proxy_async();
-            team_sync(team);
-            if (j == 0) {
-                mbar_expect_tx(bar, kF_PolyBytes);
-                tma_load_3d(buf, &mul_lo, bar, 0, 0, (int) tile);
-                tma_load_3d(buf + kF_PolyBytes / 2, &mul_hi, bar, 0, 0, (int) tile);
-            }
-        }
-        if (L4) {
-            ct_round_l4<kBCol>(v, TwShared{tws + j * 16}, q, two_q, four_q, zero);
-        } else {
-            ct_round<true>(v, TwShared{tws + j * 16}, q, two_q, zero);
-        }
-        if (MULT) {
-            if (cur == 0) {
-                mbar_wait(bar, parity0);
-                parity0 ^= 1;
-            } else {
-                mbar_wait(bar, parity1);
-                parity1 ^= 1;
-            }
-        }
-#pragma unroll
-        for (int c = 0; c < 16; c++) {
-            uint32_t o[4];
-            uint4 other = make_uint4(0, 0, 0, 0);
-            if (MULT) {
-                other = lds128(r1_row + (c >> 3) * (kF_PolyBytes / 2) + (((c & 7) << 4) ^ r1_xor));
-            }
-            const uint32_t ob[4] = {other.x, other.y, other.z, other.w};
-#pragma unroll
-            for (int e = 0; e < 4; e++) {
-                uint32_t r = v[4 * c + e];
-                if (MULT) {
-                    // any word times a canonical value is below 2^32 q: no reduction first
-                    uint64_t prod = (uint64_t) r * ob[e];
-                    uint32_t m = (uint32_t) prod * prm.qinv;
-                    r = (uint32_t) (prod >> 32) - __umulhi(m, q) + q;
-                    o[e] = min(r - q, r);
-                } else if (L4) {
-                    o[e] = canon_l4(kBRow, r, q, two_q, four_q);
-                } else {
-                    r = min(r - two_q, r);
-                    o[e] = min(r - q, r);
-                }
-            }
-            sts128(r1_row + (c >> 3) * (kF_PolyBytes / 2) + (((c & 7) << 4) ^ r1_xor), o[0], o[1],
-                   o[2], o[3]);
-        }
-        fence_proxy_async();
-        team_sync(team);
-        if (j == 0) {
-            tma_store_3d(&out_lo, buf, 0, 0, (int) tile);
-            tma_store_3d(&out_hi, buf + kF_PolyBytes / 2, 0, 0, (int) tile);
-            asm volatile("cp.async.bulk.commit_group;" ::: "memory");
-        }
-    }
+    // the last tile's halves may still be read out of the staging slot by their stores: no
+    // CTA leaves before that; the writes themselves complete before the grid does
     if (j == 0) asm volatile("cp.async.bulk.wait_group.read 0;" ::: "memory");
 }
+
 
 // N = 4096 forward transform with EIGHT teams: 16 KiB input buffer + 8 KiB output staging per
 // team.  The input arrives by TMA and the next tile is prefetched into the input buffer as soon
@@ -979,165 +558,6 @@ tile_ct_h_kernel(const __grid_constant__ CUtensorMap map_lo, const __grid_consta
     if (j == 0) asm volatile("cp.async.bulk.wait_group.read 0;" ::: "memory");
 }
 
-// Forward partner of poly_gs_kernel: N = 2^13..2^15 in one pass.  The cross-tile stages
-// come FIRST in the CT order (largest strides): once the G tiles of a polynomial have
-// landed, every thread gathers its slice of rows from all G tile buffers, runs stages
-// logn-1 .. 12 in registers and puts the values back; then each team finishes its own
-// tile exactly like tile_ct_kernel.
-template <int LOGG>
-__global__ void __launch_bounds__(kM_Threads, 1)
-poly_ct_kernel(const __grid_constant__ CUtensorMap map_lo, const __grid_constant__ CUtensorMap map_hi,
-               const __grid_constant__ CUtensorMap out_lo, const __grid_constant__ CUtensorMap out_hi,
-               const TileParams prm, const uint2 *__restrict__ tw_flat) {
-    constexpr int G = 1 << LOGG;
-    constexpr int kGroups = kM_Teams / G;
-    constexpr int kSlice = 64 / G;
-    extern __shared__ uint8_t smem_raw[];
-    const uint32_t data_base = (smem_u32(smem_raw) + 1023u) & ~1023u;
-    const uint32_t bar_base = data_base + kM_Teams * kF_PolyBytes;
-    const int tid = threadIdx.x;
-    const int team = __shfl_sync(0xffffffffu, tid >> 6, 0);
-    const int j = tid & 63;
-    const int grp = team >> LOGG, t = team & (G - 1);
-    const uint32_t q = prm.q, two_q = 2u * prm.q, zero = prm.zero;
-
-    if (tid < kM_Teams) mbar_init(bar_base + tid * 8, 1);
-    asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
-    __syncthreads();
-
-    const uint32_t buf = data_base + team * kF_PolyBytes;
-    const uint32_t gbuf = data_base + (grp << LOGG) * kF_PolyBytes;
-    const uint32_t bar = bar_base + team * 8;
-    const uint32_t stride = gridDim.x * kGroups;
-    uint32_t poly = blockIdx.x * kGroups + grp;
-    uint32_t parity = 0;
-    if (j == 0 && poly < prm.batch) {
-        mbar_expect_tx(bar, kF_PolyBytes);
-        tma_load_3d(buf, &map_lo, bar, 0, 0, (int) (poly * G + t));
-        tma_load_3d(buf + kF_PolyBytes / 2, &map_hi, bar, 0, 0, (int) (poly * G + t));
-    }
-    const uint32_t r1_row = buf + j * 128;
-    const uint32_t r1_xor = (j & 7) << 4;
-    const uint32_t col_off = (j >> 5) * (kF_PolyBytes / 2) + (j & 3) * 4;  // column j of a tile buffer
-    const uint32_t r2_col = buf + col_off;
-    const uint32_t r2_chunk = ((j & 31) >> 2) << 4;
-    const uint4 *tw = prm.tw_tile + (size_t) t * kM_TwTile;
-    auto group_sync = [&]() {
-        asm volatile("bar.sync %0, %1;" ::"r"(9 + grp), "n"(G * 64) : "memory");
-    };
-
-    for (; poly < prm.batch; poly += stride) {
-        uint32_t v[64];
-        const int tile = (int) (poly * G + t);
-        mbar_wait(bar, parity);
-        parity ^= 1;
-        group_sync();  // all G tiles of the polynomial are in shared memory
-        // ---- cross-tile stages logn-1 .. 12 on rows t*kSlice .. +kSlice-1 of every tile
-#pragma unroll
-        for (int tt = 0; tt < G; tt++) {
-#pragma unroll
-            for (int ii = 0; ii < kSlice; ii++) {
-                const int i = t * kSlice + ii;  // not a compile-time constant: t is per team
-                v[tt * kSlice + ii] = lds32(gbuf + tt * kF_PolyBytes + col_off + i * 128 +
-                                            (r2_chunk ^ ((i & 7) << 4)));
-            }
-        }
-#pragma unroll
-        for (int mm = 0; mm < LOGG; mm++) {
-            const int m = LOGG - 1 - mm;
-#pragma unroll
-            for (int b2 = 0; b2 < (G >> (m + 1)); b2++) {
-                const uint2 tq = __ldg(tw_flat + (G >> (m + 1)) + b2);
-#pragma unroll
-                for (int e = 0; e < (1 << m); e++) {
-                    const int t0 = (b2 << (m + 1)) + e;
-#pragma unroll
-                    for (int ii = 0; ii < kSlice; ii++) {
-                        if (mm == 0) {
-                            ct_bfly<false>(v[t0 * kSlice + ii], v[(t0 + (1 << m)) * kSlice + ii], tq.x,
-                                           tq.y, q, two_q, zero);
-                        } else {
-                            ct_bfly<true>(v[t0 * kSlice + ii], v[(t0 + (1 << m)) * kSlice + ii], tq.x,
-                                          tq.y, q, two_q, zero);
-                        }
-                    }
-                }
-            }
-        }
-#pragma unroll
-        for (int tt = 0; tt < G; tt++) {
-#pragma unroll
-            for (int ii = 0; ii < kSlice; ii++) {
-                const int i = t * kSlice + ii;
-                asm volatile("st.shared.u32 [%0], %1;" ::"r"(gbuf + tt * kF_PolyBytes + col_off + i * 128 +
-                                                             (r2_chunk ^ ((i & 7) << 4))),
-                             "r"(v[tt * kSlice + ii])
-                             : "memory");
-            }
-        }
-        group_sync();
-        // ---- this team's tile: columns (stages 11..6), exchange, rows (stages 5..0)
-#pragma unroll
-        for (int i = 0; i < 64; i++) {
-            v[i] = lds32(r2_col + i * 128 + (r2_chunk ^ ((i & 7) << 4)));
-        }
-        const uint4 *tw2 = tw + 64;
-        ct_stage_g<5, true>(v, tw2, q, two_q, zero);
-        ct_stage_g<4, true>(v, tw2, q, two_q, zero);
-        ct_stage_g<3, true>(v, tw2, q, two_q, zero);
-        ct_stage_g<2, true>(v, tw2, q, two_q, zero);
-        ct_stage_g<1, true>(v, tw2, q, two_q, zero);
-        ct_stage_g<0, true>(v, tw2, q, two_q, zero);
-#pragma unroll
-        for (int i = 0; i < 64; i++) {
-            asm volatile("st.shared.u32 [%0], %1;" ::"r"(r2_col + i * 128 + (r2_chunk ^ ((i & 7) << 4))),
-                         "r"(v[i])
-                         : "memory");
-        }
-        team_sync(team);
-#pragma unroll
-        for (int c = 0; c < 16; c++) {
-            uint4 x = lds128(r1_row + (c >> 3) * (kF_PolyBytes / 2) + (((c & 7) << 4) ^ r1_xor));
-            v[4 * c + 0] = x.x;
-            v[4 * c + 1] = x.y;
-            v[4 * c + 2] = x.z;
-            v[4 * c + 3] = x.w;
-        }
-        const uint4 *tw1 = tw + j;
-        ct_stage_g<5, true>(v, tw1, q, two_q, zero);
-        ct_stage_g<4, true>(v, tw1, q, two_q, zero);
-        ct_stage_g<3, true>(v, tw1, q, two_q, zero);
-        ct_stage_g<2, true>(v, tw1, q, two_q, zero);
-        ct_stage_g<1, true>(v, tw1, q, two_q, zero);
-        ct_stage_g<0, true>(v, tw1, q, two_q, zero);
-#pragma unroll
-        for (int c = 0; c < 16; c++) {
-            uint32_t o[4];
-#pragma unroll
-            for (int e = 0; e < 4; e++) {
-                uint32_t r = v[4 * c + e];
-                r = min(r - two_q, r);
-                o[e] = min(r - q, r);
-            }
-            sts128(r1_row + (c >> 3) * (kF_PolyBytes / 2) + (((c & 7) << 4) ^ r1_xor), o[0], o[1],
-                   o[2], o[3]);
-        }
-        fence_proxy_async();
-        team_sync(team);
-        const uint32_t next = poly + stride;
-        if (j == 0) {
-            tma_store_3d(&out_lo, buf, 0, 0, tile);
-            tma_store_3d(&out_hi, buf + kF_PolyBytes / 2, 0, 0, tile);
-            tma_store_commit_and_wait_read();
-            if (next < prm.batch) {
-                mbar_expect_tx(bar, kF_PolyBytes);
-                tma_load_3d(buf, &map_lo, bar, 0, 0, (int) (next * G + t));
-                tma_load_3d(buf + kF_PolyBytes / 2, &map_hi, bar, 0, 0, (int) (next * G + t));
-            }
-        }
-    }
-}
-
 // ------------------------------------------------------------------ column pass
 struct ColParams {
     uint32_t logn;
@@ -1258,27 +678,18 @@ int tile_maps(CUtensorMap *lo, CUtensorMap *hi, const int32_t *base, size_t tile
 
 static const RnsConsts kNoRns{};
 constexpr int kM_SmemBytesStaged = kM_SmemBytes + kM_Teams * (kF_PolyBytes / 2) + 1024;
-static bool ct_staged() {   // NTTB200_CT_UNSTAGED=1: the first version (A/B)
-    static const bool on = getenv("NTTB200_CT_UNSTAGED") == nullptr;
-    return on;
-}
 
 int multi_set_attrs() {
     const auto attr = cudaFuncAttributeMaxDynamicSharedMemorySize;
     NTTB200_CUDA(cudaFuncSetAttribute(tile_gs_kernel<false, false>, attr, kM_SmemBytes));
     NTTB200_CUDA(cudaFuncSetAttribute(tile_gs_kernel<true, false>, attr, kM_SmemBytes));
-    NTTB200_CUDA(cudaFuncSetAttribute(tile_gs_kernel<false, true>, attr, kM_SmemBytes));
-    NTTB200_CUDA(cudaFuncSetAttribute(tile_gs_kernel<true, true>, attr, kM_SmemBytes));
-    NTTB200_CUDA(cudaFuncSetAttribute(tile_ct_kernel<false>, attr, kM_SmemBytes));
-    NTTB200_CUDA(cudaFuncSetAttribute(tile_ct_kernel<true>, attr, kM_SmemBytes));
-    NTTB200_CUDA(cudaFuncSetAttribute(tile_ct_kernel<false, false, false, true>, attr, kM_SmemBytesStaged));
-    NTTB200_CUDA(cudaFuncSetAttribute(tile_ct_kernel<true, false, false, true>, attr, kM_SmemBytesStaged));
-    NTTB200_CUDA(cudaFuncSetAttribute(tile_ct_kernel<false, false, false, true, true>, attr, kM_SmemBytesStaged));
-    NTTB200_CUDA(cudaFuncSetAttribute(tile_gs_kernel<false, false, 1>, attr, kM_SmemBytesTw));
+    NTTB200_CUDA(cudaFuncSetAttribute(tile_gs_kernel<false, kRnsTile>, attr, kM_SmemBytes));
+    NTTB200_CUDA(cudaFuncSetAttribute(tile_ct_kernel<kRnsOff>, attr, kM_SmemBytesStaged));
+    NTTB200_CUDA(cudaFuncSetAttribute(tile_ct_kernel<kRnsTile>, attr, kM_SmemBytesStaged));
+    NTTB200_CUDA(cudaFuncSetAttribute(tile_ct_kernel<kRnsOff, true>, attr, kM_SmemBytesStaged));
     NTTB200_CUDA(cudaFuncSetAttribute(tile_gs_kernel<false, false, 2>, attr, kM_SmemBytesTw));
     NTTB200_CUDA(cudaFuncSetAttribute(tile_gs_kernel<true, false, 2>, attr, kM_SmemBytesTw));
-    NTTB200_CUDA(cudaFuncSetAttribute(tile_gs_kernel<false, true, 2>, attr, kM_SmemBytesTw));
-    NTTB200_CUDA(cudaFuncSetAttribute(tile_gs_kernel<true, true, 2>, attr, kM_SmemBytesTw));
+    NTTB200_CUDA(cudaFuncSetAttribute(tile_gs_kernel<false, kRnsTile, 2>, attr, kM_SmemBytesTw));
     NTTB200_CUDA(cudaFuncSetAttribute(tile_gs_kernel<false, kRnsSpan>, attr, kM_SmemBytes));
     NTTB200_CUDA(cudaFuncSetAttribute(tile_gs_kernel<true, kRnsSpan>, attr, kM_SmemBytes));
     NTTB200_CUDA(cudaFuncSetAttribute(tile_gs_kernel<false, kRnsSpan, 2>, attr, kM_SmemBytesTw));
@@ -1287,30 +698,13 @@ int multi_set_attrs() {
     NTTB200_CUDA(cudaFuncSetAttribute(tile_gs_kernel<false, kRnsSpan, 0, false, true>, attr, kM_SmemBytes));
     NTTB200_CUDA(cudaFuncSetAttribute(tile_gs_kernel<false, kRnsTile, 2, false, true>, attr, kM_SmemBytesTw));
     NTTB200_CUDA(cudaFuncSetAttribute(tile_gs_kernel<false, kRnsSpan, 2, false, true>, attr, kM_SmemBytesTw));
-    NTTB200_CUDA(cudaFuncSetAttribute(tile_ct_kernel<kRnsSpan>, attr, kM_SmemBytes));
-    NTTB200_CUDA(cudaFuncSetAttribute(tile_ct_kernel<kRnsSpan, false, false, true>, attr, kM_SmemBytesStaged));
-    NTTB200_CUDA(cudaFuncSetAttribute(tile_gs_kernel<true, false, 1>, attr, kM_SmemBytesTw));
+    NTTB200_CUDA(cudaFuncSetAttribute(tile_ct_kernel<kRnsSpan>, attr, kM_SmemBytesStaged));
     NTTB200_CUDA(cudaFuncSetAttribute(tile_gs_kernel<false, false, 0, true>, attr, kM_SmemBytes));
     NTTB200_CUDA(cudaFuncSetAttribute(tile_gs_kernel<true, false, 0, true>, attr, kM_SmemBytes));
     NTTB200_CUDA(cudaFuncSetAttribute(tile_gs_kernel<false, false, 2, true>, attr, kM_SmemBytesTw));
     NTTB200_CUDA(cudaFuncSetAttribute(tile_gs_kernel<true, false, 2, true>, attr, kM_SmemBytesTw));
-    NTTB200_CUDA(cudaFuncSetAttribute(tile_ct_kernel<false, true>, attr, kM_SmemBytesTw));
     NTTB200_CUDA(cudaFuncSetAttribute(tile_ct_h_kernel<false>, attr, kH_SmemBytes));
     NTTB200_CUDA(cudaFuncSetAttribute(tile_ct_h_kernel<true>, attr, kH_SmemBytes));
-    NTTB200_CUDA(cudaFuncSetAttribute(tile_ct_kernel<false, true, true>, attr, kM_SmemBytesTw));
-    NTTB200_CUDA(cudaFuncSetAttribute(tile_ct_db_kernel<false>, attr, kD_SmemBytes));
-    NTTB200_CUDA(cudaFuncSetAttribute(tile_ct_db_kernel<true>, attr, kD_SmemBytes));
-    NTTB200_CUDA(cudaFuncSetAttribute(tile_ct_db_kernel<false, true>, attr, kD_SmemBytes));
-    NTTB200_CUDA(cudaFuncSetAttribute(tile_ct_db_kernel<true, true>, attr, kD_SmemBytes));
-    NTTB200_CUDA(cudaFuncSetAttribute(poly_ct_kernel<1>, attr, kM_SmemBytes));
-    NTTB200_CUDA(cudaFuncSetAttribute(poly_ct_kernel<2>, attr, kM_SmemBytes));
-    NTTB200_CUDA(cudaFuncSetAttribute(poly_ct_kernel<3>, attr, kM_SmemBytes));
-    NTTB200_CUDA(cudaFuncSetAttribute(poly_gs_kernel<1, false>, attr, kM_SmemBytes));
-    NTTB200_CUDA(cudaFuncSetAttribute(poly_gs_kernel<2, false>, attr, kM_SmemBytes));
-    NTTB200_CUDA(cudaFuncSetAttribute(poly_gs_kernel<3, false>, attr, kM_SmemBytes));
-    NTTB200_CUDA(cudaFuncSetAttribute(poly_gs_kernel<1, true>, attr, kM_SmemBytes));
-    NTTB200_CUDA(cudaFuncSetAttribute(poly_gs_kernel<2, true>, attr, kM_SmemBytes));
-    NTTB200_CUDA(cudaFuncSetAttribute(poly_gs_kernel<3, true>, attr, kM_SmemBytes));
     return NTTB200_OK;
 }
 
@@ -1438,65 +832,14 @@ static int tile_grid(nttb200_plan *p, uint64_t tiles) {
     return (int) (ctas < (uint64_t) p->sm_count ? ctas : (uint64_t) p->sm_count);
 }
 
-template <int LOGG, bool DUAL>
-static void poly_launch_t(int grid, cudaStream_t st, const CUtensorMap &a_lo, const CUtensorMap &a_hi,
-                          const CUtensorMap &b_lo, const CUtensorMap &b_hi, const TileParams &tp,
-                          const uint2 *tw) {
-    poly_gs_kernel<LOGG, DUAL><<<grid, kM_Threads, kM_SmemBytes, st>>>(a_lo, a_hi, b_lo, b_hi, tp, tw);
-}
+// from this batch on, the runs of one tile position are long enough to stage the position's
+// table in shared memory (TWMODE 2)
+constexpr size_t kM_SegTablesMinBatch = 64;
 
-static bool poly_kernel_enabled() {
-    static const bool on = getenv("NTTB200_NO_POLY_KERNEL") == nullptr;
-    return on;
-}
-
-// N = 2^13..2^15 in one pass (poly_gs_kernel).  d_b != nullptr: input = d_in (*) d_b,
-// output scaled by N^-1.
-static int launch_poly_gs(nttb200_plan *p, const int32_t *d_in, const int32_t *d_b, int32_t *d_out,
-                          size_t batch, cudaStream_t st) {
-    const int logg = (int) p->logn - 12;
-    if (logg < 1 || logg > 3 || !poly_kernel_enabled()) return NTTB200_ERR_UNSUPPORTED;
-    const uint64_t tiles = (uint64_t) batch << logg;
-    CUtensorMap a_lo, a_hi, b_lo, b_hi;
-    if (tile_maps(&a_lo, &a_hi, d_in, (size_t) tiles) != NTTB200_OK) return NTTB200_ERR_UNSUPPORTED;
-    TileParams tp = tile_params(p, d_out, batch);
-    if (d_b) {
-        if (tile_maps(&b_lo, &b_hi, d_b, (size_t) tiles) != NTTB200_OK) return NTTB200_ERR_UNSUPPORTED;
-        tp.qinv = inv_mod_2_32(p->q);
-        uint64_t sc = ((uint64_t) p->n_inv << 32) % p->q;
-        tp.scale = (uint32_t) sc;
-        tp.scale_shoup = (uint32_t) ((sc << 32) / p->q);
-    } else {
-        b_lo = a_lo;
-        b_hi = a_hi;
-    }
-    const uint64_t groups = kM_Teams >> logg;
-    uint64_t ctas = (batch + groups - 1) / groups;
-    int grid = (int) (ctas < (uint64_t) p->sm_count ? ctas : (uint64_t) p->sm_count);
-    const bool dual = d_b != nullptr;
-    switch (logg * 2 + (dual ? 1 : 0)) {
-        case 2: poly_launch_t<1, false>(grid, st, a_lo, a_hi, b_lo, b_hi, tp, p->d_tw); break;
-        case 3: poly_launch_t<1, true>(grid, st, a_lo, a_hi, b_lo, b_hi, tp, p->d_tw); break;
-        case 4: poly_launch_t<2, false>(grid, st, a_lo, a_hi, b_lo, b_hi, tp, p->d_tw); break;
-        case 5: poly_launch_t<2, true>(grid, st, a_lo, a_hi, b_lo, b_hi, tp, p->d_tw); break;
-        case 6: poly_launch_t<3, false>(grid, st, a_lo, a_hi, b_lo, b_hi, tp, p->d_tw); break;
-        default: poly_launch_t<3, true>(grid, st, a_lo, a_hi, b_lo, b_hi, tp, p->d_tw); break;
-    }
-    g_launches.fetch_add(1, std::memory_order_relaxed);
-    NTTB200_CUDA(cudaGetLastError());
-    return NTTB200_OK;
-}
-
-// long same-position runs (batched workloads): stage each position's table in shared memory
-static bool seg_tables(size_t batch) {
-    static const bool off = getenv("NTTB200_NO_SEG_TABLES") != nullptr;
-    return !off && batch >= 64;
-}
-
-// d_b == nullptr: plain transform of d_in.  Otherwise the input is d_in (*) d_b and the
-// output is scaled by N^-1 (inverse transform of a negacyclic product).
-static int launch_multi_gs_once(nttb200_plan *p, const int32_t *d_in, const int32_t *d_b,
-                                int32_t *d_out, size_t batch, cudaStream_t st) {
+// Tile pass + column passes.  d_b == nullptr: plain transform of d_in.  Otherwise the input
+// is d_in (*) d_b and the output is scaled by N^-1 (inverse transform of a negacyclic product).
+static int launch_tile_column_gs(nttb200_plan *p, const int32_t *d_in, const int32_t *d_b,
+                                 int32_t *d_out, size_t batch, cudaStream_t st) {
     const uint64_t tiles = (uint64_t) batch * (p->n >> 12);
     CUtensorMap map_lo, map_hi, b_lo, b_hi;
     if (tile_maps(&map_lo, &map_hi, d_in, (size_t) tiles) != NTTB200_OK) {
@@ -1505,6 +848,7 @@ static int launch_multi_gs_once(nttb200_plan *p, const int32_t *d_in, const int3
     TileParams tp = tile_params(p, d_out, batch);
     int grid = tile_grid(p, tiles);
     const bool l4 = use_l4(p) && tp.chunks > 1;
+    const bool seg = batch >= kM_SegTablesMinBatch;
     if (d_b) {
         if (tile_maps(&b_lo, &b_hi, d_b, (size_t) tiles) != NTTB200_OK) return NTTB200_ERR_UNSUPPORTED;
         tp.qinv = inv_mod_2_32(p->q);
@@ -1512,13 +856,10 @@ static int launch_multi_gs_once(nttb200_plan *p, const int32_t *d_in, const int3
         uint64_t sc = ((uint64_t) p->n_inv << 32) % p->q;
         tp.scale = (uint32_t) sc;
         tp.scale_shoup = (uint32_t) ((sc << 32) / p->q);
-        if (tp.chunks == 1) {  // N = 4096: one table for every tile, kept in shared memory
-            tile_gs_kernel<true, false, 1><<<grid, kM_Threads, kM_SmemBytesTw, st>>>(
-                map_lo, map_hi, b_lo, b_hi, tp, kNoRns);
-        } else if (seg_tables(batch) && l4) {
+        if (seg && l4) {
             tile_gs_kernel<true, false, 2, true><<<grid, kM_Threads, kM_SmemBytesTw, st>>>(
                 map_lo, map_hi, b_lo, b_hi, tp, kNoRns);
-        } else if (seg_tables(batch)) {
+        } else if (seg) {
             tile_gs_kernel<true, false, 2><<<grid, kM_Threads, kM_SmemBytesTw, st>>>(
                 map_lo, map_hi, b_lo, b_hi, tp, kNoRns);
         } else if (l4) {
@@ -1528,13 +869,10 @@ static int launch_multi_gs_once(nttb200_plan *p, const int32_t *d_in, const int3
             tile_gs_kernel<true, false><<<grid, kM_Threads, kM_SmemBytes, st>>>(map_lo, map_hi, b_lo,
                                                                                 b_hi, tp, kNoRns);
         }
-    } else if (tp.chunks == 1) {
-        tile_gs_kernel<false, false, 1><<<grid, kM_Threads, kM_SmemBytesTw, st>>>(
-            map_lo, map_hi, map_lo, map_hi, tp, kNoRns);
-    } else if (seg_tables(batch) && l4) {
+    } else if (seg && l4) {
         tile_gs_kernel<false, false, 2, true><<<grid, kM_Threads, kM_SmemBytesTw, st>>>(
             map_lo, map_hi, map_lo, map_hi, tp, kNoRns);
-    } else if (seg_tables(batch)) {
+    } else if (seg) {
         tile_gs_kernel<false, false, 2><<<grid, kM_Threads, kM_SmemBytesTw, st>>>(
             map_lo, map_hi, map_lo, map_hi, tp, kNoRns);
     } else if (l4) {
@@ -1569,36 +907,13 @@ int launch_multi_gs(nttb200_plan *p, const int32_t *d_in, int32_t *d_out, size_t
         ((uintptr_t) d_out & 15u)) {
         return NTTB200_ERR_UNSUPPORTED;
     }
-    // L2 blocking: run the passes over sub-batches small enough that what the tile
-    // pass writes is still in the 126 MB L2 when the column pass reads it, so the
-    // intermediate never costs HBM bandwidth.
-    {
-        int rc = launch_polyc_gs(p, d_in, nullptr, d_out, batch, st);   // opt-in (NTTB200_CLUSTER16)
-        if (rc != NTTB200_ERR_UNSUPPORTED) return rc;
-        rc = launch_tilecol_gs(p, d_in, nullptr, d_out, batch, st);
-        if (rc != NTTB200_ERR_UNSUPPORTED) return rc;
-        rc = launch_polyt_gs(p, d_in, nullptr, d_out, batch, st);
-        if (rc != NTTB200_ERR_UNSUPPORTED) return rc;
-        rc = launch_poly_gs(p, d_in, nullptr, d_out, batch, st);
-        if (rc == NTTB200_OK) p->last_path = "poly_tma_3round";
-        if (rc != NTTB200_ERR_UNSUPPORTED) return rc;
-    }
-    static const long l2_mb = []() {
-        const char *e = getenv("NTTB200_L2_CHUNK_MB");
-        return e ? atol(e) : 0L;  // measured: separate sub-batch launches lose more than L2 hits win
-    }();
-    size_t sub = batch;
-    if (l2_mb > 0) {
-        sub = ((size_t) l2_mb << 20) / ((size_t) p->n * 4);
-        if (sub < 1) sub = 1;
-    }
-    for (size_t b0 = 0; b0 < batch; b0 += sub) {
-        size_t nb = batch - b0 < sub ? batch - b0 : sub;
-        int rc = launch_multi_gs_once(p, d_in + b0 * p->n, nullptr, d_out + b0 * p->n, nb, st);
-        if (rc != NTTB200_OK) return rc;
-    }
-    p->last_path = "tile_tma + column_passes";
-    return NTTB200_OK;
+    int rc = launch_tilecol_gs(p, d_in, nullptr, d_out, batch, st);
+    if (rc != NTTB200_ERR_UNSUPPORTED) return rc;
+    rc = launch_polyt_gs(p, d_in, nullptr, d_out, batch, st);
+    if (rc != NTTB200_ERR_UNSUPPORTED) return rc;
+    rc = launch_tile_column_gs(p, d_in, nullptr, d_out, batch, st);
+    if (rc == NTTB200_OK) p->last_path = "tile_tma + column_passes";
+    return rc;
 }
 
 // Stages [sb, se) of ONE length-N vector (batch 1) with the result scattered to the
@@ -1672,16 +987,11 @@ int launch_multi_gs_dual(nttb200_plan *p, const int32_t *d_a, const int32_t *d_b
         return NTTB200_ERR_UNSUPPORTED;
     }
     if (batch == 0) return NTTB200_OK;
-    int rc = launch_polyc_gs(p, d_a, d_b, d_out, batch, st);   // opt-in (NTTB200_CLUSTER16)
-    if (rc != NTTB200_ERR_UNSUPPORTED) return rc;
-    rc = launch_tilecol_gs(p, d_a, d_b, d_out, batch, st);
+    int rc = launch_tilecol_gs(p, d_a, d_b, d_out, batch, st);
     if (rc != NTTB200_ERR_UNSUPPORTED) return rc;
     rc = launch_polyt_gs(p, d_a, d_b, d_out, batch, st);
     if (rc != NTTB200_ERR_UNSUPPORTED) return rc;
-    rc = launch_poly_gs(p, d_a, d_b, d_out, batch, st);
-    if (rc == NTTB200_OK) p->last_path = "poly_tma_3round_dual";
-    if (rc != NTTB200_ERR_UNSUPPORTED) return rc;
-    rc = launch_multi_gs_once(p, d_a, d_b, d_out, batch, st);
+    rc = launch_tile_column_gs(p, d_a, d_b, d_out, batch, st);
     if (rc == NTTB200_OK) p->last_path = "tile_tma_dual + column_passes";
     return rc;
 }
@@ -1690,59 +1000,25 @@ int launch_multi_gs_dual(nttb200_plan *p, const int32_t *d_a, const int32_t *d_b
 // CT tile pass
 int launch_multi_ct(nttb200_plan *p, const int32_t *d_in, int32_t *d_out, size_t batch,
                     cudaStream_t st) {
-    return launch_multi_ct_mul(p, d_in, nullptr, d_out, batch, st);
-}
-
-// d_mul != nullptr (N = 4096 only): out = CT(d_in) (*) d_mul as a Montgomery product
-// (x*y*2^-32 mod q, canonical) -- the pointwise product fused into the second forward
-// transform of a negacyclic multiplication
-int launch_multi_ct_mul(nttb200_plan *p, const int32_t *d_in, const int32_t *d_mul, int32_t *d_out,
-                        size_t batch, cudaStream_t st) {
-    if (!multi_args_ok(p, d_in, d_out, batch)) return NTTB200_ERR_UNSUPPORTED;
-    if (d_mul && (p->logn != 12 || ((uintptr_t) d_mul & 15u) || !(p->q & 1u))) {
+    // N = 4096 reads table[1..63] from uni_gs, which fused_prepare fills with d_tw_r1
+    if (!multi_args_ok(p, d_in, d_out, batch) || (p->logn == 12 && !p->d_tw_r1)) {
         return NTTB200_ERR_UNSUPPORTED;
     }
     if (batch == 0) return NTTB200_OK;
-    const int logg = (int) p->logn - 12;
-    if (!d_mul) {
-        // (measured and kept out: an 8-team forward kernel that stores each thread's 64
-        // consecutive results as 16 x STG.128 -- 32 lines per warp store -- ran 0.588 ms per
-        // 65,536 tiles against 0.516 ms for the double-buffered TMA-store kernel below)
-        int rc = launch_polyt_ct(p, d_in, d_out, batch, st);
-        if (rc != NTTB200_ERR_UNSUPPORTED) return rc;
-        rc = launch_tilecol_ct(p, d_in, d_out, batch, st);
-        if (rc != NTTB200_ERR_UNSUPPORTED) return rc;
-    }
-    if (logg >= 1 && logg <= 3 && poly_kernel_enabled()) {
-        // N = 2^13..2^15: one pass, cross-tile stages inside the CTA
-        const uint64_t ptiles = (uint64_t) batch << logg;
-        CUtensorMap i_lo, i_hi, o_lo, o_hi;
-        if (tile_maps(&i_lo, &i_hi, d_in, (size_t) ptiles) == NTTB200_OK &&
-            tile_maps(&o_lo, &o_hi, d_out, (size_t) ptiles) == NTTB200_OK) {
-            TileParams tp = tile_params(p, d_out, batch);
-            const uint64_t groups = kM_Teams >> logg;
-            uint64_t ctas = (batch + groups - 1) / groups;
-            int grid = (int) (ctas < (uint64_t) p->sm_count ? ctas : (uint64_t) p->sm_count);
-            if (logg == 1) {
-                poly_ct_kernel<1><<<grid, kM_Threads, kM_SmemBytes, st>>>(i_lo, i_hi, o_lo, o_hi, tp, p->d_tw);
-            } else if (logg == 2) {
-                poly_ct_kernel<2><<<grid, kM_Threads, kM_SmemBytes, st>>>(i_lo, i_hi, o_lo, o_hi, tp, p->d_tw);
-            } else {
-                poly_ct_kernel<3><<<grid, kM_Threads, kM_SmemBytes, st>>>(i_lo, i_hi, o_lo, o_hi, tp, p->d_tw);
-            }
-            g_launches.fetch_add(1, std::memory_order_relaxed);
-            NTTB200_CUDA(cudaGetLastError());
-            p->last_path = "poly_tma_3round_ct";
-            return NTTB200_OK;
-        }
-    }
+    // (measured and kept out: an 8-team forward kernel that stores each thread's 64
+    // consecutive results as 16 x STG.128 -- 32 lines per warp store -- ran 0.588 ms per
+    // 65,536 tiles against 0.516 ms for a double-buffered TMA-store kernel)
+    int rc = launch_polyt_ct(p, d_in, d_out, batch, st);
+    if (rc != NTTB200_ERR_UNSUPPORTED) return rc;
+    rc = launch_tilecol_ct(p, d_in, d_out, batch, st);
+    if (rc != NTTB200_ERR_UNSUPPORTED) return rc;
     const int32_t *src = d_in;
     int rest = (int) p->logn - 12;
     int passes = (rest + 5) / 6;
     int top = (int) p->logn;
     for (int k = 0; k < passes; k++) {
         int take = (rest + (passes - k) - 1) / (passes - k);
-        int rc = column_pass_t<true>(p, src, d_out, batch, top - take, take, st);
+        rc = column_pass_t<true>(p, src, d_out, batch, top - take, take, st);
         if (rc != NTTB200_OK) return rc;
         src = d_out;
         top -= take;
@@ -1755,68 +1031,28 @@ int launch_multi_ct_mul(nttb200_plan *p, const int32_t *d_in, const int32_t *d_m
         return NTTB200_ERR_UNSUPPORTED;
     }
     TileParams tp = tile_params(p, d_out, batch);
-    CUtensorMap mul_lo, mul_hi;
-    if (d_mul) {
-        if (tile_maps(&mul_lo, &mul_hi, d_mul, (size_t) tiles) != NTTB200_OK) return NTTB200_ERR_UNSUPPORTED;
-        tp.qinv = inv_mod_2_32(p->q);
-    }
-    static const bool use_db = getenv("NTTB200_CT_SINGLE_BUFFER") == nullptr;
-    static const int h_mode = []() {    // 0: off, 1: classic butterflies, 2: 4q-lazy where q allows
-        const char *e = getenv("NTTB200_CT_H");
-        return e ? atoi(e) : 2;   // per 65,536 tiles: 0.515 ms (two buffers, six teams), 0.504, 0.487
-    }();
-    if (tp.chunks == 1 && h_mode && !d_mul && p->d_tw_r1) {
+    const bool l4 = use_l4(p);
+    if (tp.chunks == 1) {
+        // per 65,536 tiles: 0.515 ms (two buffers, six teams), 0.504 (tile_ct_h_kernel, classic
+        // butterflies), 0.487 (4q-lazy)
         const int grid = (int) (tiles < (uint64_t) p->sm_count ? tiles : (uint64_t) p->sm_count);
-        if (h_mode == 2 && use_l4(p)) {
+        if (l4) {
             tile_ct_h_kernel<true><<<grid, kM_Threads, kH_SmemBytes, st>>>(in_lo, in_hi, out_lo, out_hi,
                                                                            p->uni_gs, tp);
         } else {
             tile_ct_h_kernel<false><<<grid, kM_Threads, kH_SmemBytes, st>>>(in_lo, in_hi, out_lo, out_hi,
                                                                             p->uni_gs, tp);
         }
-    } else if (tp.chunks == 1 && use_db && p->d_tw_r1) {  // d_tw_r1 set <=> uni_gs holds table[1..63]
-        uint64_t ctas = (tiles + kD_Teams - 1) / kD_Teams;
-        int grid = (int) (ctas < (uint64_t) p->sm_count ? ctas : (uint64_t) p->sm_count);
-        // measured: the 4q-lazy schedule is 4.7 % SLOWER in this kernel (0.542 against 0.518 ms per
-        // 65,536 tiles; its conditional subtractions bunch up at the end of the tile while the six
-        // teams run in lockstep), so it stays opt-in (NTTB200_CT_L4=1)
-        static const bool ct_l4 = getenv("NTTB200_CT_L4") != nullptr;
-        const bool l4 = ct_l4 && use_l4(p);
-        if (d_mul && l4) {
-            tile_ct_db_kernel<true, true><<<grid, kD_Threads, kD_SmemBytes, st>>>(
-                in_lo, in_hi, out_lo, out_hi, mul_lo, mul_hi, p->uni_gs, tp);
-        } else if (d_mul) {
-            tile_ct_db_kernel<true><<<grid, kD_Threads, kD_SmemBytes, st>>>(in_lo, in_hi, out_lo, out_hi,
-                                                                           mul_lo, mul_hi, p->uni_gs, tp);
-        } else if (l4) {
-            tile_ct_db_kernel<false, true><<<grid, kD_Threads, kD_SmemBytes, st>>>(
-                in_lo, in_hi, out_lo, out_hi, in_lo, in_hi, p->uni_gs, tp);
-        } else {
-            tile_ct_db_kernel<false><<<grid, kD_Threads, kD_SmemBytes, st>>>(in_lo, in_hi, out_lo, out_hi,
-                                                                            in_lo, in_hi, p->uni_gs, tp);
-        }
-    } else if (tp.chunks == 1) {
-        if (d_mul) {
-            tile_ct_kernel<false, true, true><<<tile_grid(p, tiles), kM_Threads, kM_SmemBytesTw, st>>>(
-                in_lo, in_hi, out_lo, out_hi, tp, kNoRns, mul_lo, mul_hi);
-        } else {
-            tile_ct_kernel<false, true><<<tile_grid(p, tiles), kM_Threads, kM_SmemBytesTw, st>>>(
-                in_lo, in_hi, out_lo, out_hi, tp, kNoRns, in_lo, in_hi);
-        }
-    } else if (ct_staged() && use_l4(p)) {
-        tile_ct_kernel<false, false, false, true, true><<<tile_grid(p, tiles), kM_Threads, kM_SmemBytesStaged, st>>>(
-            in_lo, in_hi, out_lo, out_hi, tp, kNoRns, in_lo, in_hi);
-    } else if (ct_staged()) {
-        tile_ct_kernel<false, false, false, true><<<tile_grid(p, tiles), kM_Threads, kM_SmemBytesStaged, st>>>(
-            in_lo, in_hi, out_lo, out_hi, tp, kNoRns, in_lo, in_hi);
+    } else if (l4) {
+        tile_ct_kernel<kRnsOff, true><<<tile_grid(p, tiles), kM_Threads, kM_SmemBytesStaged, st>>>(
+            in_lo, in_hi, out_lo, out_hi, tp, kNoRns);
     } else {
-        tile_ct_kernel<false><<<tile_grid(p, tiles), kM_Threads, kM_SmemBytes, st>>>(
-            in_lo, in_hi, out_lo, out_hi, tp, kNoRns, in_lo, in_hi);
+        tile_ct_kernel<kRnsOff><<<tile_grid(p, tiles), kM_Threads, kM_SmemBytesStaged, st>>>(
+            in_lo, in_hi, out_lo, out_hi, tp, kNoRns);
     }
     g_launches.fetch_add(1, std::memory_order_relaxed);
     NTTB200_CUDA(cudaGetLastError());
-    p->last_path = p->logn == 12 ? (d_mul ? "tile_tma_ct_mul" : "tile_tma_ct")
-                                 : "column_passes_ct + tile_tma_ct";
+    p->last_path = p->logn == 12 ? "tile_tma_ct" : "column_passes_ct + tile_tma_ct";
     return NTTB200_OK;
 }
 
@@ -1839,22 +1075,8 @@ static void rns_tile_launch(int kind, int grid, bool seg, const CUtensorMap &a_l
                                                                                tp, rc);
         }
     } else if (kind == 1) {  // CT (b_lo / b_hi: output tensor maps)
-        if (ct_staged()) {
-            tile_ct_kernel<RNS, false, false, true><<<grid, kM_Threads, kM_SmemBytesStaged, st>>>(
-                a_lo, a_hi, b_lo, b_hi, tp, rc, a_lo, a_hi);
-        } else {
-            tile_ct_kernel<RNS><<<grid, kM_Threads, kM_SmemBytes, st>>>(a_lo, a_hi, b_lo, b_hi, tp, rc, a_lo,
-                                                                        a_hi);
-        }
-    } else if (kind == 2) {  // GS of the pointwise product, scaled
-        if (seg) {
-            tile_gs_kernel<true, RNS, 2><<<grid, kM_Threads, kM_SmemBytesTw, st>>>(a_lo, a_hi, b_lo,
-                                                                                  b_hi, tp, rc);
-        } else {
-            tile_gs_kernel<true, RNS><<<grid, kM_Threads, kM_SmemBytes, st>>>(a_lo, a_hi, b_lo, b_hi,
-                                                                              tp, rc);
-        }
-    } else {                 // GS, every output times N^-1
+        tile_ct_kernel<RNS><<<grid, kM_Threads, kM_SmemBytesStaged, st>>>(a_lo, a_hi, b_lo, b_hi, tp, rc);
+    } else if (kind == 3) {  // GS, every output times N^-1
         if (seg) {
             tile_gs_kernel<false, RNS, 2, false, true><<<grid, kM_Threads, kM_SmemBytesTw, st>>>(
                 a_lo, a_hi, a_lo, a_hi, tp, rc);
@@ -1862,17 +1084,25 @@ static void rns_tile_launch(int kind, int grid, bool seg, const CUtensorMap &a_l
             tile_gs_kernel<false, RNS, 0, false, true><<<grid, kM_Threads, kM_SmemBytes, st>>>(
                 a_lo, a_hi, a_lo, a_hi, tp, rc);
         }
+    } else if constexpr (RNS == kRnsSpan) {  // kind 2: GS of the pointwise product, scaled
+        if (seg) {
+            tile_gs_kernel<true, RNS, 2><<<grid, kM_Threads, kM_SmemBytesTw, st>>>(a_lo, a_hi, b_lo,
+                                                                                  b_hi, tp, rc);
+        } else {
+            tile_gs_kernel<true, RNS><<<grid, kM_Threads, kM_SmemBytes, st>>>(a_lo, a_hi, b_lo, b_hi,
+                                                                              tp, rc);
+        }
     }
 }
 
-// kind 0: GS, 1: CT, 2: GS of the pointwise product d_a (*) d_b, scaled by N^-1,
-// 3: GS scaled by N^-1
+// kind 0: GS, 1: CT, 2: GS of the pointwise product d_a (*) d_b, scaled by N^-1 (N > 4096:
+// the N = 4096 product runs as one kernel, kernels_polymul.cu), 3: GS scaled by N^-1
 int rns_launch(const nttb200_rns_plan *rp, int kind, const int32_t *d_a, const int32_t *d_b,
                int32_t *d_out, size_t batch, cudaStream_t st) {
     const uint32_t limbs = rp->limbs, log_g = rp->logn - 12;
     const uint64_t tiles = ((uint64_t) batch * limbs) << log_g;
     if (tiles == 0) return NTTB200_OK;
-    if (limbs > (uint32_t) kM_MaxChannels) return NTTB200_ERR_UNSUPPORTED;
+    if (limbs > (uint32_t) kM_MaxChannels || (kind == 2 && log_g == 0)) return NTTB200_ERR_UNSUPPORTED;
     if (tiles > 0x7fffffffull || batch > 0xffffffffull || ((uintptr_t) d_a & 15u) ||
         ((uintptr_t) d_out & 15u) || (d_b && ((uintptr_t) d_b & 15u))) {
         return NTTB200_ERR_UNSUPPORTED;
@@ -1910,10 +1140,11 @@ int rns_launch(const nttb200_rns_plan *rp, int kind, const int32_t *d_a, const i
         b_lo = a_lo;
         b_hi = a_hi;
     }
+    const bool seg = batch >= kM_SegTablesMinBatch;
     if (log_g == 0) {
-        rns_tile_launch<kRnsTile>(kind, grid, seg_tables(batch), a_lo, a_hi, b_lo, b_hi, tp, rc, st);
+        rns_tile_launch<kRnsTile>(kind, grid, seg, a_lo, a_hi, b_lo, b_hi, tp, rc, st);
     } else {
-        rns_tile_launch<kRnsSpan>(kind, grid, seg_tables(batch), a_lo, a_hi, b_lo, b_hi, tp, rc, st);
+        rns_tile_launch<kRnsSpan>(kind, grid, seg, a_lo, a_hi, b_lo, b_hi, tp, rc, st);
     }
     g_launches.fetch_add(1, std::memory_order_relaxed);
     NTTB200_CUDA(cudaGetLastError());

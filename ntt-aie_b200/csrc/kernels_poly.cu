@@ -1,28 +1,25 @@
 // kernels_poly.cu -- N = 2^13 .. 2^15 in ONE pass with every private twiddle in tensor memory.
 //
-// As poly_gs_kernel / poly_ct_kernel of kernels_multi.cu: the G = N/4096 tiles of a
-// polynomial are taken by G teams of one CTA at the same time, two register rounds per
-// tile (stages 0-11) and a third round through the tile buffers for the log2 G cross-tile
-// stages -- one HBM read + one write per coefficient.  The successor of the reference's
-// tile-local stages followed by cross-tile ntt_1stage calls (src/aie_core.cc:161-361,
-// src/aie2.py:178-295).
+// The G = N/4096 tiles of a polynomial are taken by G teams of one CTA at the same time, two
+// register rounds per tile (stages 0-11) and a third round through the tile buffers for the
+// log2 G cross-tile stages -- one HBM read + one write per coefficient.  The successor of the
+// reference's tile-local stages followed by cross-tile ntt_1stage calls
+// (src/aie_core.cc:161-361, src/aie2.py:178-295).
 //
-// What changed against the first version: there a tile position's 4032 private (w, w')
-// pairs were fetched with LDG.128 on the critical path (G x 33 KiB per CTA does not fit
-// L1 next to 132 KiB of shared memory: 41 % hit rate, long-scoreboard stalls, issue slots
-// 51 % busy -- profiles/r1_secondary_kernels_ncu.txt).  Here each position's table sits in
-// TENSOR MEMORY: 128 columns per table, lanes = threads; positions of equal parity share a
-// lane half, so G = 8 fills exactly the 512 columns.  Round-2 pairs (63 per position) are
-// staged in shared memory, the G-1 cross-tile pairs travel as kernel parameters (constant
-// bank).  After the prologue the kernel touches global memory for data only.
+// Why tensor memory: a first version fetched a tile position's 4032 private (w, w') pairs with
+// LDG.128 on the critical path (G x 33 KiB per CTA does not fit L1 next to 132 KiB of shared
+// memory: 41 % hit rate, long-scoreboard stalls, issue slots 51 % busy --
+// profiles/r1_secondary_kernels_ncu.txt).  Here each position's table sits in TENSOR MEMORY:
+// 128 columns per table, lanes = threads; positions of equal parity share a lane half, so
+// G = 8 fills exactly the 512 columns.  Round-2 pairs (63 per position) are staged in shared
+// memory, the G-1 cross-tile pairs travel as kernel parameters (constant bank).  After the
+// prologue the kernel touches global memory for data only.
 #include <cuda.h>
-#include <stdlib.h>
 
 #include "tile_common.cuh"
 
 namespace nttb200 {
 
-constexpr int kY_SmemBytes = kM_Teams * kF_PolyBytes + 128 + 8 * 512 + 1024;
 // forward kernel: + one 8 KiB output staging slot per team (half a tile, see polyt_ct_kernel)
 constexpr int kY_StageBase = kM_Teams * kF_PolyBytes + 128 + 8 * 512;
 constexpr int kY_SmemBytesCt = ((kY_StageBase + 1023) / 1024) * 1024 + kM_Teams * (kF_PolyBytes / 2) + 1024;
@@ -307,195 +304,6 @@ polyt_gs_kernel(const __grid_constant__ CUtensorMap map_lo, const __grid_constan
     if (warp == 0) tmem_dealloc_512(tmem_base);
 }
 
-// N = 2^16 with the same scheme on a CLUSTER of two CTAs (the alternative to the persistent
-// kernel of kernels_tilecol.cu that SURVEY 7.6 and the round-1 review asked to be measured):
-// the 16 tiles of a polynomial are taken by the 2 x 8 teams of a cluster, CTA rank r holding
-// tiles 8r .. 8r+7 and their twiddle tables; the third round gathers rows 4p .. 4p+3 (p = the
-// team's position 8r + t) of all 16 tile buffers -- eight of them in the partner CTA, read
-// through distributed shared memory (mapa + ld.shared::cluster) -- between two cluster
-// barriers, then runs the four cross-tile stages in registers.
-__device__ __forceinline__ uint32_t cluster_ctarank() {
-    uint32_t r;
-    asm volatile("mov.u32 %0, %%cluster_ctarank;" : "=r"(r));
-    return r;
-}
-__device__ __forceinline__ void cluster_sync_all() {
-    asm volatile("barrier.cluster.arrive.release.aligned;" ::: "memory");
-    asm volatile("barrier.cluster.wait.acquire.aligned;" ::: "memory");
-}
-__device__ __forceinline__ uint32_t mapa_u32(uint32_t addr, uint32_t rank) {
-    uint32_t r;
-    asm volatile("mapa.shared::cluster.u32 %0, %1, %2;" : "=r"(r) : "r"(addr), "r"(rank));
-    return r;
-}
-__device__ __forceinline__ uint32_t lds32_cluster(uint32_t addr) {
-    uint32_t v;
-    asm volatile("ld.shared::cluster.u32 %0, [%1];" : "=r"(v) : "r"(addr) : "memory");
-    return v;
-}
-
-template <bool DUAL, bool L4>
-__global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(kM_Threads, 1)
-polyc_gs_kernel(const __grid_constant__ CUtensorMap map_lo, const __grid_constant__ CUtensorMap map_hi,
-                const __grid_constant__ CUtensorMap map_b_lo,
-                const __grid_constant__ CUtensorMap map_b_hi, const TileParams prm,
-                const __grid_constant__ CrossTw cross) {
-    constexpr int G = 16, kSlice = 4, LOGG = 4;
-    extern __shared__ uint8_t smem_raw[];
-    const uint32_t data_base = (smem_u32(smem_raw) + 1023u) & ~1023u;
-    const uint32_t bar_base = data_base + kM_Teams * kF_PolyBytes;
-    const int tid = threadIdx.x;
-    const int warp = __shfl_sync(0xffffffffu, tid >> 5, 0);
-    const int t = warp >> 1;                       // team = tile of this CTA's half
-    const int j = tid & 63;
-    const uint32_t rank = cluster_ctarank();
-    const int pos = (int) rank * 8 + t;            // tile position inside the polynomial
-    const uint32_t q = prm.q, two_q = 2u * prm.q, four_q = prm.four_q, zero = prm.zero;
-
-    uint32_t tmem_base;
-    const uint32_t lane_base =
-        poly_prologue<8>(prm.tw_tile + (size_t) rank * 8 * kM_TwTile, bar_base, tid, warp, j, tmem_base);
-    const uint32_t tw1 = lane_base + (uint32_t) (t >> 1) * 128u;
-    const Tw16 tw2{bar_base + 128 + (uint32_t) t * 512u};
-
-    const uint32_t buf = data_base + t * kF_PolyBytes;
-    const uint32_t bar = bar_base + t * 8;
-    const uint32_t other_base = mapa_u32(data_base, rank ^ 1u);   // the partner CTA's tile buffers
-    const uint32_t stride = gridDim.x >> 1;
-    uint32_t poly = blockIdx.x >> 1;
-    uint32_t parity = 0;
-    if (j == 0 && poly < prm.batch) {
-        mbar_expect_tx(bar, kF_PolyBytes);
-        tma_load_3d(buf, &map_lo, bar, 0, 0, (int) (poly * G + pos));
-        tma_load_3d(buf + kF_PolyBytes / 2, &map_hi, bar, 0, 0, (int) (poly * G + pos));
-    }
-    const uint32_t r1_row = buf + j * 128;
-    const uint32_t r1_xor = (j & 7) << 4;
-    const uint32_t r2_col = buf + (j >> 5) * (kF_PolyBytes / 2) + (j & 3) * 4;
-    const uint32_t r2_chunk = ((j & 31) >> 2) << 4;
-    cluster_sync_all();   // both CTAs are resident and their barriers initialised
-
-    for (; poly < prm.batch; poly += stride) {
-        uint32_t v[64];
-        const int tile = (int) (poly * G + pos);
-        mbar_wait(bar, parity);
-        parity ^= 1;
-#pragma unroll
-        for (int c = 0; c < 16; c++) {
-            uint4 x = lds128(r1_row + (c >> 3) * (kF_PolyBytes / 2) + (((c & 7) << 4) ^ r1_xor));
-            v[4 * c + 0] = x.x;
-            v[4 * c + 1] = x.y;
-            v[4 * c + 2] = x.z;
-            v[4 * c + 3] = x.w;
-        }
-        if (DUAL) {
-            team_sync(t);
-            if (j == 0) {
-                mbar_expect_tx(bar, kF_PolyBytes);
-                tma_load_3d(buf, &map_b_lo, bar, 0, 0, tile);
-                tma_load_3d(buf + kF_PolyBytes / 2, &map_b_hi, bar, 0, 0, tile);
-            }
-            mbar_wait(bar, parity);
-            parity ^= 1;
-#pragma unroll
-            for (int c = 0; c < 16; c++) {
-                uint4 x = lds128(r1_row + (c >> 3) * (kF_PolyBytes / 2) + (((c & 7) << 4) ^ r1_xor));
-                const uint32_t bb[4] = {x.x, x.y, x.z, x.w};
-#pragma unroll
-                for (int e = 0; e < 4; e++) {
-                    uint64_t prod = (uint64_t) v[4 * c + e] * bb[e];
-                    uint32_t m = (uint32_t) prod * prm.qinv;
-                    v[4 * c + e] = (uint32_t) (prod >> 32) - __umulhi(m, q) + q;
-                }
-            }
-        }
-        if (L4) {
-            gs_round_tmem_l4<(DUAL ? 2 : 1)>(v, tw1, q, two_q, four_q, zero);
-        } else {
-            gs_round_tmem<DUAL>(v, tw1, q, two_q, zero);
-        }
-#pragma unroll
-        for (int c = 0; c < 16; c++) {
-            sts128(r1_row + (c >> 3) * (kF_PolyBytes / 2) + (((c & 7) << 4) ^ r1_xor), v[4 * c],
-                   v[4 * c + 1], v[4 * c + 2], v[4 * c + 3]);
-        }
-        team_sync(t);
-#pragma unroll
-        for (int i = 0; i < 64; i++) {
-            v[i] = lds32(r2_col + i * 128 + (r2_chunk ^ ((i & 7) << 4)));
-        }
-        team_sync(t);
-        if (L4) {
-            gs_round_l4<4>(v, tw2, q, two_q, four_q, zero);
-        } else {
-            gs_round<true>(v, tw2, q, two_q, zero);
-        }
-        // ---- round 3 across the cluster
-#pragma unroll
-        for (int i = 0; i < 64; i++) {
-            asm volatile("st.shared.u32 [%0], %1;" ::"r"(buf + (i * 64 + j) * 4), "r"(v[i]) : "memory");
-        }
-        cluster_sync_all();
-        uint32_t w[64];
-#pragma unroll
-        for (int tt = 0; tt < G; tt++) {
-            const bool mine = (uint32_t) (tt >> 3) == rank;   // warp-uniform
-#pragma unroll
-            for (int ii = 0; ii < kSlice; ii++) {
-                const uint32_t off = (uint32_t) (tt & 7) * kF_PolyBytes + (((pos * kSlice + ii) * 64 + j) << 2);
-                w[tt * kSlice + ii] = mine ? lds32(data_base + off) : lds32_cluster(other_base + off);
-            }
-        }
-        fence_proxy_async();
-        cluster_sync_all();
-        const uint32_t next = poly + stride;
-        if (j == 0 && next < prm.batch) {
-            mbar_expect_tx(bar, kF_PolyBytes);
-            tma_load_3d(buf, &map_lo, bar, 0, 0, (int) (next * G + pos));
-            tma_load_3d(buf + kF_PolyBytes / 2, &map_hi, bar, 0, 0, (int) (next * G + pos));
-        }
-#pragma unroll
-        for (int m = 0; m < LOGG; m++) {
-#pragma unroll
-            for (int b2 = 0; b2 < (G >> (m + 1)); b2++) {
-                const uint32_t cw = cross.w[(G >> (m + 1)) + b2], cwp = cross.wp[(G >> (m + 1)) + b2];
-#pragma unroll
-                for (int e = 0; e < (1 << m); e++) {
-                    const int t0 = (b2 << (m + 1)) + e;
-#pragma unroll
-                    for (int ii = 0; ii < kSlice; ii++) {
-                        if (L4) {
-                            gs_bfly_l4(l4_bound(m, e, 4), w[t0 * kSlice + ii], w[(t0 + (1 << m)) * kSlice + ii],
-                                       cw, cwp, q, two_q, four_q, zero);
-                        } else {
-                            gs_bfly<true>(w[t0 * kSlice + ii], w[(t0 + (1 << m)) * kSlice + ii], cw, cwp, q,
-                                          two_q, zero);
-                        }
-                    }
-                }
-            }
-        }
-        uint32_t *dst = prm.out + ((size_t) poly << 16) + j + 64 * (pos * kSlice);
-#pragma unroll
-        for (int tt = 0; tt < G; tt++) {
-#pragma unroll
-            for (int ii = 0; ii < kSlice; ii++) {
-                uint32_t r = w[tt * kSlice + ii];
-                if (DUAL) {
-                    r = shoup_mul_lazy(r, prm.scale, prm.scale_shoup, q);
-                } else if (L4 && !((tt >> (LOGG - 1)) & 1)) {
-                    r = min(r - two_q, r);
-                }
-                dst[tt * 4096 + ii * 64] = min(r - q, r);
-            }
-        }
-    }
-    cluster_sync_all();   // nobody leaves while its partner may still read its buffers
-    tmem_fence_before_sync();
-    __syncthreads();
-    if (warp == 0) tmem_dealloc_512(tmem_base);
-}
-
 // Forward partner: the cross-tile stages come FIRST in the CT order (largest strides),
 // then every team finishes its own tile (columns, exchange, rows) and the rows leave
 // through a TMA store -- in two halves through an 8 KiB staging slot, like tile_ct_h_kernel
@@ -706,22 +514,10 @@ static int polyt_attrs() {
 }
 
 int polyt_prepare() {
-    {
-        const auto attr = cudaFuncAttributeMaxDynamicSharedMemorySize;
-        NTTB200_CUDA(cudaFuncSetAttribute(polyc_gs_kernel<false, false>, attr, kY_SmemBytes));
-        NTTB200_CUDA(cudaFuncSetAttribute(polyc_gs_kernel<false, true>, attr, kY_SmemBytes));
-        NTTB200_CUDA(cudaFuncSetAttribute(polyc_gs_kernel<true, false>, attr, kY_SmemBytes));
-        NTTB200_CUDA(cudaFuncSetAttribute(polyc_gs_kernel<true, true>, attr, kY_SmemBytes));
-    }
     int rc = polyt_attrs<1>();
     if (rc == NTTB200_OK) rc = polyt_attrs<2>();
     if (rc == NTTB200_OK) rc = polyt_attrs<3>();
     return rc;
-}
-
-static bool polyt_enabled() {
-    static const bool on = getenv("NTTB200_POLY_NO_TMEM") == nullptr;
-    return on;
 }
 
 template <int LOGG, bool DUAL>
@@ -752,7 +548,7 @@ static void polyt_ct_launch(int grid, cudaStream_t st, const CUtensorMap &i_lo, 
 int launch_polyt_gs(nttb200_plan *p, const int32_t *d_in, const int32_t *d_b, int32_t *d_out,
                     size_t batch, cudaStream_t st) {
     const int logg = (int) p->logn - 12;
-    if (logg < 1 || logg > 3 || !p->d_tw_tile || !polyt_enabled()) return NTTB200_ERR_UNSUPPORTED;
+    if (logg < 1 || logg > 3 || !p->d_tw_tile) return NTTB200_ERR_UNSUPPORTED;
     const uint64_t tiles = (uint64_t) batch << logg;
     if (tiles > 0x7fffffffull) return NTTB200_ERR_UNSUPPORTED;
     CUtensorMap a_lo, a_hi, b_lo, b_hi;
@@ -794,57 +590,10 @@ int launch_polyt_gs(nttb200_plan *p, const int32_t *d_in, const int32_t *d_b, in
     return NTTB200_OK;
 }
 
-// N = 2^16 on clusters of two CTAs (opt-in: NTTB200_CLUSTER16=1; the persistent tile/column
-// kernel is the default -- see the measurements in DESIGN.md 3.3)
-int launch_polyc_gs(nttb200_plan *p, const int32_t *d_in, const int32_t *d_b, int32_t *d_out,
-                    size_t batch, cudaStream_t st) {
-    static const bool on = getenv("NTTB200_CLUSTER16") != nullptr;
-    if (!on || p->logn != 16 || !p->d_tw_tile) return NTTB200_ERR_UNSUPPORTED;
-    const uint64_t tiles = (uint64_t) batch << 4;
-    if (batch == 0 || tiles > 0x7fffffffull) return NTTB200_ERR_UNSUPPORTED;
-    CUtensorMap a_lo, a_hi, b_lo, b_hi;
-    if (tile_maps(&a_lo, &a_hi, d_in, (size_t) tiles) != NTTB200_OK) return NTTB200_ERR_UNSUPPORTED;
-    TileParams tp;
-    tp.out = reinterpret_cast<uint32_t *>(d_out);
-    tp.tw_tile = p->d_tw_tile;
-    tp.batch = (uint32_t) batch;
-    tp.chunks = 16;
-    tp.q = p->q;
-    tp.zero = 0;
-    tp.qinv = tp.scale = tp.scale_shoup = 0;
-    tp.four_q = 4u * p->q;
-    if (d_b) {
-        if (tile_maps(&b_lo, &b_hi, d_b, (size_t) tiles) != NTTB200_OK) return NTTB200_ERR_UNSUPPORTED;
-        tp.qinv = inv_mod_2_32(p->q);
-        const uint64_t sc = ((uint64_t) p->n_inv << 32) % p->q;
-        tp.scale = (uint32_t) sc;
-        tp.scale_shoup = (uint32_t) ((sc << 32) / p->q);
-    } else {
-        b_lo = a_lo;
-        b_hi = a_hi;
-    }
-    const uint64_t max_clusters = (uint64_t) p->sm_count / 2;
-    const int grid = 2 * (int) (batch < max_clusters ? batch : max_clusters);
-    const bool l4 = use_l4(p);
-    if (d_b && l4) {
-        polyc_gs_kernel<true, true><<<grid, kM_Threads, kY_SmemBytes, st>>>(a_lo, a_hi, b_lo, b_hi, tp, p->cross_tw);
-    } else if (d_b) {
-        polyc_gs_kernel<true, false><<<grid, kM_Threads, kY_SmemBytes, st>>>(a_lo, a_hi, b_lo, b_hi, tp, p->cross_tw);
-    } else if (l4) {
-        polyc_gs_kernel<false, true><<<grid, kM_Threads, kY_SmemBytes, st>>>(a_lo, a_hi, b_lo, b_hi, tp, p->cross_tw);
-    } else {
-        polyc_gs_kernel<false, false><<<grid, kM_Threads, kY_SmemBytes, st>>>(a_lo, a_hi, b_lo, b_hi, tp, p->cross_tw);
-    }
-    g_launches.fetch_add(1, std::memory_order_relaxed);
-    NTTB200_CUDA(cudaGetLastError());
-    p->last_path = d_b ? "poly_cluster2_dual" : "poly_cluster2";
-    return NTTB200_OK;
-}
-
 int launch_polyt_ct(nttb200_plan *p, const int32_t *d_in, int32_t *d_out, size_t batch,
                     cudaStream_t st) {
     const int logg = (int) p->logn - 12;
-    if (logg < 1 || logg > 3 || !p->d_tw_tile || !polyt_enabled()) return NTTB200_ERR_UNSUPPORTED;
+    if (logg < 1 || logg > 3 || !p->d_tw_tile) return NTTB200_ERR_UNSUPPORTED;
     const uint64_t tiles = (uint64_t) batch << logg;
     if (tiles > 0x7fffffffull) return NTTB200_ERR_UNSUPPORTED;
     CUtensorMap i_lo, i_hi, o_lo, o_hi;

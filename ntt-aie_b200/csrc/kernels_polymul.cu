@@ -26,7 +26,6 @@
 // Reference counterpart: none (the reference has only the forward network,
 // src/test.cpp:34-60); the networks are nttb200_ct_batch / nttb200_gs_batch, bit for bit.
 #include <cuda.h>
-#include <stdlib.h>
 
 #include "tile_common.cuh"
 
@@ -105,11 +104,12 @@ __device__ __forceinline__ void pm_gs_uniform_l4(uint32_t (&v)[64], const Unifor
 // LOCKSTEP: the loop body is ~90 KB of straight-line code, twice the instruction-cache reach,
 // and 16 warps streaming it at their own pace stall on instruction fetch (ncu: no_instruction
 // 0.88 stall cycles per issue).  Widening the team barriers makes warps run in step and share
-// every fetch: 0 = team (64 threads), 1 = the two teams that share a pair of schedulers
-// (t, t^2), 2 = the four teams of a scheduler pair (t & 1), 3 = the whole CTA.  Modes > 0 need
-// batch % 8 == 0 so that all teams of a CTA have the same trip count.
-// L4: 0 classic butterflies, 1 the inverse (GS) half 4q-lazy, 2 both halves.
-template <int LOCKSTEP, int L4 = 0>
+// every fetch: the barriers span the two teams that share a pair of schedulers (t, t^2)
+// instead of one team.  Measured per 16,384 products: team 0.458 ms, team pair 0.417, the four
+// teams of a scheduler pair 0.417, the whole CTA 0.423.  Needs batch % 8 == 0 so that all teams
+// of a CTA have the same trip count.
+// L4 (q < 2^29): 4q-lazy butterflies in both halves.
+template <bool LOCKSTEP, bool L4>
 __global__ void __launch_bounds__(kP_Threads, 1)
 polymul4096_kernel(const __grid_constant__ CUtensorMap a_lo, const __grid_constant__ CUtensorMap a_hi,
                    const __grid_constant__ CUtensorMap b_lo, const __grid_constant__ CUtensorMap b_hi,
@@ -124,7 +124,7 @@ polymul4096_kernel(const __grid_constant__ CUtensorMap a_lo, const __grid_consta
     const int team = warp >> 1;   // warp-uniform for the compiler (see kernels_fused.cu)
     const int j = tid & 63;
     const uint32_t q = prm.q, two_q = 2u * prm.q, four_q = prm.four_q, zero = prm.zero;
-    constexpr int kBCol = ct_l4_out_n(1, 6), kBRow = ct_l4_out_n(kBCol, 6);   // forward bounds when L4 == 2
+    constexpr int kBCol = ct_l4_out_n(1, 6), kBRow = ct_l4_out_n(kBCol, 6);   // forward bounds when L4
 
     if (warp == 0) tmem_alloc_512(tmem_slot);
     if (tid < kP_Teams) mbar_init(bar_base + tid * 8, 1);
@@ -161,13 +161,9 @@ polymul4096_kernel(const __grid_constant__ CUtensorMap a_lo, const __grid_consta
     const uint32_t r1_xor = (j & 7) << 4;
     const uint32_t r2_col = buf + (j >> 5) * (kF_PolyBytes / 2) + (j & 3) * 4;
     const uint32_t r2_chunk = ((j & 31) >> 2) << 4;
-    const int pair_id = 9 + ((team & 1) | ((team >> 2) << 1)), group_id = 13 + (team & 1);
+    const int pair_id = 9 + ((team & 1) | ((team >> 2) << 1));
     auto sync = [&]() {
-        if (LOCKSTEP == 3) {
-            __syncthreads();
-        } else if (LOCKSTEP == 2) {
-            asm volatile("bar.sync %0, %1;" ::"r"(group_id), "n"(256) : "memory");
-        } else if (LOCKSTEP == 1) {
+        if (LOCKSTEP) {
             asm volatile("bar.sync %0, %1;" ::"r"(pair_id), "n"(128) : "memory");
         } else {
             team_sync(team);
@@ -185,7 +181,7 @@ polymul4096_kernel(const __grid_constant__ CUtensorMap a_lo, const __grid_consta
             for (int i = 0; i < 64; i++) {
                 v[i] = lds32(r2_col + i * 128 + (r2_chunk ^ ((i & 7) << 4)));
             }
-            if (L4 == 2) {
+            if (L4) {
                 ct_round_uniform_l4<1>(v, uni_fwd, q, two_q, four_q, zero);
             } else {
                 pm_ct_uniform<5, false>(v, uni_fwd, q, two_q, zero);
@@ -222,7 +218,7 @@ polymul4096_kernel(const __grid_constant__ CUtensorMap a_lo, const __grid_consta
                 }
             }
             // ---- rows: CT stages 5..0, private twiddles from tensor memory
-            if (L4 == 2) {
+            if (L4) {
                 ct_round_tmem_l4<kBCol>(v, tw_fwd, q, two_q, four_q, zero);
             } else {
                 ct_round_tmem<true>(v, tw_fwd, q, two_q, zero);
@@ -231,7 +227,7 @@ polymul4096_kernel(const __grid_constant__ CUtensorMap a_lo, const __grid_consta
                 // a^ canonical, parked in this warp's 64 TMEM columns
 #pragma unroll
                 for (int i = 0; i < 64; i++) {
-                    if (L4 == 2) {
+                    if (L4) {
                         v[i] = canon_l4(kBRow, v[i], q, two_q, four_q);
                     } else {
                         uint32_t r = min(v[i] - two_q, v[i]);
@@ -315,14 +311,10 @@ int tile_maps_strided(CUtensorMap *lo, CUtensorMap *hi, const int32_t *base, siz
 
 int polymul_prepare() {
     const auto attr = cudaFuncAttributeMaxDynamicSharedMemorySize;
-    NTTB200_CUDA(cudaFuncSetAttribute(polymul4096_kernel<0>, attr, kP_SmemBytes));
-    NTTB200_CUDA(cudaFuncSetAttribute(polymul4096_kernel<1>, attr, kP_SmemBytes));
-    NTTB200_CUDA(cudaFuncSetAttribute(polymul4096_kernel<2>, attr, kP_SmemBytes));
-    NTTB200_CUDA(cudaFuncSetAttribute(polymul4096_kernel<3>, attr, kP_SmemBytes));
-    NTTB200_CUDA(cudaFuncSetAttribute(polymul4096_kernel<0, 1>, attr, kP_SmemBytes));
-    NTTB200_CUDA(cudaFuncSetAttribute(polymul4096_kernel<1, 1>, attr, kP_SmemBytes));
-    NTTB200_CUDA(cudaFuncSetAttribute(polymul4096_kernel<0, 2>, attr, kP_SmemBytes));
-    NTTB200_CUDA(cudaFuncSetAttribute(polymul4096_kernel<1, 2>, attr, kP_SmemBytes));
+    NTTB200_CUDA(cudaFuncSetAttribute(polymul4096_kernel<false, false>, attr, kP_SmemBytes));
+    NTTB200_CUDA(cudaFuncSetAttribute(polymul4096_kernel<true, false>, attr, kP_SmemBytes));
+    NTTB200_CUDA(cudaFuncSetAttribute(polymul4096_kernel<false, true>, attr, kP_SmemBytes));
+    NTTB200_CUDA(cudaFuncSetAttribute(polymul4096_kernel<true, true>, attr, kP_SmemBytes));
     return NTTB200_OK;
 }
 
@@ -366,52 +358,21 @@ int launch_polymul4096_strided(nttb200_plan *fwd, nttb200_plan *inv, const int32
     prm.out_words = tile_mul * 4096u;
     const uint64_t ctas = (batch + kP_Teams - 1) / kP_Teams;
     const int grid = (int) (ctas < (uint64_t) fwd->sm_count ? ctas : (uint64_t) fwd->sm_count);
-    static const int lockstep = []() {
-        const char *e = getenv("NTTB200_POLYMUL_LOCKSTEP");
-        return e ? atoi(e) : 1;  // measured: 0 0.458 ms, 1 0.417, 2 0.417, 3 0.423 per 16,384 products
-    }();
-    int mode = batch % kP_Teams == 0 ? lockstep : 0;
-    static const int l4_level = []() {
-        const char *e = getenv("NTTB200_POLYMUL_L4");
-        return e ? atoi(e) : 2;
-    }();
-    const int l4 = use_l4(fwd) ? l4_level : 0;
-    if (l4 && mode > 1) mode = 1;
-    switch (l4 ? 4 + (l4 - 1) * 2 + mode : mode) {
-        case 4:
-            polymul4096_kernel<0, 1><<<grid, kP_Threads, kP_SmemBytes, st>>>(a_lo, a_hi, b_lo, b_hi,
-                                                                             fwd->uni_gs, inv->uni_gs, prm);
-            break;
-        case 5:
-            polymul4096_kernel<1, 1><<<grid, kP_Threads, kP_SmemBytes, st>>>(a_lo, a_hi, b_lo, b_hi,
-                                                                             fwd->uni_gs, inv->uni_gs, prm);
-            break;
-        case 6:
-            polymul4096_kernel<0, 2><<<grid, kP_Threads, kP_SmemBytes, st>>>(a_lo, a_hi, b_lo, b_hi,
-                                                                             fwd->uni_gs, inv->uni_gs, prm);
-            break;
-        case 7:
-            polymul4096_kernel<1, 2><<<grid, kP_Threads, kP_SmemBytes, st>>>(a_lo, a_hi, b_lo, b_hi,
-                                                                             fwd->uni_gs, inv->uni_gs, prm);
-            break;
-        case 1:
-            polymul4096_kernel<1><<<grid, kP_Threads, kP_SmemBytes, st>>>(a_lo, a_hi, b_lo, b_hi,
-                                                                          fwd->uni_gs, inv->uni_gs, prm);
-            break;
-        case 2:
-            polymul4096_kernel<2><<<grid, kP_Threads, kP_SmemBytes, st>>>(a_lo, a_hi, b_lo, b_hi,
-                                                                          fwd->uni_gs, inv->uni_gs, prm);
-            break;
-        case 3:
-            polymul4096_kernel<3><<<grid, kP_Threads, kP_SmemBytes, st>>>(a_lo, a_hi, b_lo, b_hi,
-                                                                          fwd->uni_gs, inv->uni_gs, prm);
-            break;
-        default:
-            polymul4096_kernel<0><<<grid, kP_Threads, kP_SmemBytes, st>>>(a_lo, a_hi, b_lo, b_hi,
-                                                                          fwd->uni_gs, inv->uni_gs, prm);
-            break;
+    const bool lockstep = batch % kP_Teams == 0;
+    if (lockstep && use_l4(fwd)) {
+        polymul4096_kernel<true, true><<<grid, kP_Threads, kP_SmemBytes, st>>>(a_lo, a_hi, b_lo, b_hi,
+                                                                               fwd->uni_gs, inv->uni_gs, prm);
+    } else if (lockstep) {
+        polymul4096_kernel<true, false><<<grid, kP_Threads, kP_SmemBytes, st>>>(a_lo, a_hi, b_lo, b_hi,
+                                                                                fwd->uni_gs, inv->uni_gs, prm);
+    } else if (use_l4(fwd)) {
+        polymul4096_kernel<false, true><<<grid, kP_Threads, kP_SmemBytes, st>>>(a_lo, a_hi, b_lo, b_hi,
+                                                                                fwd->uni_gs, inv->uni_gs, prm);
+    } else {
+        polymul4096_kernel<false, false><<<grid, kP_Threads, kP_SmemBytes, st>>>(a_lo, a_hi, b_lo, b_hi,
+                                                                                 fwd->uni_gs, inv->uni_gs, prm);
     }
-    inv->last_path = mode ? "polymul4096_one_kernel_tmem_lockstep" : "polymul4096_one_kernel_tmem";
+    inv->last_path = lockstep ? "polymul4096_one_kernel_tmem_lockstep" : "polymul4096_one_kernel_tmem";
     g_launches.fetch_add(1, std::memory_order_relaxed);
     NTTB200_CUDA(cudaGetLastError());
     return NTTB200_OK;

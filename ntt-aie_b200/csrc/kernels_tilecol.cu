@@ -1,4 +1,4 @@
-// kernels_tilecol.cu -- N = 2^13 .. 2^16 as ONE persistent kernel whose teams are never in
+// kernels_tilecol.cu -- N = 2^16 as ONE persistent kernel whose teams are never in
 // lock step: tile items and column items, ordered by counters, intermediate kept in L2.
 //
 // The reference runs a transform as tile-local stages followed by cross-tile stages, with
@@ -25,7 +25,6 @@
 // Forward (Cooley-Tukey) partner: the same two item kinds in the opposite order (C-items
 // read the input, T-items finish the tiles: columns, exchange, rows, TMA store).
 #include <cuda.h>
-#include <stdlib.h>
 
 #include "tile_common.cuh"
 
@@ -89,12 +88,13 @@ __device__ __forceinline__ void wait_counter(const uint32_t *ctr, uint32_t targe
 // L4 (q < 2^29): 4q-lazy butterflies; the intermediate between the two item kinds is then
 // left LAZY as well (values below 4q), so a T-item stores its registers as they are and the
 // C-item's first stage does the one conditional subtraction its sums need.
-template <int LOGG, bool DUAL, bool L4>
+template <bool DUAL, bool L4>
 __global__ void __launch_bounds__(kM_Threads, 1)
 tilecol_gs_kernel(const __grid_constant__ CUtensorMap map_lo, const __grid_constant__ CUtensorMap map_hi,
                   const __grid_constant__ CUtensorMap map_b_lo,
                   const __grid_constant__ CUtensorMap map_b_hi, const TileColParams prm,
                   const __grid_constant__ CrossTw cross) {
+    constexpr int LOGG = 4;                // N = 2^16
     constexpr int G = 1 << LOGG;
     constexpr int H = G > 8 ? 2 : 1;       // CTA classes: 8 position tables fit one CTA's TMEM
     constexpr int K = G / (2 * H);         // positions per (CTA class, team parity)
@@ -635,48 +635,27 @@ tilecol_ct_kernel(const uint32_t *__restrict__ in, const __grid_constant__ CUten
 // --------------------------------------------------------------------- host side
 int tile_maps(CUtensorMap *lo, CUtensorMap *hi, const int32_t *base, size_t tiles);  // kernels_fused.cu
 
-template <int LOGG>
-static int tilecol_attrs() {
+int tilecol_prepare() {
     const auto attr = cudaFuncAttributeMaxDynamicSharedMemorySize;
-    NTTB200_CUDA(cudaFuncSetAttribute(tilecol_gs_kernel<LOGG, false, false>, attr, kTC_SmemBytes));
-    NTTB200_CUDA(cudaFuncSetAttribute(tilecol_gs_kernel<LOGG, true, false>, attr, kTC_SmemBytes));
-    NTTB200_CUDA(cudaFuncSetAttribute(tilecol_gs_kernel<LOGG, false, true>, attr, kTC_SmemBytes));
-    NTTB200_CUDA(cudaFuncSetAttribute(tilecol_gs_kernel<LOGG, true, true>, attr, kTC_SmemBytes));
+    NTTB200_CUDA(cudaFuncSetAttribute(tilecol_ct_kernel<false>, attr, kTC_SmemBytesCt));
+    NTTB200_CUDA(cudaFuncSetAttribute(tilecol_ct_kernel<true>, attr, kTC_SmemBytesCt));
+    NTTB200_CUDA(cudaFuncSetAttribute(tilecol_gs_kernel<false, false>, attr, kTC_SmemBytes));
+    NTTB200_CUDA(cudaFuncSetAttribute(tilecol_gs_kernel<true, false>, attr, kTC_SmemBytes));
+    NTTB200_CUDA(cudaFuncSetAttribute(tilecol_gs_kernel<false, true>, attr, kTC_SmemBytes));
+    NTTB200_CUDA(cudaFuncSetAttribute(tilecol_gs_kernel<true, true>, attr, kTC_SmemBytes));
     return NTTB200_OK;
 }
 
-int tilecol_prepare() {
-    {
-        const auto attr = cudaFuncAttributeMaxDynamicSharedMemorySize;
-        NTTB200_CUDA(cudaFuncSetAttribute(tilecol_ct_kernel<false>, attr, kTC_SmemBytesCt));
-        NTTB200_CUDA(cudaFuncSetAttribute(tilecol_ct_kernel<true>, attr, kTC_SmemBytesCt));
-    }
-    int rc = tilecol_attrs<1>();
-    if (rc == NTTB200_OK) rc = tilecol_attrs<2>();
-    if (rc == NTTB200_OK) rc = tilecol_attrs<3>();
-    if (rc == NTTB200_OK) rc = tilecol_attrs<4>();
-    return rc;
-}
-
-// which transform lengths take this kernel: 16 by default -- measured at 2^28 coefficients:
-// 0.439 of the HBM roofline against 0.403 for the two passes; for N = 2^13..2^15 the
-// one-CTA-per-polynomial kernels of kernels_poly.cu are faster (0.50/0.49/0.42 against
-// 0.42/0.41/0.38).  NTTB200_TILECOL_LOGN="13,14,15,16" overrides (empty string = none).
-static bool tilecol_enabled(uint32_t logn) {
-    static const uint32_t mask = []() {
-        const char *e = getenv("NTTB200_TILECOL_LOGN");
-        if (!e) return 1u << 16;
-        uint32_t m = 0;
-        for (const char *c = e; *c;) {
-            int v = atoi(c);
-            if (v >= 13 && v <= 16) m |= 1u << v;
-            while (*c && *c != ',') c++;
-            if (*c == ',') c++;
-        }
-        return m;
-    }();
-    return (mask >> logn) & 1u;
-}
+// Only N = 2^16 takes these kernels -- measured at 2^28 coefficients: 0.439 of the HBM roofline
+// against 0.403 for the two passes; for N = 2^13..2^15 the one-CTA-per-polynomial kernels of
+// kernels_poly.cu are faster (0.50/0.49/0.42 against 0.42/0.41/0.38).
+// Below ~14 tiles per team the prologue, the lag and the drain phase cost more than the saved
+// HBM pass (measured at N = 2^16: 512 polynomials 0.199 ms against 0.12 ms for the two passes,
+// 1024 polynomials 0.214 against 0.227, 4096 polynomials 0.748 against 0.814).
+constexpr uint64_t kTC_MinTilesPerTeam = 12;
+// in flight at any time: one tile per team; the items that wait on a counter trail by this
+// share of that, in percent
+constexpr uint64_t kTC_LagPct = 150;
 
 // The error word of the plan: mapped host memory, so the host can read it without a
 // synchronisation.  Checked (and cleared) at the start of the next persistent launch.
@@ -701,33 +680,12 @@ void tilecol_release(nttb200_plan *p) {
     p->tc_err_host = p->tc_err_dev = nullptr;
 }
 
-template <int LOGG, bool DUAL>
-static void tilecol_gs_launch(int grid, cudaStream_t st, const CUtensorMap &a_lo, const CUtensorMap &a_hi,
-                              const CUtensorMap &b_lo, const CUtensorMap &b_hi, const TileColParams &tp,
-                              const CrossTw &cross, bool l4) {
-    if (l4) {
-        tilecol_gs_kernel<LOGG, DUAL, true><<<grid, kM_Threads, kTC_SmemBytes, st>>>(a_lo, a_hi, b_lo, b_hi,
-                                                                                    tp, cross);
-    } else {
-        tilecol_gs_kernel<LOGG, DUAL, false><<<grid, kM_Threads, kTC_SmemBytes, st>>>(a_lo, a_hi, b_lo, b_hi,
-                                                                                     tp, cross);
-    }
-}
-
 int launch_tilecol_gs(nttb200_plan *p, const int32_t *d_in, const int32_t *d_b, int32_t *d_out,
                       size_t batch, cudaStream_t st) {
-    const int logg = (int) p->logn - 12;
-    if (logg < 1 || logg > 4 || !p->d_tw_tile || !tilecol_enabled(p->logn)) return NTTB200_ERR_UNSUPPORTED;
-    const uint64_t tiles = (uint64_t) batch << logg;
+    if (p->logn != 16 || !p->d_tw_tile) return NTTB200_ERR_UNSUPPORTED;
+    const uint64_t tiles = (uint64_t) batch << 4;
     if (tiles > 0x7fffffffull || ((uintptr_t) d_out & 15u)) return NTTB200_ERR_UNSUPPORTED;
-    // below ~14 tiles per team the prologue, the lag and the drain phase cost more than the
-    // saved HBM pass (measured at N = 2^16: 512 polynomials 0.199 ms against 0.12 ms for the
-    // two passes, 1024 polynomials 0.214 against 0.227, 4096 polynomials 0.748 against 0.814)
-    static const long min_per_team = []() {
-        const char *e = getenv("NTTB200_TILECOL_MIN_TILES_PER_TEAM");
-        return e ? atol(e) : 12L;
-    }();
-    if (tiles < (uint64_t) p->sm_count * kM_Teams * (uint64_t) min_per_team) return NTTB200_ERR_UNSUPPORTED;
+    if (tiles < (uint64_t) p->sm_count * kM_Teams * kTC_MinTilesPerTeam) return NTTB200_ERR_UNSUPPORTED;
     CUtensorMap a_lo, a_hi, b_lo, b_hi;
     if (tile_maps(&a_lo, &a_hi, d_in, (size_t) tiles) != NTTB200_OK) return NTTB200_ERR_UNSUPPORTED;
     TileColParams tp;
@@ -748,18 +706,12 @@ int launch_tilecol_gs(nttb200_plan *p, const int32_t *d_in, const int32_t *d_b, 
         b_lo = a_lo;
         b_hi = a_hi;
     }
-    // one CTA per SM, all co-resident; an even grid when the positions are split over two
-    // CTA classes (N = 2^16)
+    // one CTA per SM, all co-resident; an even grid: the positions are split over two CTA classes
     uint64_t ctas = (tiles + kM_Teams - 1) / kM_Teams;
     int grid = (int) (ctas < (uint64_t) p->sm_count ? ctas : (uint64_t) p->sm_count);
-    if (logg == 4) grid = grid < 2 ? 2 : (grid & ~1);
-    static const long lag_pct = []() {
-        const char *e = getenv("NTTB200_TILECOL_LAG_PCT");
-        return e ? atol(e) : 150L;
-    }();
-    // in flight at any time: one tile per team; trail by lag_pct % of that, in polynomials
-    const uint64_t lag_tiles = (uint64_t) grid * kM_Teams * (uint64_t) (lag_pct < 100 ? 100 : lag_pct) / 100;
-    tp.lag = (uint32_t) ((lag_tiles >> logg) + 2);   // > one queue step (grid * 8 / G polynomials)
+    grid = grid < 2 ? 2 : (grid & ~1);
+    const uint64_t lag_tiles = (uint64_t) grid * kM_Teams * kTC_LagPct / 100;
+    tp.lag = (uint32_t) ((lag_tiles >> 4) + 2);   // > one queue step (grid * 8 / G polynomials)
     // counters: one per polynomial + the error word, stream-ordered scratch
     {
         int rce = tilecol_error_word(p);
@@ -773,16 +725,19 @@ int launch_tilecol_gs(nttb200_plan *p, const int32_t *d_in, const int32_t *d_b, 
     NTTB200_CUDA(cudaMemsetAsync(ctr, 0, sizeof(uint32_t) * (batch + 1), st));
     tp.done = ctr;
     tp.error = p->tc_err_dev;
-    const bool dual = d_b != nullptr, l4 = use_l4(p);
-    switch (logg * 2 + (dual ? 1 : 0)) {
-        case 2: tilecol_gs_launch<1, false>(grid, st, a_lo, a_hi, b_lo, b_hi, tp, p->cross_tw, l4); break;
-        case 3: tilecol_gs_launch<1, true>(grid, st, a_lo, a_hi, b_lo, b_hi, tp, p->cross_tw, l4); break;
-        case 4: tilecol_gs_launch<2, false>(grid, st, a_lo, a_hi, b_lo, b_hi, tp, p->cross_tw, l4); break;
-        case 5: tilecol_gs_launch<2, true>(grid, st, a_lo, a_hi, b_lo, b_hi, tp, p->cross_tw, l4); break;
-        case 6: tilecol_gs_launch<3, false>(grid, st, a_lo, a_hi, b_lo, b_hi, tp, p->cross_tw, l4); break;
-        case 7: tilecol_gs_launch<3, true>(grid, st, a_lo, a_hi, b_lo, b_hi, tp, p->cross_tw, l4); break;
-        case 8: tilecol_gs_launch<4, false>(grid, st, a_lo, a_hi, b_lo, b_hi, tp, p->cross_tw, l4); break;
-        default: tilecol_gs_launch<4, true>(grid, st, a_lo, a_hi, b_lo, b_hi, tp, p->cross_tw, l4); break;
+    const bool dual = d_b != nullptr;
+    if (dual && use_l4(p)) {
+        tilecol_gs_kernel<true, true><<<grid, kM_Threads, kTC_SmemBytes, st>>>(a_lo, a_hi, b_lo, b_hi, tp,
+                                                                               p->cross_tw);
+    } else if (dual) {
+        tilecol_gs_kernel<true, false><<<grid, kM_Threads, kTC_SmemBytes, st>>>(a_lo, a_hi, b_lo, b_hi, tp,
+                                                                                p->cross_tw);
+    } else if (use_l4(p)) {
+        tilecol_gs_kernel<false, true><<<grid, kM_Threads, kTC_SmemBytes, st>>>(a_lo, a_hi, b_lo, b_hi, tp,
+                                                                                p->cross_tw);
+    } else {
+        tilecol_gs_kernel<false, false><<<grid, kM_Threads, kTC_SmemBytes, st>>>(a_lo, a_hi, b_lo, b_hi, tp,
+                                                                                 p->cross_tw);
     }
     g_launches.fetch_add(1, std::memory_order_relaxed);
     cudaError_t e = cudaGetLastError();
@@ -795,17 +750,11 @@ int launch_tilecol_gs(nttb200_plan *p, const int32_t *d_in, const int32_t *d_b, 
 
 // N = 2^16 forward transform in one persistent kernel: 4096 polynomials 0.811 ms against 0.901 ms
 // for column passes + tile pass (0.405 against 0.365 of the HBM roofline).
-// NTTB200_TILECOL_CT_OFF=1: the two-pass path (A/B).
 int launch_tilecol_ct(nttb200_plan *p, const int32_t *d_in, int32_t *d_out, size_t batch, cudaStream_t st) {
-    static const bool on = getenv("NTTB200_TILECOL_CT_OFF") == nullptr;
-    if (!on || p->logn != 16 || !p->d_tw_tile) return NTTB200_ERR_UNSUPPORTED;
+    if (p->logn != 16 || !p->d_tw_tile) return NTTB200_ERR_UNSUPPORTED;
     const uint64_t tiles = (uint64_t) batch << 4;
     if (tiles > 0x7fffffffull || ((uintptr_t) d_out & 15u) || ((uintptr_t) d_in & 15u)) return NTTB200_ERR_UNSUPPORTED;
-    static const long min_per_team = []() {
-        const char *e = getenv("NTTB200_TILECOL_MIN_TILES_PER_TEAM");
-        return e ? atol(e) : 12L;
-    }();
-    if (tiles < (uint64_t) p->sm_count * kM_Teams * (uint64_t) min_per_team) return NTTB200_ERR_UNSUPPORTED;
+    if (tiles < (uint64_t) p->sm_count * kM_Teams * kTC_MinTilesPerTeam) return NTTB200_ERR_UNSUPPORTED;
     CUtensorMap m_lo, m_hi;
     if (tile_maps(&m_lo, &m_hi, d_out, (size_t) tiles) != NTTB200_OK) return NTTB200_ERR_UNSUPPORTED;
     TileColParams tp;
@@ -819,11 +768,7 @@ int launch_tilecol_ct(nttb200_plan *p, const int32_t *d_in, int32_t *d_out, size
     uint64_t ctas = (tiles + kM_Teams - 1) / kM_Teams;
     int grid = (int) (ctas < (uint64_t) p->sm_count ? ctas : (uint64_t) p->sm_count);
     grid = grid < 2 ? 2 : (grid & ~1);
-    static const long lag_pct = []() {
-        const char *e = getenv("NTTB200_TILECOL_LAG_PCT");
-        return e ? atol(e) : 150L;
-    }();
-    const uint64_t lag_tiles = (uint64_t) grid * kM_Teams * (uint64_t) (lag_pct < 100 ? 100 : lag_pct) / 100;
+    const uint64_t lag_tiles = (uint64_t) grid * kM_Teams * kTC_LagPct / 100;
     tp.lag = (uint32_t) ((lag_tiles >> 4) + 2);
     {
         int rce = tilecol_error_word(p);

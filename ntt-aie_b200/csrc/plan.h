@@ -120,9 +120,7 @@ int cuda_fail(cudaError_t e, const char *what);
     } while (0)
 
 // 4q-lazy kernels (fused_common.cuh, gs_bfly_l4 / ct_bfly_l4) serve moduli whose 8q fits a word.
-// NTTB200_NO_L4=1 is the A/B switch for measurements.
-bool l4_enabled();
-inline bool use_l4(const nttb200_plan *p) { return p->q < (1u << 29) && l4_enabled(); }
+inline bool use_l4(const nttb200_plan *p) { return p->q < (1u << 29); }
 
 // Stream-ordered scratch (transform scratch of the multi-kernel products, the counters of the
 // persistent kernel) from a library-private memory pool of the CURRENT device that keeps its
@@ -149,10 +147,8 @@ int launch_polyt_gs(nttb200_plan *p, const int32_t *d_in, const int32_t *d_b, in
                     size_t batch, cudaStream_t st);
 int launch_polyt_ct(nttb200_plan *p, const int32_t *d_in, int32_t *d_out, size_t batch,
                     cudaStream_t st);
-int launch_polyc_gs(nttb200_plan *p, const int32_t *d_in, const int32_t *d_b, int32_t *d_out,
-                    size_t batch, cudaStream_t st);
 
-// N = 2^13..2^16 as one persistent kernel of tile items and column items (kernels_tilecol.cu)
+// N = 2^16 as one persistent kernel of tile items and column items (kernels_tilecol.cu)
 int tilecol_prepare();
 int launch_tilecol_gs(nttb200_plan *p, const int32_t *d_in, const int32_t *d_b, int32_t *d_out,
                       size_t batch, cudaStream_t st);
@@ -231,10 +227,6 @@ inline uint32_t inv_mod_2_32(uint32_t q) {
 constexpr int kRnsTwTile = 32 * 65;  // uint4s per tile position in d_tw_tile (kernels_multi.cu)
 int launch_multi_ct(nttb200_plan *p, const int32_t *d_in, int32_t *d_out, size_t batch,
                     cudaStream_t st);
-int launch_multi_ct_mul(nttb200_plan *p, const int32_t *d_in, const int32_t *d_mul, int32_t *d_out,
-                        size_t batch, cudaStream_t st);
-int launch_fused_gs_scaled(nttb200_plan *p, const int32_t *d_in, int32_t *d_out, size_t batch,
-                           cudaStream_t st);
 int launch_multi_gs_dual(nttb200_plan *p, const int32_t *d_a, const int32_t *d_b, int32_t *d_out,
                          size_t batch, cudaStream_t st);
 

@@ -15,7 +15,8 @@ constexpr int kM_SmemBytes = kM_Teams * kF_PolyBytes + 64 + 1024;
 __device__ __forceinline__ uint4 ldg128(const uint4 *p) { return __ldg(p); }
 
 // Where a team's twiddle slots come from: global memory (LDG, L1-resident across a
-// batch) or -- when every tile uses the same table (N = 4096) -- a shared-memory copy.
+// batch) or a shared-memory copy of one position's table (N = 4096, or a run of tiles
+// at the same position).
 struct TwGlobal {
     const uint4 *p;
     __device__ __forceinline__ uint4 slot(int s) const { return ldg128(p + s * 65); }
@@ -199,17 +200,6 @@ __device__ __forceinline__ void ct_half_stage(uint32_t (&v)[64], const TW tw, ui
             }
         }
     }
-}
-
-template <int S, bool REDUCE>
-__device__ __forceinline__ void gs_stage_g(uint32_t (&v)[64], const uint4 *tw, uint32_t q,
-                                           uint32_t two_q, uint32_t zero) {
-    gs_stage_t<S, REDUCE>(v, TwGlobal{tw}, q, two_q, zero);
-}
-template <int S, bool REDUCE_X>
-__device__ __forceinline__ void ct_stage_g(uint32_t (&v)[64], const uint4 *tw, uint32_t q,
-                                           uint32_t two_q, uint32_t zero) {
-    ct_stage_t<S, REDUCE_X>(v, TwGlobal{tw}, q, two_q, zero);
 }
 
 template <bool REDUCE0, class TW>

@@ -1031,47 +1031,3 @@ def test_persistent_forward_kernel_n65536(lib, oracle_mod):
             plan.ct(d_a, d_a, batch)
             torch.cuda.synchronize()
             assert torch.equal(d_a, d_o), (q, "in place")
-
-
-def test_cluster_kernel_n65536_opt_in(lib, oracle_mod):
-    """The 2-CTA-cluster kernel for N = 2^16 (third round through distributed shared memory,
-    NTTB200_CLUSTER16=1; measured slower than the persistent kernel, kept as the documented
-    alternative).  The switch is read once per process, so this runs in a child process:
-    transform rows and one product against the oracle."""
-    import subprocess
-    import sys
-    code = r"""
-import sys, numpy as np, torch
-sys.path.insert(0, %r)
-import ntt_aie_b200 as nt, oracle
-Q = 469762049
-n, batch = 1 << 16, 150
-rng = np.random.default_rng(777)
-for q in (Q, (1 << 30) - 35):
-    table = rng.integers(0, q, n, dtype=np.int32)
-    a = rng.integers(0, q, (batch, n), dtype=np.int32)
-    a[0] = q - 1
-    d_a = torch.from_numpy(a).cuda()
-    d_o = torch.empty_like(d_a)
-    with nt.Plan(16, q, table) as p:
-        p.gs(d_a, d_o, batch)
-        torch.cuda.synchronize()
-        assert p.last_path == "poly_cluster2", p.last_path
-    rows = [0, 1, 77, batch - 1]
-    assert np.array_equal(d_o.cpu().numpy()[rows], oracle.ntt_gs(a[rows], table, q)), q
-fwd, inv = nt.negacyclic_tables(n, Q, 3)
-a = rng.integers(0, Q, (3, n), dtype=np.int32)
-b = rng.integers(0, Q, (3, n), dtype=np.int32)
-prod = oracle.pointwise(oracle.ntt_ct(a, fwd, Q), oracle.ntt_ct(b, fwd, Q), Q)
-want = oracle.scale(oracle.ntt_gs(prod, inv, Q), oracle.powmod(n, Q - 2, Q), Q)
-with nt.Plan(16, Q, fwd) as pf, nt.Plan(16, Q, inv) as pi:
-    d_c = torch.zeros(3, n, dtype=torch.int32, device="cuda")
-    nt.polymul_negacyclic(pf, pi, torch.from_numpy(a).cuda(), torch.from_numpy(b).cuda(), d_c, 3)
-    torch.cuda.synchronize()
-    assert pi.last_path == "poly_cluster2_dual", pi.last_path
-assert np.array_equal(d_c.cpu().numpy(), want)
-print("cluster kernel ok")
-""" % (os.path.dirname(os.path.dirname(os.path.abspath(__file__))),)
-    env = dict(os.environ, NTTB200_CLUSTER16="1")
-    res = subprocess.run([sys.executable, "-c", code], env=env, capture_output=True, text=True, timeout=600)
-    assert res.returncode == 0 and "cluster kernel ok" in res.stdout, res.stdout + res.stderr

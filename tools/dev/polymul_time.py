@@ -25,4 +25,4 @@ for logn in [int(x) for x in (sys.argv[1] if len(sys.argv) > 1 else "12").split(
         ms = sorted(ev[k].elapsed_time(ev[k + 1]) for k in range(20))
         t = statistics.mean(ms[1:-1])
         print(json.dumps({"logn": logn, "ms": t, "frac": batch * n * 12 / (t * 1e-3) / 1e9 / peak,
-                          "path": pi.last_path, "env3k": os.environ.get("NTTB200_POLYMUL_3KERNEL")}), flush=True)
+                          "path": pi.last_path}), flush=True)

@@ -326,6 +326,34 @@ NTTB200_API int nttb200_rns_dot(nttb200_rns_plan *plan, const int32_t *d_a, cons
 NTTB200_API int nttb200_rns_gs_scaled_batch(nttb200_rns_plan *plan, const int32_t *d_in, int32_t *d_out,
                                             size_t batch, void *cuda_stream);
 
+/* ---- RNS Galois automorphisms (new) --------------------------------------------
+ * sigma_g : a(X) -> a(X^g) mod (X^N + 1) for odd g, the permutation under slot rotations
+ * (g = 5^r mod 2N rotates CKKS slots by r) and conjugation (g = 2N - 1).
+ *   NTTB200_AUTO_COEFF: coefficient domain.  With e = j * g^-1 mod 2N: out[j] = in[e] for
+ *     e < N, (q[l] - in[e - N]) mod q[l] otherwise.
+ *   NTTB200_AUTO_EVAL: evaluation domain, in the order nttb200_rns_ct_batch produces on a plan
+ *     of psi_l^bitrev tables (index k holds a(psi^(2 brev(k) + 1)), brev over logn bits) and
+ *     nttb200_rns_gs_scaled_batch consumes on psi_l^-bitrev tables: the permutation
+ *     out[k] = in[brev((g * brev(k) + (g - 1) / 2) mod N)], the same for every channel and
+ *     every choice of psi_l.  So rns_ct(sigma_coeff(x)) == sigma_eval(rns_ct(x)) bit for bit.
+ * Rules of the evaluation-domain operators: inputs canonical, outputs canonical; galois: count
+ * words on the HOST, every g odd with 1 <= g < 2N, 1 <= count <= 64; a null plan, a null
+ * galois, a bad g or count or an unknown domain -> NTTB200_ERR_INVALID_ARG, also when
+ * batch == 0; a null buffer with batch > 0 or an output that overlaps the input (in place
+ * included: in the evaluation domain block t is written from another block) -> INVALID_ARG;
+ * batch == 0 -> NTTB200_OK with nothing launched; a buffer that is not 16-byte aligned ->
+ * NTTB200_ERR_UNSUPPORTED (nothing is written in either case); indexing is 64-bit, with no
+ * 2^31-word limit; one launch per call.  Only N, L and the moduli are read from the plan, so
+ * either plan of a forward / inverse pair will do. */
+#define NTTB200_AUTO_COEFF 0u
+#define NTTB200_AUTO_EVAL 1u
+/* out[c][b][l] = sigma_{galois[c]}(in[b][l]) for c < count: X -> X^g on every channel of every
+ * polynomial, in the coefficient domain or in the evaluation (rns_ct) order.  d_in [batch][L][N],
+ * d_out [count][batch][L][N] (count outputs from one read of the input: hoisted rotations). */
+NTTB200_API int nttb200_rns_automorphism(nttb200_rns_plan *plan, const int32_t *d_in, int32_t *d_out,
+                                         size_t batch, const uint32_t *galois, uint32_t count,
+                                         uint32_t domain, void *cuda_stream);
+
 /* ---- RNS basis conversion (new) -------------------------------------------------
  * Moves coefficient-domain values from the primes of one plan to those of another: the step
  * under CKKS rescale, the BGV-style modulus drop and the ModUp / ModDown of hybrid key

@@ -21,6 +21,10 @@ from .api import (  # noqa: F401
     RNS_SUB,
     RNS_MUL,
     RNS_ROUND,
+    AUTO_COEFF,
+    AUTO_EVAL,
+    galois_rotation,
+    galois_conjugate,
     ORDER_AIE_DEVICE,
     ORDER_GOLDEN,
     FORCE_GENERIC,

@@ -24,6 +24,8 @@ RNS_ADD = 0
 RNS_SUB = 1
 RNS_MUL = 2
 RNS_ROUND = 1
+AUTO_COEFF = 0
+AUTO_EVAL = 1
 
 _lib = None
 _i32p = ctypes.POINTER(ctypes.c_int32)
@@ -94,6 +96,7 @@ def load_library():
         "nttb200_rns_scale": (ctypes.c_int, [vp, vp, vp, sz, ctypes.POINTER(u32), vp]),
         "nttb200_rns_dot": (ctypes.c_int, [vp, vp, vp, vp, u32, sz, sz, ctypes.c_int, vp]),
         "nttb200_rns_gs_scaled_batch": (ctypes.c_int, [vp, vp, vp, sz, vp]),
+        "nttb200_rns_automorphism": (ctypes.c_int, [vp, vp, vp, sz, ctypes.POINTER(u32), u32, u32, vp]),
         "nttb200_rns_conv_create": (ctypes.c_int, [ctypes.POINTER(vp), vp, vp, u32]),
         "nttb200_rns_conv_destroy": (ctypes.c_int, [vp]),
         "nttb200_rns_base_convert": (ctypes.c_int, [vp, vp, sz, vp, sz, sz, vp]),
@@ -125,7 +128,7 @@ EXPORTED_SYMBOLS = (
     "nttb200_rns_plan_destroy", "nttb200_rns_gs_batch",
     "nttb200_rns_ct_batch", "nttb200_rns_polymul_negacyclic",
     "nttb200_rns_pointwise", "nttb200_rns_scale", "nttb200_rns_dot", "nttb200_rns_gs_scaled_batch",
-    "nttb200_rns_conv_create", "nttb200_rns_conv_destroy", "nttb200_rns_base_convert", "nttb200_rns_mod_down",
+    "nttb200_rns_automorphism", "nttb200_rns_conv_create", "nttb200_rns_conv_destroy", "nttb200_rns_base_convert", "nttb200_rns_mod_down",
     "nttb200_strerror", "nttb200_last_error", "nttb200_kernel_launches", "nttb200_plan_last_path",
     "nttb200_plan_logn", "nttb200_plan_modulus", "nttb200_version",
 )
@@ -420,6 +423,15 @@ class RnsPlan:
         _check(self._lib.nttb200_rns_scale(self._h, _addr(d_a), _addr(d_c), batch, arr, _stream(stream)),
                "rns_scale")
 
+    def automorphism(self, d_in, d_out, batch: int, galois, domain: int = AUTO_EVAL, stream=None) -> None:
+        """out[c][b][l] = sigma_{galois[c]}(in[b][l]): X -> X^g on every channel, in the evaluation
+        (rns_ct) order (AUTO_EVAL) or on coefficients (AUTO_COEFF).  galois: one odd g in [1, 2N) or
+        a sequence of 1..64 of them; d_out holds [len(galois)][batch][L][N]."""
+        gs = [int(galois)] if isinstance(galois, (int, np.integer)) else [int(g) for g in galois]
+        arr = (ctypes.c_uint32 * max(len(gs), 1))(*gs)
+        _check(self._lib.nttb200_rns_automorphism(self._h, _addr(d_in), _addr(d_out), batch, arr, len(gs),
+                                                  domain, _stream(stream)), "rns_automorphism")
+
 
 class RnsConv:
     """Basis conversion from the primes of `src` (S channels, product B) to those of `dst`
@@ -478,6 +490,17 @@ def rns_dot(plan: RnsPlan, d_a, d_w, d_c, terms: int, batch: int, w_batch: Optio
     _check(plan._lib.nttb200_rns_dot(plan._h, _addr(d_a), _addr(d_w), _addr(d_c), terms, batch,
                                      batch if w_batch is None else w_batch, 1 if accumulate else 0,
                                      _stream(stream)), "rns_dot")
+
+
+def galois_rotation(n: int, steps: int) -> int:
+    """Galois element of a CKKS slot rotation by `steps` (negative: the other way) at ring
+    degree n: 5^steps mod 2n.  5 has order n/2 modulo 2n, so -r is 5^(r mod n/2)."""
+    return pow(5, steps % (n // 2), 2 * n)
+
+
+def galois_conjugate(n: int) -> int:
+    """Galois element of complex conjugation of the CKKS slots: 2n - 1 (X -> X^-1)."""
+    return 2 * n - 1
 
 
 def polymul_negacyclic(fwd: Plan, inv: Plan, d_a, d_b, d_c, batch: int, stream=None) -> None:

@@ -992,6 +992,25 @@ int nttb200_rns_dot(nttb200_rns_plan *rp, const int32_t *d_a, const int32_t *d_w
     return launch_rns_dot(rp, d_a, d_w, d_c, terms, batch, w_shared, accumulate != 0, (cudaStream_t) stream);
 }
 
+int nttb200_rns_automorphism(nttb200_rns_plan *rp, const int32_t *d_in, int32_t *d_out, size_t batch,
+                             const uint32_t *galois, uint32_t count, uint32_t domain, void *stream) {
+    if (!rp || !galois || count < 1 || count > kAutoMaxElems || domain > NTTB200_AUTO_EVAL) {
+        return NTTB200_ERR_INVALID_ARG;
+    }
+    for (uint32_t c = 0; c < count; c++) {
+        if (!(galois[c] & 1u) || galois[c] >= (2u << rp->logn)) return NTTB200_ERR_INVALID_ARG;
+    }
+    if (batch && (!d_in || !d_out)) return NTTB200_ERR_INVALID_ARG;
+    if (batch == 0) return NTTB200_OK;
+    const uint64_t words = rns_words(rp, batch), out_words = rns_words(rp, (uint64_t) count * batch);
+    if (!words || !out_words) return NTTB200_ERR_UNSUPPORTED;
+    if (byte_range(d_out, out_words).overlaps(byte_range(d_in, words))) return NTTB200_ERR_INVALID_ARG;
+    if (!aligned16(d_in, d_in, d_out)) return NTTB200_ERR_UNSUPPORTED;
+    DeviceGuard guard(rp->device);
+    return launch_rns_automorph(rp, d_in, d_out, batch, galois, count, domain == NTTB200_AUTO_EVAL,
+                                (cudaStream_t) stream);
+}
+
 /* ------------------------------------------------------- RNS basis conversion */
 int nttb200_rns_conv_create(nttb200_rns_conv **conv, const nttb200_rns_plan *from, const nttb200_rns_plan *to,
                             uint32_t flags) {

@@ -218,6 +218,19 @@ int launch_rns_dot(const nttb200_rns_plan *rp, const int32_t *a, const int32_t *
 int rns_conv_prepare(nttb200_rns_conv *cv, const uint32_t *b, const uint32_t *c);
 int launch_rns_conv(const nttb200_rns_conv *cv, const int32_t *src, const int32_t *tin, uint64_t src_stride,
                     int32_t *out, uint64_t out_stride, size_t batch, bool down, bool round, cudaStream_t st);
+// Galois automorphisms (kernels_rns_automorph.cu), one __grid_constant__ parameter block
+// (896 bytes).  launch_rns_automorph: the caller has checked the arguments (1 <= count <= 64,
+// every g odd in [1, 2N)), the overlap and the 16-byte alignment; eval selects the
+// evaluation-domain (rns_ct order) permutation, else the coefficient domain.
+constexpr int kAutoMaxElems = 64;
+struct RnsAutoConsts {
+    uint32_t g[kAutoMaxElems];      // g
+    uint32_t ginv[kAutoMaxElems];   // g^-1 mod 2N
+    uint32_t off[kAutoMaxElems];    // (g - 1) / 2 mod N, the evaluation-domain offset
+    uint32_t q[kConvMaxChannels];   // q_l
+};
+int launch_rns_automorph(const nttb200_rns_plan *rp, const int32_t *in, int32_t *out, size_t batch,
+                         const uint32_t *galois, uint32_t count, bool eval, cudaStream_t st);
 // q^-1 mod 2^32 for odd q (Montgomery products): Newton iteration, 3 correct bits doubling per step
 inline uint32_t inv_mod_2_32(uint32_t q) {
     uint32_t x = q;

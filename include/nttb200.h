@@ -407,6 +407,32 @@ NTTB200_API int nttb200_rns_base_convert(nttb200_rns_conv *conv, const int32_t *
 NTTB200_API int nttb200_rns_mod_down(nttb200_rns_conv *conv, const int32_t *d_in, int32_t *d_out,
                                      size_t batch, uint32_t flags, void *cuda_stream);
 
+/* Exact forms, for BFV multiplication and decryption (Halevi-Polyakov-Shoup): the overshoot
+ * of the fast conversion is removed with v = round(sum_i y_i / b_i), computed in FP64 in the
+ * same pass.  Exactness: for S <= 32 and moduli <= 2^30 the FP64 sum is within 2^-43 of
+ * sum_i y_i / b_i (DESIGN 3.6), so both results are exact unless the fractional part of x / B
+ * (of t X / B for scale_round) lies within eps = 2^-40 of 1/2.  In that band either neighbour
+ * may be returned: x_c +- B for the conversion, the result +- 1 for scale_round.  Uniform
+ * random x meets the band with probability 2^-39; values that must be exact (BFV) stay far from
+ * it by the parameter choice. */
+
+/* Exact base conversion of the centred value: out[b][j] = x_c mod c_j, where x_c == x (mod B)
+ * and -B/2 < x_c <= B/2.  Arguments, strides and rules as nttb200_rns_base_convert. */
+NTTB200_API int nttb200_rns_base_convert_exact(nttb200_rns_conv *conv, const int32_t *d_in,
+                                               size_t in_stride, int32_t *d_out, size_t out_stride,
+                                               size_t batch, void *cuda_stream);
+
+/* Scale by t / B and round, with the source channels dropped.  d_in [batch][T+S][N], target
+ * channels first (the nttb200_rns_mod_down layout); d_out [batch][T][N]:
+ *   out[b][j] = round(t * X / B) mod c_j,
+ * X the CRT value of all T + S channels.  Valid for every representative of X mod C*B, so a
+ * centred X is covered too.  1 <= t < 2^32: t == 0 -> NTTB200_ERR_INVALID_ARG, also when
+ * batch == 0.  With t = 1 and S = 1 the result equals nttb200_rns_mod_down(ROUND) bit for bit;
+ * with t = 1 and S > 1 it is the exact rounded division by B (rescale by several primes at
+ * once).  Layout and no-overlap rule as nttb200_rns_mod_down. */
+NTTB200_API int nttb200_rns_scale_round(nttb200_rns_conv *conv, const int32_t *d_in, int32_t *d_out,
+                                        size_t batch, uint32_t t, void *cuda_stream);
+
 /* ---- introspection ---------------------------------------------------------- */
 NTTB200_API const char *nttb200_strerror(int status);
 /* text of the last CUDA error seen by the calling thread ("" if none) */

@@ -101,6 +101,8 @@ def load_library():
         "nttb200_rns_conv_destroy": (ctypes.c_int, [vp]),
         "nttb200_rns_base_convert": (ctypes.c_int, [vp, vp, sz, vp, sz, sz, vp]),
         "nttb200_rns_mod_down": (ctypes.c_int, [vp, vp, vp, sz, u32, vp]),
+        "nttb200_rns_base_convert_exact": (ctypes.c_int, [vp, vp, sz, vp, sz, sz, vp]),
+        "nttb200_rns_scale_round": (ctypes.c_int, [vp, vp, vp, sz, u32, vp]),
         "nttb200_strerror": (ctypes.c_char_p, [ctypes.c_int]),
         "nttb200_last_error": (ctypes.c_char_p, []),
         "nttb200_kernel_launches": (ctypes.c_uint64, []),
@@ -129,6 +131,7 @@ EXPORTED_SYMBOLS = (
     "nttb200_rns_ct_batch", "nttb200_rns_polymul_negacyclic",
     "nttb200_rns_pointwise", "nttb200_rns_scale", "nttb200_rns_dot", "nttb200_rns_gs_scaled_batch",
     "nttb200_rns_automorphism", "nttb200_rns_conv_create", "nttb200_rns_conv_destroy", "nttb200_rns_base_convert", "nttb200_rns_mod_down",
+    "nttb200_rns_base_convert_exact", "nttb200_rns_scale_round",
     "nttb200_strerror", "nttb200_last_error", "nttb200_kernel_launches", "nttb200_plan_last_path",
     "nttb200_plan_logn", "nttb200_plan_modulus", "nttb200_version",
 )
@@ -463,18 +466,32 @@ class RnsConv:
     def __exit__(self, *exc):
         self.close()
 
-    def convert(self, d_in, d_out, batch: int, in_stride: int = 0, out_stride: int = 0, stream=None) -> None:
+    def convert(self, d_in, d_out, batch: int, in_stride: int = 0, out_stride: int = 0, exact: bool = False,
+                stream=None) -> None:
         """Fast base conversion (ModUp): out[b][j] = sum_i [in[b][i] (B/b_i)^-1]_{b_i} (B/b_i) mod c_j,
-        i.e. (x + alpha B) mod c_j with 0 <= alpha < S.  Strides in words between polynomials
-        (0: dense S*N / T*N)."""
-        _check(self._lib.nttb200_rns_base_convert(self._h, _addr(d_in), in_stride, _addr(d_out), out_stride,
-                                                  batch, _stream(stream)), "rns_base_convert")
+        i.e. (x + alpha B) mod c_j with 0 <= alpha < S.  exact: the centred value instead,
+        x_c mod c_j with x_c = x (mod B) in (-B/2, B/2] (see nttb200_rns_base_convert_exact for the
+        rounding band).  Strides in words between polynomials (0: dense S*N / T*N)."""
+        if exact:
+            _check(self._lib.nttb200_rns_base_convert_exact(self._h, _addr(d_in), in_stride, _addr(d_out),
+                                                            out_stride, batch, _stream(stream)),
+                   "rns_base_convert_exact")
+        else:
+            _check(self._lib.nttb200_rns_base_convert(self._h, _addr(d_in), in_stride, _addr(d_out), out_stride,
+                                                      batch, _stream(stream)), "rns_base_convert")
 
     def mod_down(self, d_in, d_out, batch: int, round: bool = False, stream=None) -> None:
         """Divide by B and drop the source channels: d_in [batch][T+S][N] (target channels
         first), d_out [batch][T][N]; floor((X + (floor(B/2) if round else 0)) / B) - alpha."""
         _check(self._lib.nttb200_rns_mod_down(self._h, _addr(d_in), _addr(d_out), batch,
                                               RNS_ROUND if round else 0, _stream(stream)), "rns_mod_down")
+
+    def scale_round(self, d_in, d_out, batch: int, t: int = 1, stream=None) -> None:
+        """round(t X / B) on the target channels: d_in [batch][T+S][N] (target channels first),
+        d_out [batch][T][N]; 1 <= t < 2^32.  The BFV tensor-product scaling (t/Q) and, with
+        t = 1, the exact rounded division by B."""
+        _check(self._lib.nttb200_rns_scale_round(self._h, _addr(d_in), _addr(d_out), batch, t, _stream(stream)),
+               "rns_scale_round")
 
 
 def rns_polymul_negacyclic(fwd: RnsPlan, inv: RnsPlan, d_a, d_b, d_c, batch: int, stream=None) -> None:

@@ -1060,10 +1060,10 @@ static bool rows_overlap(uintptr_t in, uint64_t sa, uintptr_t out, uint64_t ta, 
     return k <= (int64_t) batch - 1 && k * p < d + (int64_t) sa;
 }
 
-extern "C" {
-
-int nttb200_rns_base_convert(nttb200_rns_conv *conv, const int32_t *d_in, size_t in_stride, int32_t *d_out,
-                             size_t out_stride, size_t batch, void *stream) {
+// The strided conversions (base_convert, base_convert_exact): null pointers, strides (0: dense),
+// extents, the row overlap and the alignment are checked in that order, then one launch.
+static int conv_strided(nttb200_rns_conv *conv, const int32_t *d_in, size_t in_stride, int32_t *d_out,
+                        size_t out_stride, size_t batch, ConvMode mode, void *stream) {
     if (!conv || (batch && (!d_in || !d_out))) return NTTB200_ERR_INVALID_ARG;
     const uint64_t n = (uint64_t) 1 << conv->logn;
     const uint64_t s_words = conv->src * n, t_words = conv->dst * n;
@@ -1082,13 +1082,15 @@ int nttb200_rns_base_convert(nttb200_rns_conv *conv, const int32_t *d_in, size_t
     if (overlap) return NTTB200_ERR_INVALID_ARG;
     if (!aligned16(d_in, d_in, d_out)) return NTTB200_ERR_UNSUPPORTED;
     DeviceGuard guard(conv->device);
-    return launch_rns_conv(conv, d_in, nullptr, is, d_out, os, batch, false, false, (cudaStream_t) stream);
+    return launch_rns_conv(conv, d_in, nullptr, is, d_out, os, batch, mode, false, 0, (cudaStream_t) stream);
 }
 
-int nttb200_rns_mod_down(nttb200_rns_conv *conv, const int32_t *d_in, int32_t *d_out, size_t batch, uint32_t flags,
-                         void *stream) {
-    if (!conv || (batch && (!d_in || !d_out))) return NTTB200_ERR_INVALID_ARG;
-    if (flags & ~NTTB200_RNS_ROUND) return NTTB200_ERR_INVALID_ARG;
+// The operations on [batch][T+S][N] (mod_down, scale_round; the source rows follow the T target
+// rows of each polynomial): null pointers and a rejected option (bad_option), extents, overlap
+// and alignment are checked in that order, then one launch.
+static int conv_down(nttb200_rns_conv *conv, const int32_t *d_in, int32_t *d_out, size_t batch, bool bad_option,
+                     ConvMode mode, bool round, uint32_t t, void *stream) {
+    if (!conv || (batch && (!d_in || !d_out)) || bad_option) return NTTB200_ERR_INVALID_ARG;
     if (batch == 0) return NTTB200_OK;
     const uint64_t n = (uint64_t) 1 << conv->logn;
     const uint64_t row = (conv->src + conv->dst) * n, t_words = conv->dst * n;
@@ -1096,8 +1098,31 @@ int nttb200_rns_mod_down(nttb200_rns_conv *conv, const int32_t *d_in, int32_t *d
     if (byte_range(d_in, batch * row).overlaps(byte_range(d_out, batch * t_words))) return NTTB200_ERR_INVALID_ARG;
     if (!aligned16(d_in, d_in, d_out)) return NTTB200_ERR_UNSUPPORTED;
     DeviceGuard guard(conv->device);
-    return launch_rns_conv(conv, d_in + t_words, d_in, row, d_out, t_words, batch, true,
-                           (flags & NTTB200_RNS_ROUND) != 0, (cudaStream_t) stream);
+    return launch_rns_conv(conv, d_in + t_words, d_in, row, d_out, t_words, batch, mode, round, t,
+                           (cudaStream_t) stream);
+}
+
+extern "C" {
+
+int nttb200_rns_base_convert(nttb200_rns_conv *conv, const int32_t *d_in, size_t in_stride, int32_t *d_out,
+                             size_t out_stride, size_t batch, void *stream) {
+    return conv_strided(conv, d_in, in_stride, d_out, out_stride, batch, ConvMode::Fast, stream);
+}
+
+int nttb200_rns_base_convert_exact(nttb200_rns_conv *conv, const int32_t *d_in, size_t in_stride, int32_t *d_out,
+                                   size_t out_stride, size_t batch, void *stream) {
+    return conv_strided(conv, d_in, in_stride, d_out, out_stride, batch, ConvMode::Exact, stream);
+}
+
+int nttb200_rns_mod_down(nttb200_rns_conv *conv, const int32_t *d_in, int32_t *d_out, size_t batch, uint32_t flags,
+                         void *stream) {
+    return conv_down(conv, d_in, d_out, batch, (flags & ~NTTB200_RNS_ROUND) != 0, ConvMode::Down,
+                     (flags & NTTB200_RNS_ROUND) != 0, 0, stream);
+}
+
+int nttb200_rns_scale_round(nttb200_rns_conv *conv, const int32_t *d_in, int32_t *d_out, size_t batch, uint32_t t,
+                            void *stream) {
+    return conv_down(conv, d_in, d_out, batch, t == 0, ConvMode::Scale, false, t, stream);
 }
 
 /* ---------------------------------------------------------- introspection */

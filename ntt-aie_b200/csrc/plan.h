@@ -81,7 +81,8 @@ namespace nttb200 {
 constexpr int kConvMaxChannels = 32;
 
 // Constants of one basis conversion (source moduli b_i, product B; target moduli c_j), passed
-// to the kernel as one __grid_constant__ parameter block (5376 bytes).
+// to the kernel as one __grid_constant__ parameter block (6016 bytes).  The fields after wp serve
+// the exact operations only; they come last so that the others keep their offsets.
 struct RnsConvConsts {
     uint32_t m[kConvMaxChannels][kConvMaxChannels];   // [j][i] = (B / b_i) mod c_j
     uint64_t mu[kConvMaxChannels];     // floor(2^64 / c_j) for reduce64
@@ -93,7 +94,15 @@ struct RnsConvConsts {
     uint32_t hb[kConvMaxChannels];     // floor(B/2) mod b_i (0 when not rounding)
     uint32_t w[kConvMaxChannels];      // (B / b_i)^-1 mod b_i
     uint32_t wp[kConvMaxChannels];     // its Shoup companion
+    double binvd[kConvMaxChannels];    // 1 / b_i, correctly rounded
+    uint32_t nbc[kConvMaxChannels];    // -B mod c_j
+    uint32_t tc[kConvMaxChannels];     // t mod c_j (scale-and-round, set per call)
+    uint32_t tcp[kConvMaxChannels];    // its Shoup companion
 };
+
+// What rns_conv_kernel computes: the fast conversion, the division by B, the exact conversion
+// of the centred value, round(t X / B).
+enum class ConvMode : int { Fast, Down, Exact, Scale };
 
 }  // namespace nttb200
 
@@ -213,11 +222,12 @@ int launch_rns_dot(const nttb200_rns_plan *rp, const int32_t *a, const int32_t *
 // basis conversion (kernels_rns_conv.cu).  rns_conv_prepare fills cv->k from the moduli
 // (host only; NTTB200_ERR_MODULUS when two of them share a factor).  launch_rns_conv: the
 // caller has checked the arguments, the overlap and the 16-byte alignment; src rows (S
-// channels) at src + b * src_stride, target input rows (mod_down only) at tin + b * src_stride,
-// output rows (T channels) at out + b * out_stride.
+// channels) at src + b * src_stride, target input rows (Down and Scale) at tin + b * src_stride,
+// output rows (T channels) at out + b * out_stride; round applies to Down, t (>= 1) to Scale.
 int rns_conv_prepare(nttb200_rns_conv *cv, const uint32_t *b, const uint32_t *c);
 int launch_rns_conv(const nttb200_rns_conv *cv, const int32_t *src, const int32_t *tin, uint64_t src_stride,
-                    int32_t *out, uint64_t out_stride, size_t batch, bool down, bool round, cudaStream_t st);
+                    int32_t *out, uint64_t out_stride, size_t batch, ConvMode mode, bool round, uint32_t t,
+                    cudaStream_t st);
 // Galois automorphisms (kernels_rns_automorph.cu), one __grid_constant__ parameter block
 // (896 bytes).  launch_rns_automorph: the caller has checked the arguments (1 <= count <= 64,
 // every g odd in [1, 2N)), the overlap and the 16-byte alignment; eval selects the

@@ -82,7 +82,7 @@ tile_gs_kernel(const __grid_constant__ CUtensorMap map_lo, const __grid_constant
     uint32_t q = prm.q, two_q = 2u * prm.q;
     uint32_t qinv = prm.qinv, scale = prm.scale, scale_shoup = prm.scale_shoup;
     const uint32_t zero = prm.zero, four_q = prm.four_q;
-    static_assert(!L4 || !RNS, "the channels of an RNS batch sit just below 2^30");
+    static_assert(!L4 || !RNS, "an RNS channel may be any modulus in [2, 2^30]: classic butterflies only");
     static_assert(!(DUAL && SCALED) && !(L4 && SCALED), "SCALED is the plain-load form of DUAL's store");
 
     const uint32_t tws = bar_base + 64;
@@ -1119,7 +1119,7 @@ int rns_launch(const nttb200_rns_plan *rp, int kind, const int32_t *d_a, const i
     tp.q = 0;
     tp.zero = 0;
     tp.qinv = tp.scale = tp.scale_shoup = 0;
-    tp.four_q = 0;   // RNS primes sit just below 2^30: classic butterflies
+    tp.four_q = 0;   // a channel may be any modulus in [2, 2^30]: classic butterflies
     uint64_t ctas = (tiles + kM_Teams - 1) / kM_Teams;
     int grid = (int) (ctas < (uint64_t) rp->sm_count ? ctas : (uint64_t) rp->sm_count);
     const size_t polys = batch * limbs;

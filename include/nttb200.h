@@ -433,6 +433,51 @@ NTTB200_API int nttb200_rns_base_convert_exact(nttb200_rns_conv *conv, const int
 NTTB200_API int nttb200_rns_scale_round(nttb200_rns_conv *conv, const int32_t *d_in, int32_t *d_out,
                                         size_t batch, uint32_t t, void *cuda_stream);
 
+/* ---- CKKS slot encoding (new) ----------------------------------------------------
+ * The canonical embedding of the ring Z[X]/(X^N + 1) into n = N/2 complex slots, computed as an
+ * FP64 negacyclic FFT on the device.  With zeta = e^(i pi / N), slot j holds m(zeta^(5^j mod 2N)):
+ * for real coefficients x_k (k < N), s_j = (5^j mod 2N - 1) / 4 (a permutation of 0..n-1),
+ *   decode: y_k = (x_k + i x_(k+n)) zeta^k (k < n),  Y_s = sum_k y_k e^(+2 pi i s k / n),
+ *           z_j = Y_(s_j) / scale;
+ *   encode: v_(s_j) = z_j,  y_k = (1/n) sum_s v_s e^(-2 pi i s k / n),
+ *           m_k + i m_(k+n) = y_k zeta^-k,  a_k = rint(scale * m_k) (half to even).
+ * With this order nttb200_rns_automorphism by galois = 5^r mod 2N takes the slots z to z rotated
+ * left by r (slot j receives z_(j+r)), and by 2N - 1 to conj(z), in both domains.
+ * An encoder is built from an RNS plan as a conversion object is: it copies N, the device and the
+ * moduli, so the plan may be destroyed afterwards.  It owns device tables: the FFT twiddles
+ * e^(2 pi i t / n) and zeta^k, each built once in FP64 within 1 ulp, and the permutation s_j.
+ * A null pointer or flags != 0 -> NTTB200_ERR_INVALID_ARG.
+ * Shared rules of encode and decode: a null encoder, a null pointer with batch > 0 or a scale
+ * that is not finite and > 0 -> NTTB200_ERR_INVALID_ARG, also when batch == 0; batch == 0 ->
+ * NTTB200_OK with nothing launched; overlapping input and output -> NTTB200_ERR_INVALID_ARG; a
+ * buffer that is not 16-byte aligned -> NTTB200_ERR_UNSUPPORTED (nothing is written in either
+ * case); argument errors are returned before any device is touched; indexing is 64-bit.  One
+ * launch per call for N <= 2^14, two above (the transform is split into a column pass and a
+ * row pass through stream-ordered scratch of 16 n bytes per polynomial). */
+typedef struct nttb200_ckks_encoder nttb200_ckks_encoder;
+NTTB200_API int nttb200_ckks_encoder_create(nttb200_ckks_encoder **enc, const nttb200_rns_plan *plan,
+                                            uint32_t flags);
+NTTB200_API int nttb200_ckks_encoder_destroy(nttb200_ckks_encoder *enc);
+
+/* d_slots: complex128 [batch][n], interleaved (re, im) doubles; d_out: int32 [batch][L][N], the
+ * residues a_k mod q_l of every channel, coefficient domain (nttb200_rns_ct_batch takes them from
+ * there).  The residues are exact for every finite scale * m_k, also beyond 2^64 (a = M 2^e with
+ * M < 2^53 is reduced as (M mod q)(2^e mod q)).  A value that is not finite gives unspecified
+ * residues and no fault.  The FFT error is bounded in DESIGN 3.6. */
+NTTB200_API int nttb200_ckks_encode(nttb200_ckks_encoder *enc, const void *d_slots, double scale,
+                                    int32_t *d_out, size_t batch, void *cuda_stream);
+
+/* Reads the first `channels` rows (moduli b_0..b_(C-1), product B) of each polynomial at
+ * d_in + b * in_stride (0: dense channels * N; else a multiple of N and at least channels * N,
+ * the nttb200_rns_base_convert rule) and writes d_slots [batch][n] complex128.  1 <= channels <=
+ * min(L, 4), else NTTB200_ERR_INVALID_ARG; the first `channels` moduli not pairwise coprime ->
+ * NTTB200_ERR_MODULUS.  The centred value x_c in (-B/2, B/2] is exact (128-bit CRT) and enters
+ * the FFT as a double with relative error at most 2^-53.  A message with |x| < B'/2 decodes from
+ * any prefix of channels whose product is B': a level-L ciphertext needs no mod_down first. */
+NTTB200_API int nttb200_ckks_decode(nttb200_ckks_encoder *enc, const int32_t *d_in, size_t in_stride,
+                                    uint32_t channels, double scale, void *d_slots, size_t batch,
+                                    void *cuda_stream);
+
 /* ---- introspection ---------------------------------------------------------- */
 NTTB200_API const char *nttb200_strerror(int status);
 /* text of the last CUDA error seen by the calling thread ("" if none) */

@@ -15,6 +15,7 @@ from .api import (  # noqa: F401
     HostBuffer,
     RnsPlan,
     RnsConv,
+    CkksEncoder,
     rns_polymul_negacyclic,
     rns_dot,
     RNS_ADD,

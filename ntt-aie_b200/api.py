@@ -103,6 +103,10 @@ def load_library():
         "nttb200_rns_mod_down": (ctypes.c_int, [vp, vp, vp, sz, u32, vp]),
         "nttb200_rns_base_convert_exact": (ctypes.c_int, [vp, vp, sz, vp, sz, sz, vp]),
         "nttb200_rns_scale_round": (ctypes.c_int, [vp, vp, vp, sz, u32, vp]),
+        "nttb200_ckks_encoder_create": (ctypes.c_int, [ctypes.POINTER(vp), vp, u32]),
+        "nttb200_ckks_encoder_destroy": (ctypes.c_int, [vp]),
+        "nttb200_ckks_encode": (ctypes.c_int, [vp, vp, ctypes.c_double, vp, sz, vp]),
+        "nttb200_ckks_decode": (ctypes.c_int, [vp, vp, sz, u32, ctypes.c_double, vp, sz, vp]),
         "nttb200_strerror": (ctypes.c_char_p, [ctypes.c_int]),
         "nttb200_last_error": (ctypes.c_char_p, []),
         "nttb200_kernel_launches": (ctypes.c_uint64, []),
@@ -132,6 +136,7 @@ EXPORTED_SYMBOLS = (
     "nttb200_rns_pointwise", "nttb200_rns_scale", "nttb200_rns_dot", "nttb200_rns_gs_scaled_batch",
     "nttb200_rns_automorphism", "nttb200_rns_conv_create", "nttb200_rns_conv_destroy", "nttb200_rns_base_convert", "nttb200_rns_mod_down",
     "nttb200_rns_base_convert_exact", "nttb200_rns_scale_round",
+    "nttb200_ckks_encoder_create", "nttb200_ckks_encoder_destroy", "nttb200_ckks_encode", "nttb200_ckks_decode",
     "nttb200_strerror", "nttb200_last_error", "nttb200_kernel_launches", "nttb200_plan_last_path",
     "nttb200_plan_logn", "nttb200_plan_modulus", "nttb200_version",
 )
@@ -492,6 +497,51 @@ class RnsConv:
         t = 1, the exact rounded division by B."""
         _check(self._lib.nttb200_rns_scale_round(self._h, _addr(d_in), _addr(d_out), batch, t, _stream(stream)),
                "rns_scale_round")
+
+
+class CkksEncoder:
+    """CKKS slot encoding on the moduli and N of `plan`: n = N/2 complex slots, slot j holding
+    m(zeta^(5^j mod 2N)) with zeta = e^(i pi / N).  Slots are complex128 [batch][n] tensors,
+    polynomials int32 [batch][L][N] residues in the coefficient domain.  The object copies what
+    it needs: the plan may be closed afterwards.  See nttb200_ckks_encoder_create for the rules."""
+
+    def __init__(self, plan: RnsPlan):
+        self._lib = load_library()
+        handle = ctypes.c_void_p()
+        _check(self._lib.nttb200_ckks_encoder_create(ctypes.byref(handle), plan._h, 0), "ckks_encoder_create")
+        self._h = handle
+        self.qs = list(plan.qs)
+        self.logn, self.n, self.slots = plan.logn, plan.n, plan.n // 2
+
+    def close(self) -> None:
+        if getattr(self, "_h", None):
+            self._lib.nttb200_ckks_encoder_destroy(self._h)
+            self._h = None
+
+    def __del__(self):
+        try:
+            self.close()
+        except Exception:
+            pass
+
+    def __enter__(self):
+        return self
+
+    def __exit__(self, *exc):
+        self.close()
+
+    def encode(self, d_slots, d_out, batch: int, scale: float, stream=None) -> None:
+        """d_out[b][l][k] = rint(scale * m_k) mod q_l, m the real polynomial whose slots are d_slots[b]."""
+        _check(self._lib.nttb200_ckks_encode(self._h, _addr(d_slots), float(scale), _addr(d_out), batch,
+                                             _stream(stream)), "ckks_encode")
+
+    def decode(self, d_in, d_slots, batch: int, scale: float, channels: Optional[int] = None, in_stride: int = 0,
+               stream=None) -> None:
+        """d_slots[b] = the slots of x_c / scale, x_c the centred CRT value of the first `channels`
+        rows (default min(L, 4)) of polynomial b at d_in + b * in_stride (0: dense)."""
+        c = min(len(self.qs), 4) if channels is None else channels
+        _check(self._lib.nttb200_ckks_decode(self._h, _addr(d_in), in_stride, c, float(scale), _addr(d_slots),
+                                             batch, _stream(stream)), "ckks_decode")
 
 
 def rns_polymul_negacyclic(fwd: RnsPlan, inv: RnsPlan, d_a, d_b, d_c, batch: int, stream=None) -> None:

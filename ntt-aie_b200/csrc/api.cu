@@ -6,9 +6,11 @@
 // nttb200_plan_create; kernel(bo_inA, bo_root, bo_outC) + run.wait() ->
 // nttb200_gs_batch / nttb200_gs_host.  There is no CPU compute path in here:
 // without a usable CUDA device every compute entry point returns an error.
+#include <float.h>
 #include <stdio.h>
 #include <string.h>
 
+#include <algorithm>
 #include <new>
 #include <stdexcept>
 #include <vector>
@@ -1123,6 +1125,87 @@ int nttb200_rns_mod_down(nttb200_rns_conv *conv, const int32_t *d_in, int32_t *d
 int nttb200_rns_scale_round(nttb200_rns_conv *conv, const int32_t *d_in, int32_t *d_out, size_t batch, uint32_t t,
                             void *stream) {
     return conv_down(conv, d_in, d_out, batch, t == 0, ConvMode::Scale, false, t, stream);
+}
+
+/* ------------------------------------------------------- CKKS slot encoding */
+int nttb200_ckks_encoder_create(nttb200_ckks_encoder **enc, const nttb200_rns_plan *plan, uint32_t flags) {
+    if (!enc) return NTTB200_ERR_INVALID_ARG;
+    *enc = nullptr;
+    if (!plan || flags != 0) return NTTB200_ERR_INVALID_ARG;
+    nttb200_ckks_encoder *e = new (std::nothrow) nttb200_ckks_encoder();
+    if (!e) return NTTB200_ERR_ALLOC;
+    e->device = plan->device;
+    e->logn = plan->logn;
+    e->limbs = plan->limbs;
+    e->sm_count = plan->sm_count;
+    for (uint32_t l = 0; l < e->limbs; l++) {
+        e->k.q[l] = plan->pos[l].x;
+        e->k.mu[l] = (uint64_t) ((((unsigned __int128) 1) << 64) / e->k.q[l]);
+    }
+    int rc;
+    {
+        DeviceGuard guard(e->device);
+        try {
+            rc = ckks_prepare(e);
+        } catch (...) {
+            rc = NTTB200_ERR_ALLOC;
+        }
+        if (rc != NTTB200_OK) ckks_release(e);
+    }
+    if (rc != NTTB200_OK) {
+        delete e;
+        return rc;
+    }
+    *enc = e;
+    return NTTB200_OK;
+}
+
+int nttb200_ckks_encoder_destroy(nttb200_ckks_encoder *enc) {
+    if (!enc) return NTTB200_OK;
+    {
+        DeviceGuard guard(enc->device);
+        ckks_release(enc);
+    }
+    delete enc;
+    return NTTB200_OK;
+}
+
+static bool bad_scale(double scale) { return !(scale > 0.0 && scale <= DBL_MAX); }
+
+int nttb200_ckks_encode(nttb200_ckks_encoder *enc, const void *d_slots, double scale, int32_t *d_out, size_t batch,
+                        void *stream) {
+    if (!enc || bad_scale(scale) || (batch && (!d_slots || !d_out))) return NTTB200_ERR_INVALID_ARG;
+    if (batch == 0) return NTTB200_OK;
+    const uint64_t n = (uint64_t) 1 << (enc->logn - 1), row = (uint64_t) enc->limbs << enc->logn;
+    if (batch > ((uint64_t) 1 << 60) / row) return NTTB200_ERR_UNSUPPORTED;
+    if (byte_range(d_out, batch * row).overlaps(byte_range(d_slots, 4 * batch * n))) return NTTB200_ERR_INVALID_ARG;
+    if (!aligned16(d_slots, d_slots, d_out)) return NTTB200_ERR_UNSUPPORTED;
+    DeviceGuard guard(enc->device);
+    return launch_ckks_encode(enc, static_cast<const double2 *>(d_slots), scale, d_out, batch, (cudaStream_t) stream);
+}
+
+int nttb200_ckks_decode(nttb200_ckks_encoder *enc, const int32_t *d_in, size_t in_stride, uint32_t channels,
+                        double scale, void *d_slots, size_t batch, void *stream) {
+    if (!enc || bad_scale(scale) || (batch && (!d_in || !d_slots))) return NTTB200_ERR_INVALID_ARG;
+    const uint64_t N = (uint64_t) 1 << enc->logn, c_words = channels * N;
+    if (channels < 1 || channels > std::min<uint32_t>(enc->limbs, kCkksMaxDecode)) return NTTB200_ERR_INVALID_ARG;
+    const uint64_t is = in_stride ? in_stride : c_words;
+    if (is % N || is < c_words) return NTTB200_ERR_INVALID_ARG;
+    CkksDecConsts k;
+    const int rc = ckks_decode_consts(enc, channels, scale, &k);
+    if (rc != NTTB200_OK) return rc;
+    if (batch == 0) return NTTB200_OK;
+    if (is > ((uint64_t) 1 << 60) || batch - 1 > (((uint64_t) 1 << 60) - c_words) / is ||
+        batch > ((uint64_t) 1 << 60) / (2 * N)) {
+        return NTTB200_ERR_UNSUPPORTED;
+    }
+    if (byte_range(d_in, (batch - 1) * is + c_words).overlaps(byte_range(d_slots, 2 * N * batch))) {
+        return NTTB200_ERR_INVALID_ARG;
+    }
+    if (!aligned16(d_in, d_in, d_slots)) return NTTB200_ERR_UNSUPPORTED;
+    DeviceGuard guard(enc->device);
+    return launch_ckks_decode(enc, d_in, is, channels, k, static_cast<double2 *>(d_slots), batch,
+                              (cudaStream_t) stream);
 }
 
 /* ---------------------------------------------------------- introspection */

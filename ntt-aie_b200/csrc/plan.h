@@ -253,4 +253,48 @@ int launch_multi_ct(nttb200_plan *p, const int32_t *d_in, int32_t *d_out, size_t
 int launch_multi_gs_dual(nttb200_plan *p, const int32_t *d_a, const int32_t *d_b, int32_t *d_out,
                          size_t batch, cudaStream_t st);
 
+// CKKS slot encoding and decoding (kernels_ckks.cu).  Channel moduli of the encoder, one
+// __grid_constant__ block per encode call.
+struct CkksEncConsts {
+    uint64_t mu[kConvMaxChannels];   // floor(2^64 / q_l) for reduce64
+    uint32_t q[kConvMaxChannels];
+};
+constexpr int kCkksMaxDecode = 4;
+// Exact CRT of the first C <= 4 channels (moduli b_i, product B < 2^120), set per decode call.
+struct CkksDecConsts {
+    uint64_t m[kCkksMaxDecode][2];   // B / b_i as (low, high) 64-bit limbs
+    uint64_t t[kCkksMaxDecode][2];   // (2k + 1) B: S > (k + 1/2) B  <=>  2S > (2k + 1) B
+    uint64_t bb[2];                  // B
+    uint32_t b[kCkksMaxDecode];      // b_i
+    uint32_t w[kCkksMaxDecode];      // (B / b_i)^-1 mod b_i
+    uint32_t wp[kCkksMaxDecode];     // its Shoup companion
+    double inv_scale;                // 1 / scale, correctly rounded
+};
+
+}  // namespace nttb200
+
+// Self-contained: copies N, the device and the moduli from the plan, which may be destroyed.
+struct nttb200_ckks_encoder {
+    int device = 0;
+    uint32_t logn = 12;
+    uint32_t limbs = 0;
+    int sm_count = 148;
+    nttb200::CkksEncConsts k{};
+    double2 *d_w = nullptr;        // [n] e^(2 pi i t / n), n = N/2 slots
+    double2 *d_zeta = nullptr;     // [n] zeta^k = e^(i pi k / N)
+    uint32_t *d_perm = nullptr;    // [n] s_j = (5^j mod 2N - 1) / 4
+    uint32_t *d_iperm = nullptr;   // [n] j of s
+};
+
+namespace nttb200 {
+// builds the device tables of a filled-in encoder (device current); ckks_release frees them
+int ckks_prepare(nttb200_ckks_encoder *enc);
+void ckks_release(nttb200_ckks_encoder *enc);
+// the CRT constants of the first `channels` moduli (NTTB200_ERR_MODULUS when two share a factor)
+int ckks_decode_consts(const nttb200_ckks_encoder *enc, uint32_t channels, double scale, CkksDecConsts *k);
+// the caller has checked the arguments, the overlap and the 16-byte alignment
+int launch_ckks_encode(const nttb200_ckks_encoder *enc, const double2 *slots, double scale, int32_t *out,
+                       size_t batch, cudaStream_t st);
+int launch_ckks_decode(const nttb200_ckks_encoder *enc, const int32_t *in, uint64_t in_stride, uint32_t channels,
+                       const CkksDecConsts &k, double2 *slots, size_t batch, cudaStream_t st);
 }  // namespace nttb200

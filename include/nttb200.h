@@ -478,6 +478,56 @@ NTTB200_API int nttb200_ckks_decode(nttb200_ckks_encoder *enc, const int32_t *d_
                                     uint32_t channels, double scale, void *d_slots, size_t batch,
                                     void *cuda_stream);
 
+/* ---- Packed integer slots for BFV and BGV (new) -----------------------------------
+ * N integer slots mod t, t a prime with t == 1 (mod 2N) and t < 2^30.  psi is the smallest
+ * primitive 2N-th root of unity mod t (the least of the N roots psi_0^(2i+1)).  The slots form
+ * a 2 x N/2 matrix: slot i = r N/2 + j holds m(psi^e_i) mod t, with e_i = 5^j mod 2N in row
+ * r = 0 and e_i = 2N - (5^j mod 2N) in row r = 1.  With this order nttb200_rns_automorphism by
+ * galois = 5^s mod 2N rotates both rows left by s (slot j receives slot j + s, as for CKKS), and
+ * by 2N - 1 swaps the rows, in both domains.  In the rns_ct order of a one-channel plan of
+ * modulus t on psi^bitrev tables, slot i sits at index k_i = brev((e_i - 1) / 2), brev over
+ * logn bits.
+ * Encode writes the plaintext m (coefficients in [0, t)) on the L channels of the plan, in one
+ * of two forms; Q is the product of the channel moduli q_l, r = Q mod t:
+ *   NTTB200_PACK_SCALED   round(Q m / t) mod q_l, the BFV message term.  Computed as
+ *                         (Delta_l m + rho) mod q_l with Delta_l = floor(Q / t) mod q_l
+ *                         = -r t^-1 mod q_l and rho = floor((2 r m + t) / 2t) = round(r m / t)
+ *                         (t odd: never a tie); no big integers.
+ *   NTTB200_PACK_CENTRED  m_c mod q_l with m_c == m (mod t) in (-t/2, t/2]: the BGV plaintext
+ *                         and the BFV plaintext operand of a plaintext x ciphertext product.
+ * nttb200_packed_encoder_create: copies N, the device and the moduli of `plan` (which may be
+ * destroyed afterwards), finds psi on the host and owns two one-channel RNS plans of modulus t
+ * (psi^bitrev and psi^-bitrev tables), the slot table k_i and its inverse.  A null pointer or
+ * flags != 0 -> NTTB200_ERR_INVALID_ARG; t not prime, t != 1 (mod 2N), t >= 2^30 or t dividing
+ * some q_l -> NTTB200_ERR_MODULUS; both before any device is touched.
+ * Shared rules of encode and decode: a null encoder or an unknown mode / flag ->
+ * NTTB200_ERR_INVALID_ARG, also when batch == 0; a null buffer with batch > 0 or overlapping
+ * input and output -> NTTB200_ERR_INVALID_ARG; batch == 0 -> NTTB200_OK with nothing launched; a
+ * buffer that is not 16-byte aligned -> NTTB200_ERR_UNSUPPORTED (nothing is written in either
+ * case); indexing is 64-bit, and batch * N / 4096 must stay below 2^31 (the transforms mod t; else
+ * NTTB200_ERR_UNSUPPORTED).  The data passes through stream-ordered scratch of 4N bytes per
+ * polynomial.  Launches per call: encode 3 at N = 4096 and 4 above (gather, the inverse
+ * transform mod t, the lift); decode 2 and 3 (the forward transform mod t, gather). */
+#define NTTB200_PACK_SCALED 0u
+#define NTTB200_PACK_CENTRED 1u
+typedef struct nttb200_packed_encoder nttb200_packed_encoder;
+NTTB200_API int nttb200_packed_encoder_create(nttb200_packed_encoder **enc, const nttb200_rns_plan *plan,
+                                              uint32_t t, uint32_t flags);
+NTTB200_API int nttb200_packed_encoder_destroy(nttb200_packed_encoder *enc);
+
+/* d_slots: int32 [batch][N], each word read as a signed integer and reduced mod t (negative
+ * values encode directly); d_out: int32 [batch][L][N], coefficient domain.  mode:
+ * NTTB200_PACK_SCALED or NTTB200_PACK_CENTRED. */
+NTTB200_API int nttb200_packed_encode(nttb200_packed_encoder *enc, const int32_t *d_slots, uint32_t mode,
+                                      int32_t *d_out, size_t batch, void *cuda_stream);
+
+/* d_in: int32 [batch][N], canonical residues mod t in the coefficient domain (what the BFV
+ * decryption rns_scale -> convert_exact -> rns_scale on a t plan, or the BGV decryption
+ * convert_exact from Q to {t}, produces); d_slots: int32 [batch][N], in [0, t) with flags 0, in
+ * (-t/2, t/2] with NTTB200_PACK_CENTRED. */
+NTTB200_API int nttb200_packed_decode(nttb200_packed_encoder *enc, const int32_t *d_in, uint32_t flags,
+                                      int32_t *d_slots, size_t batch, void *cuda_stream);
+
 /* ---- introspection ---------------------------------------------------------- */
 NTTB200_API const char *nttb200_strerror(int status);
 /* text of the last CUDA error seen by the calling thread ("" if none) */

@@ -16,6 +16,7 @@ from .api import (  # noqa: F401
     RnsPlan,
     RnsConv,
     CkksEncoder,
+    PackedEncoder,
     rns_polymul_negacyclic,
     rns_dot,
     RNS_ADD,
@@ -24,6 +25,8 @@ from .api import (  # noqa: F401
     RNS_ROUND,
     AUTO_COEFF,
     AUTO_EVAL,
+    PACK_SCALED,
+    PACK_CENTRED,
     galois_rotation,
     galois_conjugate,
     ORDER_AIE_DEVICE,

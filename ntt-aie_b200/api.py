@@ -26,6 +26,8 @@ RNS_MUL = 2
 RNS_ROUND = 1
 AUTO_COEFF = 0
 AUTO_EVAL = 1
+PACK_SCALED = 0
+PACK_CENTRED = 1
 
 _lib = None
 _i32p = ctypes.POINTER(ctypes.c_int32)
@@ -107,6 +109,10 @@ def load_library():
         "nttb200_ckks_encoder_destroy": (ctypes.c_int, [vp]),
         "nttb200_ckks_encode": (ctypes.c_int, [vp, vp, ctypes.c_double, vp, sz, vp]),
         "nttb200_ckks_decode": (ctypes.c_int, [vp, vp, sz, u32, ctypes.c_double, vp, sz, vp]),
+        "nttb200_packed_encoder_create": (ctypes.c_int, [ctypes.POINTER(vp), vp, u32, u32]),
+        "nttb200_packed_encoder_destroy": (ctypes.c_int, [vp]),
+        "nttb200_packed_encode": (ctypes.c_int, [vp, vp, u32, vp, sz, vp]),
+        "nttb200_packed_decode": (ctypes.c_int, [vp, vp, u32, vp, sz, vp]),
         "nttb200_strerror": (ctypes.c_char_p, [ctypes.c_int]),
         "nttb200_last_error": (ctypes.c_char_p, []),
         "nttb200_kernel_launches": (ctypes.c_uint64, []),
@@ -137,6 +143,8 @@ EXPORTED_SYMBOLS = (
     "nttb200_rns_automorphism", "nttb200_rns_conv_create", "nttb200_rns_conv_destroy", "nttb200_rns_base_convert", "nttb200_rns_mod_down",
     "nttb200_rns_base_convert_exact", "nttb200_rns_scale_round",
     "nttb200_ckks_encoder_create", "nttb200_ckks_encoder_destroy", "nttb200_ckks_encode", "nttb200_ckks_decode",
+    "nttb200_packed_encoder_create", "nttb200_packed_encoder_destroy", "nttb200_packed_encode",
+    "nttb200_packed_decode",
     "nttb200_strerror", "nttb200_last_error", "nttb200_kernel_launches", "nttb200_plan_last_path",
     "nttb200_plan_logn", "nttb200_plan_modulus", "nttb200_version",
 )
@@ -542,6 +550,53 @@ class CkksEncoder:
         c = min(len(self.qs), 4) if channels is None else channels
         _check(self._lib.nttb200_ckks_decode(self._h, _addr(d_in), in_stride, c, float(scale), _addr(d_slots),
                                              batch, _stream(stream)), "ckks_decode")
+
+
+class PackedEncoder:
+    """Packed integer slots mod t (BFV / BGV batch encoding) on the moduli and N of `plan`: N slots
+    as a 2 x N/2 matrix, slot r N/2 + j holding m(psi^e) mod t with e = 5^j mod 2N (row 0) or
+    2N - (5^j mod 2N) (row 1), psi the smallest primitive 2N-th root mod t.  t: a prime below 2^30
+    with t = 1 (mod 2N), dividing no channel modulus.  Slots are int32 [batch][N] tensors,
+    polynomials int32 [batch][L][N] residues in the coefficient domain.  The object copies what it
+    needs: the plan may be closed afterwards.  See nttb200_packed_encoder_create for the rules."""
+
+    def __init__(self, plan: RnsPlan, t: int):
+        self._lib = load_library()
+        handle = ctypes.c_void_p()
+        _check(self._lib.nttb200_packed_encoder_create(ctypes.byref(handle), plan._h, int(t), 0),
+               "packed_encoder_create")
+        self._h = handle
+        self.qs, self.t = list(plan.qs), int(t)
+        self.logn, self.n = plan.logn, plan.n
+
+    def close(self) -> None:
+        if getattr(self, "_h", None):
+            self._lib.nttb200_packed_encoder_destroy(self._h)
+            self._h = None
+
+    def __del__(self):
+        try:
+            self.close()
+        except Exception:
+            pass
+
+    def __enter__(self):
+        return self
+
+    def __exit__(self, *exc):
+        self.close()
+
+    def encode(self, d_slots, d_out, batch: int, centred: bool = False, stream=None) -> None:
+        """d_out[b][l] = round(Q m / t) mod q_l (BFV), or with centred m_c mod q_l, m_c in (-t/2, t/2]
+        (BGV, BFV plaintext operand); m the plaintext whose slots are d_slots[b] mod t (signed words)."""
+        _check(self._lib.nttb200_packed_encode(self._h, _addr(d_slots), PACK_CENTRED if centred else PACK_SCALED,
+                                               _addr(d_out), batch, _stream(stream)), "packed_encode")
+
+    def decode(self, d_in, d_slots, batch: int, centred: bool = False, stream=None) -> None:
+        """d_slots[b] = the slots of the plaintext d_in[b] (canonical residues mod t, coefficient
+        domain), in [0, t), or in (-t/2, t/2] with centred."""
+        _check(self._lib.nttb200_packed_decode(self._h, _addr(d_in), PACK_CENTRED if centred else 0,
+                                               _addr(d_slots), batch, _stream(stream)), "packed_decode")
 
 
 def rns_polymul_negacyclic(fwd: RnsPlan, inv: RnsPlan, d_a, d_b, d_c, batch: int, stream=None) -> None:

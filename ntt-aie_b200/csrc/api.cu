@@ -1208,6 +1208,92 @@ int nttb200_ckks_decode(nttb200_ckks_encoder *enc, const int32_t *d_in, size_t i
                               (cudaStream_t) stream);
 }
 
+/* ------------------------------------------------------ packed integer slots */
+// trial division: t < 2^30, so divisors up to 2^15
+static bool is_prime(uint32_t t) {
+    if (t < 2) return false;
+    for (uint32_t d = 2; d * d <= t; d++) {
+        if (t % d == 0) return false;
+    }
+    return true;
+}
+
+int nttb200_packed_encoder_create(nttb200_packed_encoder **enc, const nttb200_rns_plan *plan, uint32_t t,
+                                  uint32_t flags) {
+    if (!enc) return NTTB200_ERR_INVALID_ARG;
+    *enc = nullptr;
+    if (!plan || flags != 0) return NTTB200_ERR_INVALID_ARG;
+    if (t >= (1u << 30) || !is_prime(t) || (t - 1) % (2u << plan->logn)) return NTTB200_ERR_MODULUS;
+    for (uint32_t l = 0; l < plan->limbs; l++) {
+        if (plan->pos[l].x % t == 0) return NTTB200_ERR_MODULUS;
+    }
+    nttb200_packed_encoder *e = new (std::nothrow) nttb200_packed_encoder();
+    if (!e) return NTTB200_ERR_ALLOC;
+    e->device = plan->device;
+    e->logn = plan->logn;
+    e->limbs = plan->limbs;
+    e->sm_count = plan->sm_count;
+    e->k.t = t;
+    for (uint32_t l = 0; l < e->limbs; l++) e->k.q[l] = plan->pos[l].x;
+    int rc;
+    {
+        DeviceGuard guard(e->device);
+        try {
+            rc = packed_prepare(e);
+        } catch (...) {
+            rc = NTTB200_ERR_ALLOC;
+        }
+        if (rc != NTTB200_OK) packed_release(e);
+    }
+    if (rc != NTTB200_OK) {
+        delete e;
+        return rc;
+    }
+    *enc = e;
+    return NTTB200_OK;
+}
+
+int nttb200_packed_encoder_destroy(nttb200_packed_encoder *enc) {
+    if (!enc) return NTTB200_OK;
+    {
+        DeviceGuard guard(enc->device);
+        packed_release(enc);
+    }
+    delete enc;
+    return NTTB200_OK;
+}
+
+// Shared checks of encode and decode after the mode / flag: in_words and out_words per polynomial.
+static int packed_args(const nttb200_packed_encoder *enc, const int32_t *in, uint64_t in_words, const int32_t *out,
+                       uint64_t out_words, size_t batch) {
+    if (batch && (!in || !out)) return NTTB200_ERR_INVALID_ARG;
+    if (batch == 0) return NTTB200_OK;
+    if (batch > (0x7fffffffull >> (enc->logn - 12))) return NTTB200_ERR_UNSUPPORTED;   // the transforms mod t
+    if (byte_range(in, batch * in_words).overlaps(byte_range(out, batch * out_words))) return NTTB200_ERR_INVALID_ARG;
+    if (!aligned16(in, in, out)) return NTTB200_ERR_UNSUPPORTED;
+    return NTTB200_OK;
+}
+
+int nttb200_packed_encode(nttb200_packed_encoder *enc, const int32_t *d_slots, uint32_t mode, int32_t *d_out,
+                          size_t batch, void *stream) {
+    if (!enc || mode > NTTB200_PACK_CENTRED) return NTTB200_ERR_INVALID_ARG;
+    const uint64_t N = (uint64_t) 1 << enc->logn;
+    const int rc = packed_args(enc, d_slots, N, d_out, enc->limbs * N, batch);
+    if (rc != NTTB200_OK || batch == 0) return rc;
+    DeviceGuard guard(enc->device);
+    return launch_packed_encode(enc, d_slots, mode == NTTB200_PACK_CENTRED, d_out, batch, (cudaStream_t) stream);
+}
+
+int nttb200_packed_decode(nttb200_packed_encoder *enc, const int32_t *d_in, uint32_t flags, int32_t *d_slots,
+                          size_t batch, void *stream) {
+    if (!enc || (flags & ~NTTB200_PACK_CENTRED)) return NTTB200_ERR_INVALID_ARG;
+    const uint64_t N = (uint64_t) 1 << enc->logn;
+    const int rc = packed_args(enc, d_in, N, d_slots, N, batch);
+    if (rc != NTTB200_OK || batch == 0) return rc;
+    DeviceGuard guard(enc->device);
+    return launch_packed_decode(enc, d_in, flags == NTTB200_PACK_CENTRED, d_slots, batch, (cudaStream_t) stream);
+}
+
 /* ---------------------------------------------------------- introspection */
 const char *nttb200_strerror(int status) {
     switch (status) {

@@ -297,4 +297,41 @@ int launch_ckks_encode(const nttb200_ckks_encoder *enc, const double2 *slots, do
                        size_t batch, cudaStream_t st);
 int launch_ckks_decode(const nttb200_ckks_encoder *enc, const int32_t *in, uint64_t in_stride, uint32_t channels,
                        const CkksDecConsts &k, double2 *slots, size_t batch, cudaStream_t st);
+
+// Packed integer slots mod t (kernels_packed.cu): the constants of the lift onto the L channels,
+// one __grid_constant__ block (656 bytes) built at create time.
+struct PackedConsts {
+    uint64_t mu[kConvMaxChannels];      // floor(2^64 / q_l) for reduce64
+    uint32_t q[kConvMaxChannels];       // q_l
+    uint32_t delta[kConvMaxChannels];   // floor(Q / t) mod q_l = -r t^-1 mod q_l
+    uint32_t negt[kConvMaxChannels];    // -t mod q_l
+    uint64_t mu_t;                      // floor(2^64 / t)
+    uint32_t t;
+    uint32_t r;                         // Q mod t
+};
+}  // namespace nttb200
+
+// Self-contained: copies N, the device and the moduli from the plan, which may be destroyed.
+struct nttb200_packed_encoder {
+    int device = 0;
+    uint32_t logn = 12;
+    uint32_t limbs = 0;
+    int sm_count = 148;
+    nttb200::PackedConsts k{};
+    nttb200_rns_plan *fwd = nullptr;   // one channel of modulus t, psi^bitrev table (rns_ct)
+    nttb200_rns_plan *inv = nullptr;   // psi^-bitrev table (rns_gs_scaled)
+    uint32_t *d_slot = nullptr;        // [N] k_i, the rns_ct index of slot i
+    uint32_t *d_islot = nullptr;       // [N] i of k
+};
+
+namespace nttb200 {
+// psi, the plans and the slot tables of a filled-in encoder (k.q, k.t and logn set; device
+// current); packed_release frees them
+int packed_prepare(nttb200_packed_encoder *enc);
+void packed_release(nttb200_packed_encoder *enc);
+// the caller has checked the arguments, the overlap, the 16-byte alignment and the size
+int launch_packed_encode(const nttb200_packed_encoder *enc, const int32_t *slots, bool centred, int32_t *out,
+                         size_t batch, cudaStream_t st);
+int launch_packed_decode(const nttb200_packed_encoder *enc, const int32_t *in, bool centred, int32_t *slots,
+                         size_t batch, cudaStream_t st);
 }  // namespace nttb200

@@ -528,6 +528,58 @@ NTTB200_API int nttb200_packed_encode(nttb200_packed_encoder *enc, const int32_t
 NTTB200_API int nttb200_packed_decode(nttb200_packed_encoder *enc, const int32_t *d_in, uint32_t flags,
                                       int32_t *d_slots, size_t batch, void *cuda_stream);
 
+/* ---- Hybrid key switching (new) -------------------------------------------------
+ * Relinearisation and the second half of a rotation in one call, with the gadget of hybrid key
+ * switching (digits of alpha primes, special primes P).
+ * nttb200_rns_keyswitch_create: qp_fwd / qp_inv are one forward / inverse pair (psi_l^bitrev and
+ * psi_l^-bitrev tables) over L + K channels in the order [Q | P]: Q is the first q_limbs = L
+ * channels and P the remaining K >= 1, so the result lands directly in the nttb200_rns_mod_down
+ * layout.  Digit i covers the channels [i alpha, min((i + 1) alpha, L)), dnum = ceil(L / alpha)
+ * digits (the last one may be shorter); D_i is the product of its primes.  The object copies N,
+ * the device, the moduli and the tables (it builds its own forward / inverse plans on Q and on
+ * Q P, and the conversion constants of ModUp and ModDown): the plans may be destroyed afterwards.
+ * A null pointer, flags != 0, plans with different N or device or channel count, q_limbs == 0,
+ * q_limbs >= the channel count (no P channel), alpha == 0 or alpha > L, or channel moduli that
+ * differ between the two plans -> NTTB200_ERR_INVALID_ARG; moduli that are not pairwise coprime
+ * or an even modulus (no N^-1) -> NTTB200_ERR_MODULUS; all before any device is touched.
+ *
+ * nttb200_rns_keyswitch_apply: d_in holds x, [batch][L][N] on Q, polynomial b at d_in + b * in_stride
+ * (0: dense L * N; else a multiple of N and at least L * N, the nttb200_rns_base_convert rule: the
+ * c1 of a [batch][2][L][N] ciphertext batch is d_in = ct + L * N with in_stride 2 L N).
+ * d_keys: [count][dnum][2][L + K][N], in the evaluation (rns_ct) order on Q P, caller-owned.
+ * Element c, digit i holds (b_i, a_i) with
+ *     b_i + a_i s == e_i + P (Q / D_i) [(Q / D_i)^-1]_{D_i} s'   (mod Q P),
+ * s' = sigma_g(s) for the rotation key of g = galois[c], s^2 for the relinearisation key (g = 1).
+ * For every c < count (1 <= count <= 64; every g odd in [1, 2N); g = 1 allowed):
+ *     d_out[c][b] = (u0, u1) = ModDown_P( sum_i sigma_g(ModUp(x)_i) * (b_i, a_i) ),
+ * d_out [count][batch][2][L][N], ModDown the rounding division of nttb200_rns_mod_down(ROUND).
+ * Then u0 + u1 s ~ sigma_g(x) s' within the usual hybrid key-switching noise: a rotation adds
+ * sigma_g(c0) to u0 and keeps u1, relinearisation adds (u0, u1) to (d0, d1).  The result is bit
+ * for bit the one of rns_gs_scaled on Q, ModUp of every digit by nttb200_rns_base_convert (own
+ * rows copied), rns_ct on Q P, nttb200_rns_automorphism(EVAL), nttb200_rns_dot for b and for a,
+ * rns_gs_scaled on Q P, nttb200_rns_mod_down(ROUND), rns_ct on Q.
+ * NTTB200_KS_COEFF_IN: d_in holds coefficients (the first transform is skipped);
+ * NTTB200_KS_COEFF_OUT: d_out is left in coefficients (the last transform is skipped).
+ * Rules of the evaluation-domain operators: a null ks, a null galois, a bad g or count or an
+ * unknown flag -> NTTB200_ERR_INVALID_ARG, also when batch == 0; a null buffer with batch > 0, a
+ * bad stride, or d_out overlapping d_in or d_keys -> INVALID_ARG; batch == 0 -> NTTB200_OK with
+ * nothing launched; a buffer that is not 16-byte aligned -> NTTB200_ERR_UNSUPPORTED (nothing is
+ * written in either case); indexing is 64-bit; max(2 count, dnum) * batch * (L + K) * N / 4096
+ * must stay below 2^31 (the transforms; else UNSUPPORTED).  Stream-ordered scratch: the digits,
+ * dnum * batch * (L + K) * N words, and the products, 2 * count * batch * (L + K) * N words.
+ * Launches per call: 2 dnum + 5 at N = 4096 and 2 dnum + 9 above, one (two) fewer for each
+ * transform skipped by a flag. */
+#define NTTB200_KS_COEFF_IN 1u    /* d_in holds coefficients (else the rns_ct order)        */
+#define NTTB200_KS_COEFF_OUT 2u   /* leave the output in coefficients (else the rns_ct order) */
+typedef struct nttb200_rns_keyswitch nttb200_rns_keyswitch;
+NTTB200_API int nttb200_rns_keyswitch_create(nttb200_rns_keyswitch **ks, const nttb200_rns_plan *qp_fwd,
+                                             const nttb200_rns_plan *qp_inv, uint32_t q_limbs, uint32_t alpha,
+                                             uint32_t flags);
+NTTB200_API int nttb200_rns_keyswitch_destroy(nttb200_rns_keyswitch *ks);
+NTTB200_API int nttb200_rns_keyswitch_apply(nttb200_rns_keyswitch *ks, const int32_t *d_in, size_t in_stride,
+                                      const int32_t *d_keys, const uint32_t *galois, uint32_t count,
+                                      int32_t *d_out, size_t batch, uint32_t flags, void *cuda_stream);
+
 /* ---- introspection ---------------------------------------------------------- */
 NTTB200_API const char *nttb200_strerror(int status);
 /* text of the last CUDA error seen by the calling thread ("" if none) */

@@ -17,6 +17,7 @@ from .api import (  # noqa: F401
     RnsConv,
     CkksEncoder,
     PackedEncoder,
+    KeySwitcher,
     rns_polymul_negacyclic,
     rns_dot,
     RNS_ADD,
@@ -27,6 +28,8 @@ from .api import (  # noqa: F401
     AUTO_EVAL,
     PACK_SCALED,
     PACK_CENTRED,
+    KS_COEFF_IN,
+    KS_COEFF_OUT,
     galois_rotation,
     galois_conjugate,
     ORDER_AIE_DEVICE,

@@ -28,6 +28,8 @@ AUTO_COEFF = 0
 AUTO_EVAL = 1
 PACK_SCALED = 0
 PACK_CENTRED = 1
+KS_COEFF_IN = 1
+KS_COEFF_OUT = 2
 
 _lib = None
 _i32p = ctypes.POINTER(ctypes.c_int32)
@@ -113,6 +115,9 @@ def load_library():
         "nttb200_packed_encoder_destroy": (ctypes.c_int, [vp]),
         "nttb200_packed_encode": (ctypes.c_int, [vp, vp, u32, vp, sz, vp]),
         "nttb200_packed_decode": (ctypes.c_int, [vp, vp, u32, vp, sz, vp]),
+        "nttb200_rns_keyswitch_create": (ctypes.c_int, [ctypes.POINTER(vp), vp, vp, u32, u32, u32]),
+        "nttb200_rns_keyswitch_destroy": (ctypes.c_int, [vp]),
+        "nttb200_rns_keyswitch_apply": (ctypes.c_int, [vp, vp, sz, vp, ctypes.POINTER(u32), u32, vp, sz, u32, vp]),
         "nttb200_strerror": (ctypes.c_char_p, [ctypes.c_int]),
         "nttb200_last_error": (ctypes.c_char_p, []),
         "nttb200_kernel_launches": (ctypes.c_uint64, []),
@@ -145,6 +150,7 @@ EXPORTED_SYMBOLS = (
     "nttb200_ckks_encoder_create", "nttb200_ckks_encoder_destroy", "nttb200_ckks_encode", "nttb200_ckks_decode",
     "nttb200_packed_encoder_create", "nttb200_packed_encoder_destroy", "nttb200_packed_encode",
     "nttb200_packed_decode",
+    "nttb200_rns_keyswitch_create", "nttb200_rns_keyswitch_destroy", "nttb200_rns_keyswitch_apply",
     "nttb200_strerror", "nttb200_last_error", "nttb200_kernel_launches", "nttb200_plan_last_path",
     "nttb200_plan_logn", "nttb200_plan_modulus", "nttb200_version",
 )
@@ -597,6 +603,54 @@ class PackedEncoder:
         domain), in [0, t), or in (-t/2, t/2] with centred."""
         _check(self._lib.nttb200_packed_decode(self._h, _addr(d_in), PACK_CENTRED if centred else 0,
                                                _addr(d_slots), batch, _stream(stream)), "packed_decode")
+
+
+class KeySwitcher:
+    """Hybrid key switching on the [Q | P] channels of a forward / inverse plan pair: Q the first
+    q_limbs channels, digits of alpha primes (dnum = ceil(q_limbs / alpha), the last one may be
+    shorter), P the rest.  The object copies what it needs: the plans may be closed afterwards.
+    See nttb200_rns_keyswitch_create for the rules and the key layout."""
+
+    def __init__(self, qp_fwd: RnsPlan, qp_inv: RnsPlan, q_limbs: int, alpha: int):
+        self._lib = load_library()
+        handle = ctypes.c_void_p()
+        _check(self._lib.nttb200_rns_keyswitch_create(ctypes.byref(handle), qp_fwd._h, qp_inv._h, q_limbs, alpha, 0),
+               "rns_keyswitch_create")
+        self._h = handle
+        self.qs = list(qp_fwd.qs)
+        self.q_limbs, self.alpha = q_limbs, alpha
+        self.dnum = -(-q_limbs // alpha)
+        self.logn, self.n = qp_fwd.logn, qp_fwd.n
+
+    def close(self) -> None:
+        if getattr(self, "_h", None):
+            self._lib.nttb200_rns_keyswitch_destroy(self._h)
+            self._h = None
+
+    def __del__(self):
+        try:
+            self.close()
+        except Exception:
+            pass
+
+    def __enter__(self):
+        return self
+
+    def __exit__(self, *exc):
+        self.close()
+
+    def switch(self, d_in, d_keys, d_out, batch: int, galois=1, in_stride: int = 0, coeff_in: bool = False,
+               coeff_out: bool = False, stream=None) -> None:
+        """d_out[c][b] = (u0, u1) = ModDown(sum_i sigma_g(ModUp(x_b)_i) * key[c][i]) with g = galois[c]:
+        d_in [batch][L][N] on Q (rows at d_in + b * in_stride, 0: dense), d_keys
+        [count][dnum][2][L+K][N] on Q P in the rns_ct order, d_out [count][batch][2][L][N].  galois:
+        one odd g in [1, 2N) (1: relinearisation) or a sequence of 1..64 of them (hoisted rotations).
+        coeff_in / coeff_out: input / output in coefficients instead of the rns_ct order."""
+        gs = [int(galois)] if isinstance(galois, (int, np.integer)) else [int(g) for g in galois]
+        arr = (ctypes.c_uint32 * max(len(gs), 1))(*gs)
+        flags = (KS_COEFF_IN if coeff_in else 0) | (KS_COEFF_OUT if coeff_out else 0)
+        _check(self._lib.nttb200_rns_keyswitch_apply(self._h, _addr(d_in), in_stride, _addr(d_keys), arr, len(gs),
+                                               _addr(d_out), batch, flags, _stream(stream)), "rns_keyswitch_apply")
 
 
 def rns_polymul_negacyclic(fwd: RnsPlan, inv: RnsPlan, d_a, d_b, d_c, batch: int, stream=None) -> None:

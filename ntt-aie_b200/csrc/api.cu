@@ -12,6 +12,7 @@
 
 #include <algorithm>
 #include <new>
+#include <numeric>
 #include <stdexcept>
 #include <vector>
 
@@ -1292,6 +1293,97 @@ int nttb200_packed_decode(nttb200_packed_encoder *enc, const int32_t *d_in, uint
     if (rc != NTTB200_OK || batch == 0) return rc;
     DeviceGuard guard(enc->device);
     return launch_packed_decode(enc, d_in, flags == NTTB200_PACK_CENTRED, d_slots, batch, (cudaStream_t) stream);
+}
+
+/* ------------------------------------------------------- hybrid key switching */
+int nttb200_rns_keyswitch_create(nttb200_rns_keyswitch **ks, const nttb200_rns_plan *qp_fwd,
+                                 const nttb200_rns_plan *qp_inv, uint32_t q_limbs, uint32_t alpha, uint32_t flags) {
+    if (!ks) return NTTB200_ERR_INVALID_ARG;
+    *ks = nullptr;
+    if (!qp_fwd || !qp_inv || flags != 0) return NTTB200_ERR_INVALID_ARG;
+    if (qp_fwd->logn != qp_inv->logn || qp_fwd->device != qp_inv->device || qp_fwd->limbs != qp_inv->limbs) {
+        return NTTB200_ERR_INVALID_ARG;
+    }
+    const uint32_t LK = qp_fwd->limbs;
+    if (q_limbs == 0 || q_limbs >= LK || alpha == 0 || alpha > q_limbs) return NTTB200_ERR_INVALID_ARG;
+    for (uint32_t l = 0; l < LK; l++) {
+        if (qp_fwd->pos[l].x != qp_inv->pos[l].x) return NTTB200_ERR_INVALID_ARG;
+    }
+    for (uint32_t l = 0; l < LK; l++) {
+        const uint32_t q = qp_fwd->pos[l].x;
+        if (!(q & 1u)) return NTTB200_ERR_MODULUS;   // N^-1 must exist
+        for (uint32_t m = l + 1; m < LK; m++) {
+            if (std::gcd(q, qp_fwd->pos[m].x) != 1) return NTTB200_ERR_MODULUS;
+        }
+    }
+    nttb200_rns_keyswitch *k = new (std::nothrow) nttb200_rns_keyswitch();
+    if (!k) return NTTB200_ERR_ALLOC;
+    k->device = qp_fwd->device;
+    k->logn = qp_fwd->logn;
+    k->q_limbs = q_limbs;
+    k->limbs = LK;
+    k->alpha = alpha;
+    k->dnum = (q_limbs + alpha - 1) / alpha;
+    k->sm_count = qp_fwd->sm_count;
+    int rc;
+    {
+        DeviceGuard guard(k->device);
+        try {
+            rc = keyswitch_prepare(k, qp_fwd, qp_inv);
+        } catch (...) {
+            rc = NTTB200_ERR_ALLOC;
+        }
+        if (rc != NTTB200_OK) keyswitch_release(k);
+    }
+    if (rc != NTTB200_OK) {
+        delete k;
+        return rc;
+    }
+    *ks = k;
+    return NTTB200_OK;
+}
+
+int nttb200_rns_keyswitch_destroy(nttb200_rns_keyswitch *ks) {
+    if (!ks) return NTTB200_OK;
+    {
+        DeviceGuard guard(ks->device);
+        keyswitch_release(ks);
+    }
+    delete ks;
+    return NTTB200_OK;
+}
+
+int nttb200_rns_keyswitch_apply(nttb200_rns_keyswitch *ks, const int32_t *d_in, size_t in_stride, const int32_t *d_keys,
+                          const uint32_t *galois, uint32_t count, int32_t *d_out, size_t batch, uint32_t flags,
+                          void *stream) {
+    if (!ks || !galois || count < 1 || count > kAutoMaxElems) return NTTB200_ERR_INVALID_ARG;
+    if (flags & ~(NTTB200_KS_COEFF_IN | NTTB200_KS_COEFF_OUT)) return NTTB200_ERR_INVALID_ARG;
+    for (uint32_t c = 0; c < count; c++) {
+        if (!(galois[c] & 1u) || galois[c] >= (2u << ks->logn)) return NTTB200_ERR_INVALID_ARG;
+    }
+    if (batch && (!d_in || !d_keys || !d_out)) return NTTB200_ERR_INVALID_ARG;
+    const uint64_t n = (uint64_t) 1 << ks->logn, qw = ks->q_limbs * n, rw = ks->limbs * n;
+    const uint64_t is = in_stride ? in_stride : qw;
+    if (is % n || is < qw) return NTTB200_ERR_INVALID_ARG;
+    if (batch == 0) return NTTB200_OK;
+    // sizes: byte counts within 62 bits; the transforms count polynomials in 32 bits and tiles in 31
+    const uint64_t lim = (uint64_t) 1 << 60, polys = (uint64_t) 2 * count * batch;
+    if (is > lim || batch > lim / (2 * kAutoMaxElems * (ks->dnum + 2) * rw) || batch - 1 > (lim - qw) / is) {
+        return NTTB200_ERR_UNSUPPORTED;
+    }
+    const uint64_t tiles = std::max<uint64_t>(polys, (uint64_t) ks->dnum * batch) * ks->limbs << (ks->logn - 12);
+    if (tiles > 0x7fffffffull || std::max<uint64_t>(polys, (uint64_t) ks->dnum * batch) > 0xffffffffull) {
+        return NTTB200_ERR_UNSUPPORTED;
+    }
+    const ByteRange out = byte_range(d_out, polys * qw);
+    if (out.overlaps(byte_range(d_in, (batch - 1) * is + qw)) ||
+        out.overlaps(byte_range(d_keys, (uint64_t) count * ks->dnum * 2 * rw))) {
+        return NTTB200_ERR_INVALID_ARG;
+    }
+    if (!aligned16(d_in, d_keys, d_out)) return NTTB200_ERR_UNSUPPORTED;
+    DeviceGuard guard(ks->device);
+    return launch_keyswitch(ks, d_in, is, d_keys, galois, count, d_out, batch, (flags & NTTB200_KS_COEFF_IN) != 0,
+                            (flags & NTTB200_KS_COEFF_OUT) != 0, (cudaStream_t) stream);
 }
 
 /* ---------------------------------------------------------- introspection */

@@ -30,9 +30,6 @@ constexpr int kA_Threads = 256;
 constexpr int kA_BlockWords = 4096;                          // evaluation-domain work item
 constexpr int kA_BlockVecs = kA_BlockWords / 4 / kA_Threads;   // uint4 per thread
 
-// logn-bit reversal of x < 2^logn (logn >= 12)
-__device__ __forceinline__ uint32_t brev_n(uint32_t x, uint32_t logn) { return __brev(x) >> (32 - logn); }
-
 // items = rows << (logn - 12); out_elem = words of one output element (rows * N)
 __global__ void __launch_bounds__(kA_Threads)
 rns_auto_eval_kernel(const uint4 *in, uint4 *out, uint64_t items, uint64_t out_elem, uint32_t logn,

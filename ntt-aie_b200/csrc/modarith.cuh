@@ -60,4 +60,7 @@ __device__ __forceinline__ uint32_t barrett_mul(uint32_t a, uint32_t b, uint32_t
     return csub(r, q);
 }
 
+// logn-bit reversal of x < 2^logn (logn >= 12): the index map of the rns_ct order
+__device__ __forceinline__ uint32_t brev_n(uint32_t x, uint32_t logn) { return __brev(x) >> (32 - logn); }
+
 }  // namespace nttb200

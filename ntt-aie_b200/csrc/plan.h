@@ -334,4 +334,41 @@ int launch_packed_encode(const nttb200_packed_encoder *enc, const int32_t *slots
                          size_t batch, cudaStream_t st);
 int launch_packed_decode(const nttb200_packed_encoder *enc, const int32_t *in, bool centred, int32_t *slots,
                          size_t batch, cudaStream_t st);
+
+// Hybrid key switching (kernels_rns_keyswitch.cu): the Galois constants of one call and the
+// per-channel moduli of Q P, one __grid_constant__ block (896 bytes).
+struct RnsKsConsts {
+    uint32_t g[kAutoMaxElems];      // g
+    uint32_t off[kAutoMaxElems];    // (g - 1) / 2 mod N, the evaluation-domain offset
+    uint64_t mu[kConvMaxChannels];  // floor(2^64 / q_l) for reduce64
+    uint32_t q[kConvMaxChannels];   // q_l
+};
+}  // namespace nttb200
+
+// Self-contained: own transform plans built from the given plans' tables, and own conversion
+// constants; the plans given to nttb200_rns_keyswitch_create may be destroyed afterwards.
+struct nttb200_rns_keyswitch {
+    int device = 0;
+    uint32_t logn = 12;
+    uint32_t q_limbs = 0;   // L
+    uint32_t limbs = 0;     // L + K
+    uint32_t alpha = 0;
+    uint32_t dnum = 0;      // ceil(L / alpha)
+    int sm_count = 148;
+    nttb200_rns_plan *q_fwd = nullptr, *q_inv = nullptr;     // the first L channels
+    nttb200_rns_plan *qp_fwd = nullptr, *qp_inv = nullptr;   // all L + K channels
+    std::vector<nttb200_rns_conv> up_lo;   // [i - 1]: digit i -> Q channels [0, i alpha), i >= 1
+    std::vector<nttb200_rns_conv> up_hi;   // [i]: digit i -> channels [min((i + 1) alpha, L), L + K)
+    nttb200_rns_conv down;                 // P -> Q
+};
+
+namespace nttb200 {
+// the plans and conversion constants of a filled-in object (logn, limbs, alpha, dnum set; device
+// current; the moduli checked); keyswitch_release frees them
+int keyswitch_prepare(nttb200_rns_keyswitch *ks, const nttb200_rns_plan *qp_fwd, const nttb200_rns_plan *qp_inv);
+void keyswitch_release(nttb200_rns_keyswitch *ks);
+// the caller has checked the arguments, the overlap, the 16-byte alignment and the sizes
+int launch_keyswitch(const nttb200_rns_keyswitch *ks, const int32_t *in, uint64_t in_stride, const int32_t *keys,
+                     const uint32_t *galois, uint32_t count, int32_t *out, size_t batch, bool coeff_in,
+                     bool coeff_out, cudaStream_t st);
 }  // namespace nttb200

@@ -580,6 +580,52 @@ NTTB200_API int nttb200_rns_keyswitch_apply(nttb200_rns_keyswitch *ks, const int
                                       const int32_t *d_keys, const uint32_t *galois, uint32_t count,
                                       int32_t *d_out, size_t batch, uint32_t flags, void *cuda_stream);
 
+/* ---- Plaintext matrix-vector products (new) -------------------------------------
+ * y = M z on the slots of every ciphertext of a batch, M given by its generalised diagonals:
+ *     y[s] = sum_{k in offsets} d_k[s] * z[(s + k) mod n],   n = N/2,
+ * over the n complex CKKS slots, or over each of the two rows of packed BFV / BGV slots (each row
+ * its own n x n matrix).  Rotation by r is galois_rotation(N, r) = 5^r mod 2N.  Baby-step
+ * giant-step schedule: k = n1 i + j with 0 <= j < n1,
+ *     W_i = sum_j sigma_{-n1 i}(pt_{n1 i + j}) (.) rot_j(ct),   y = W_0 + sum_{i >= 1} rot_{n1 i}(W_i);
+ * the babies rot_j (j >= 1) come from one hoisted key switch of c1 (rot_0 = ct), each giant is a
+ * key switch of W_i.c1, and only the babies and giants that occur are computed.
+ *
+ * nttb200_rns_lintrans_keys: the Galois elements whose keys the call needs, in the order it reads
+ * them: the babies j >= 1 that occur in ascending order (5^j mod 2N), then the giants i >= 1 that
+ * occur in ascending order (5^(n1 i) mod 2N).  *nkeys receives their number; galois_out, when not
+ * null, receives the elements (room for *nkeys: ask with galois_out = null first).  Host only.
+ * A null offsets or nkeys, count == 0, n1 outside [1, 64], logn outside [12, 16], an offset >= N/2
+ * or a duplicated one -> NTTB200_ERR_INVALID_ARG.
+ *
+ * nttb200_rns_lintrans_apply: ks a key switcher with L = q_limbs.  d_ct [batch][2][L][N] in the
+ * rns_ct order on Q.  d_diags [count][L][N]: d_k encoded (CKKS scale Delta_pt, or packed), in the
+ * rns_ct order, in the order of offsets, not rotated (sigma_{-n1 i} is applied inside); one matrix
+ * for the whole batch.  d_keys [nkeys][dnum][2][L + K][N] in the order of nttb200_rns_lintrans_keys,
+ * each key in the format of nttb200_rns_keyswitch_apply.  d_out [batch][2][L][N] in the rns_ct
+ * order, not rescaled (CKKS scale Delta Delta_pt).  The result is bit for bit the one of the
+ * composed calls: nttb200_rns_keyswitch_apply hoisted over the babies, nttb200_rns_automorphism(EVAL)
+ * of c0 plus rns_pointwise ADD, automorphism(EVAL) of each diagonal by sigma_{-n1 i},
+ * rns_pointwise MUL / ADD per term, one nttb200_rns_keyswitch_apply per giant, automorphism of
+ * W_i.c0 and the adds.  The offsets are read before the call returns.
+ * A null ks, the errors of nttb200_rns_lintrans_keys, or nkeys different from its count ->
+ * NTTB200_ERR_INVALID_ARG, also when batch == 0; a null buffer with batch > 0 (d_keys may be null
+ * when nkeys == 0), or d_out overlapping d_ct, d_diags or d_keys (no in-place form) -> INVALID_ARG;
+ * batch == 0 -> NTTB200_OK with nothing launched; a buffer that is not 16-byte aligned ->
+ * NTTB200_ERR_UNSUPPORTED (nothing is written in either case); indexing is 64-bit; the transforms
+ * of a key-switch pass must stay below 2^31 tiles (else UNSUPPORTED), as in
+ * nttb200_rns_keyswitch_apply.  With nb babies, ng giants >= 1 and nw giants (0 included):
+ * stream-ordered scratch of (nb + nw + ng) * batch * 2 * L * N words (nb + ng when the only giant is
+ * 0) plus 16 * (2 nw + count + 1) bytes of schedule, and per key-switch pass of c elements the
+ * scratch of nttb200_rns_keyswitch_apply with c * batch inputs for the giants.
+ * Launches per call, with P = 2 dnum + 5 at N = 4096 and 2 dnum + 9 above:
+ *     [nb > 0] P + 1 + [ng > 0] (ceil(ng / 64) P + 1);   one offset 0 alone is one launch. */
+NTTB200_API int nttb200_rns_lintrans_keys(uint32_t logn, const uint32_t *offsets, uint32_t count, uint32_t n1,
+                                          uint32_t *galois_out, uint32_t *nkeys);
+NTTB200_API int nttb200_rns_lintrans_apply(nttb200_rns_keyswitch *ks, const int32_t *d_ct, const int32_t *d_diags,
+                                           const uint32_t *offsets, uint32_t count, uint32_t n1,
+                                           const int32_t *d_keys, uint32_t nkeys, int32_t *d_out, size_t batch,
+                                           void *cuda_stream);
+
 /* ---- introspection ---------------------------------------------------------- */
 NTTB200_API const char *nttb200_strerror(int status);
 /* text of the last CUDA error seen by the calling thread ("" if none) */

@@ -32,6 +32,7 @@ from .api import (  # noqa: F401
     KS_COEFF_OUT,
     galois_rotation,
     galois_conjugate,
+    lintrans_galois,
     ORDER_AIE_DEVICE,
     ORDER_GOLDEN,
     FORCE_GENERIC,

@@ -118,6 +118,9 @@ def load_library():
         "nttb200_rns_keyswitch_create": (ctypes.c_int, [ctypes.POINTER(vp), vp, vp, u32, u32, u32]),
         "nttb200_rns_keyswitch_destroy": (ctypes.c_int, [vp]),
         "nttb200_rns_keyswitch_apply": (ctypes.c_int, [vp, vp, sz, vp, ctypes.POINTER(u32), u32, vp, sz, u32, vp]),
+        "nttb200_rns_lintrans_keys": (ctypes.c_int, [u32, ctypes.POINTER(u32), u32, u32, ctypes.POINTER(u32),
+                                                     ctypes.POINTER(u32)]),
+        "nttb200_rns_lintrans_apply": (ctypes.c_int, [vp, vp, vp, ctypes.POINTER(u32), u32, u32, vp, u32, vp, sz, vp]),
         "nttb200_strerror": (ctypes.c_char_p, [ctypes.c_int]),
         "nttb200_last_error": (ctypes.c_char_p, []),
         "nttb200_kernel_launches": (ctypes.c_uint64, []),
@@ -151,6 +154,7 @@ EXPORTED_SYMBOLS = (
     "nttb200_packed_encoder_create", "nttb200_packed_encoder_destroy", "nttb200_packed_encode",
     "nttb200_packed_decode",
     "nttb200_rns_keyswitch_create", "nttb200_rns_keyswitch_destroy", "nttb200_rns_keyswitch_apply",
+    "nttb200_rns_lintrans_keys", "nttb200_rns_lintrans_apply",
     "nttb200_strerror", "nttb200_last_error", "nttb200_kernel_launches", "nttb200_plan_last_path",
     "nttb200_plan_logn", "nttb200_plan_modulus", "nttb200_version",
 )
@@ -652,6 +656,21 @@ class KeySwitcher:
         _check(self._lib.nttb200_rns_keyswitch_apply(self._h, _addr(d_in), in_stride, _addr(d_keys), arr, len(gs),
                                                _addr(d_out), batch, flags, _stream(stream)), "rns_keyswitch_apply")
 
+    def linear_transform(self, d_ct, d_diags, offsets, n1: int, d_keys, d_out, batch: int, stream=None) -> None:
+        """y = M z on the slots of every ciphertext, M given by its generalised diagonals
+        y[s] = sum_k d_k[s] z[(s + k) mod N/2], by baby-step giant-step with n1 babies: d_ct
+        [batch][2][L][N] in the rns_ct order, d_diags [count][L][N] the encoded d_k in the rns_ct order
+        and the order of offsets (each in [0, N/2)), d_keys [nkeys][dnum][2][L+K][N] for the elements of
+        lintrans_galois(N, offsets, n1) in that order (None when there are none), d_out [batch][2][L][N],
+        not rescaled."""
+        offs = [int(k) for k in offsets]
+        arr = (ctypes.c_uint32 * max(len(offs), 1))(*offs)
+        nkeys = len(lintrans_galois(self.n, offs, n1))
+        _check(self._lib.nttb200_rns_lintrans_apply(self._h, _addr(d_ct), _addr(d_diags), arr, len(offs), n1,
+                                                    0 if d_keys is None else _addr(d_keys), nkeys, _addr(d_out),
+                                                    batch, _stream(stream)),
+               "rns_lintrans_apply")
+
 
 def rns_polymul_negacyclic(fwd: RnsPlan, inv: RnsPlan, d_a, d_b, d_c, batch: int, stream=None) -> None:
     _check(fwd._lib.nttb200_rns_polymul_negacyclic(fwd._h, inv._h, _addr(d_a), _addr(d_b),
@@ -672,6 +691,21 @@ def galois_rotation(n: int, steps: int) -> int:
     """Galois element of a CKKS slot rotation by `steps` (negative: the other way) at ring
     degree n: 5^steps mod 2n.  5 has order n/2 modulo 2n, so -r is 5^(r mod n/2)."""
     return pow(5, steps % (n // 2), 2 * n)
+
+
+def lintrans_galois(n: int, offsets, n1: int) -> list:
+    """The Galois elements whose keys KeySwitcher.linear_transform needs at ring degree n, in the
+    order it reads them: the baby rotations j = k mod n1 >= 1 that occur, ascending, then the giant
+    rotations n1 i (i = k // n1 >= 1) that occur, ascending."""
+    lib = load_library()
+    offs = [int(k) for k in offsets]
+    arr = (ctypes.c_uint32 * max(len(offs), 1))(*offs)
+    count = ctypes.c_uint32()
+    logn = n.bit_length() - 1
+    _check(lib.nttb200_rns_lintrans_keys(logn, arr, len(offs), n1, None, ctypes.byref(count)), "rns_lintrans_keys")
+    out = (ctypes.c_uint32 * max(count.value, 1))()
+    _check(lib.nttb200_rns_lintrans_keys(logn, arr, len(offs), n1, out, ctypes.byref(count)), "rns_lintrans_keys")
+    return [int(g) for g in out[:count.value]]
 
 
 def galois_conjugate(n: int) -> int:

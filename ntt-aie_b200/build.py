@@ -25,7 +25,7 @@ NVCC_FLAGS = ["-O3", "-std=c++17", "-lineinfo", "-Xcompiler", "-fPIC,-fvisibilit
 SOURCES = ["api.cu", "kernels_generic.cu", "kernels_fused.cu", "kernels_multi.cu",
            "kernels_small.cu", "tables.cu", "kernels_polymul.cu", "kernels_poly.cu", "kernels_tilecol.cu",
            "kernels_rns_eval.cu", "kernels_rns_conv.cu", "kernels_rns_automorph.cu", "kernels_ckks.cu",
-           "kernels_packed.cu", "kernels_rns_keyswitch.cu"]
+           "kernels_packed.cu", "kernels_rns_keyswitch.cu", "kernels_rns_lintrans.cu"]
 HEADERS = ["plan.h", "modarith.cuh", "fused_common.cuh", "tile_common.cuh", os.path.join(ROOT, "include", "nttb200.h")]
 
 

@@ -1383,7 +1383,84 @@ int nttb200_rns_keyswitch_apply(nttb200_rns_keyswitch *ks, const int32_t *d_in, 
     if (!aligned16(d_in, d_keys, d_out)) return NTTB200_ERR_UNSUPPORTED;
     DeviceGuard guard(ks->device);
     return launch_keyswitch(ks, d_in, is, d_keys, galois, count, d_out, batch, (flags & NTTB200_KS_COEFF_IN) != 0,
-                            (flags & NTTB200_KS_COEFF_OUT) != 0, (cudaStream_t) stream);
+                            (flags & NTTB200_KS_COEFF_OUT) != 0, false, (cudaStream_t) stream);
+}
+
+/* ------------------------------------------------- matrix-vector products */
+int nttb200_rns_lintrans_keys(uint32_t logn, const uint32_t *offsets, uint32_t count, uint32_t n1,
+                              uint32_t *galois_out, uint32_t *nkeys) {
+    if (!nkeys) return NTTB200_ERR_INVALID_ARG;
+    LintransSchedule s;
+    int rc;
+    try {
+        rc = lintrans_schedule(logn, offsets, count, n1, &s);
+    } catch (...) {
+        return NTTB200_ERR_ALLOC;
+    }
+    if (rc != NTTB200_OK) return rc;
+    const uint64_t two_n = (uint64_t) 2 << logn, half = two_n / 4;
+    auto rot = [&](uint64_t r) {   // 5^r mod 2N, r < N/2
+        uint64_t x = 1, b = 5;
+        for (; r; r >>= 1, b = b * b % two_n) {
+            if (r & 1) x = x * b % two_n;
+        }
+        return (uint32_t) x;
+    };
+    uint32_t k = 0;
+    for (uint32_t j : s.babies) {
+        if (galois_out) galois_out[k] = rot(j);
+        k++;
+    }
+    for (uint32_t i : s.giants) {
+        if (i == 0) continue;
+        if (galois_out) galois_out[k] = rot((uint64_t) n1 * i % half);
+        k++;
+    }
+    *nkeys = k;
+    return NTTB200_OK;
+}
+
+int nttb200_rns_lintrans_apply(nttb200_rns_keyswitch *ks, const int32_t *d_ct, const int32_t *d_diags,
+                               const uint32_t *offsets, uint32_t count, uint32_t n1, const int32_t *d_keys,
+                               uint32_t nkeys, int32_t *d_out, size_t batch, void *stream) {
+    if (!ks) return NTTB200_ERR_INVALID_ARG;
+    LintransSchedule s;
+    int rc;
+    try {
+        rc = lintrans_schedule(ks->logn, offsets, count, n1, &s);
+    } catch (...) {
+        return NTTB200_ERR_ALLOC;
+    }
+    if (rc != NTTB200_OK) return rc;
+    const uint32_t nb = (uint32_t) s.babies.size(), nw = (uint32_t) s.giants.size();
+    const uint32_t ng = nw - (s.giants[0] == 0 ? 1 : 0);
+    if (nkeys != nb + ng) return NTTB200_ERR_INVALID_ARG;
+    if (batch && (!d_ct || !d_diags || !d_out || (nkeys && !d_keys))) return NTTB200_ERR_INVALID_ARG;
+    if (batch == 0) return NTTB200_OK;
+    const uint64_t n = (uint64_t) 1 << ks->logn, qw = ks->q_limbs * n, ctw = 2 * qw, rw = ks->limbs * n;
+    // sizes: byte counts within 62 bits (the buffers, U, W, V and one key-switch pass of up to 64
+    // elements); the transforms count polynomials in 32 bits and tiles in 31
+    const uint64_t lim = (uint64_t) 1 << 60;
+    const uint64_t per = ctw * (2 + nb + nw + ng) + rw * (ks->dnum + 2) * kAutoMaxElems;
+    if (batch > lim / per) return NTTB200_ERR_UNSUPPORTED;
+    const uint64_t polys = std::max<uint64_t>(std::max<uint64_t>(2 * nb, ks->dnum),
+                                              std::max<uint64_t>(2, ks->dnum) * std::min<uint32_t>(ng, kAutoMaxElems)) *
+                           batch;
+    if ((polys * ks->limbs << (ks->logn - 12)) > 0x7fffffffull || polys > 0xffffffffull) {
+        return NTTB200_ERR_UNSUPPORTED;
+    }
+    const ByteRange out = byte_range(d_out, batch * ctw);
+    if (out.overlaps(byte_range(d_ct, batch * ctw)) || out.overlaps(byte_range(d_diags, (uint64_t) count * qw)) ||
+        (nkeys && out.overlaps(byte_range(d_keys, (uint64_t) nkeys * ks->dnum * 2 * rw)))) {
+        return NTTB200_ERR_INVALID_ARG;
+    }
+    if (!aligned16(d_ct, d_diags, d_out) || !aligned16(d_keys, d_keys, d_keys)) return NTTB200_ERR_UNSUPPORTED;
+    DeviceGuard guard(ks->device);
+    try {
+        return launch_lintrans(ks, d_ct, d_diags, s, n1, d_keys, d_out, batch, (cudaStream_t) stream);
+    } catch (...) {
+        return NTTB200_ERR_ALLOC;
+    }
 }
 
 /* ---------------------------------------------------------- introspection */

@@ -16,6 +16,9 @@
 //     q + 16 (q-1)^2 < 2^64 for q <= 2^30; one store each for U_b and U_a.  The element index is
 //     the fastest-moving part of the item index, so the digit rows under way stay L2-resident
 //     while the count elements gather from them.
+//     Paired (P): D is [dnum][count][batch][L+K][N] and element c reads only its own polynomials
+//     c * batch + b, so one pass switches count different inputs, each under its own element
+//     (the giant steps of nttb200_rns_lintrans_apply).  A group of G stays inside one element.
 // Every pointer is 16-byte aligned (checked by the host), every index 64-bit.
 #include <algorithm>
 #include <vector>
@@ -31,14 +34,14 @@ constexpr int kK_Vecs = kK_BlockVecs / kK_Threads;          // uint4 per thread
 constexpr int kK_GroupOwn = 2;                              // G for batch > 1 (ptxas: no spills)
 
 // items = groups * rows * 2^(logn - 12) * count
-template <int G>
+template <int G, bool P = false>
 __global__ void __launch_bounds__(kK_Threads)
 rns_ks_dot_kernel(const uint4 *d, const uint4 *key, uint4 *u, uint64_t batch, uint32_t rows, uint32_t logn,
                   uint32_t dnum, uint32_t count, uint64_t items, const __grid_constant__ RnsKsConsts k) {
     __shared__ uint4 s4[G][kK_BlockVecs];
     const uint32_t log_b = logn - 12, bmask = (1u << log_b) - 1, nmask = (1u << logn) - 1;
     const uint64_t row_vecs = (uint64_t) 1 << (logn - 2);
-    const uint64_t poly_vecs = row_vecs * rows, digit_vecs = poly_vecs * batch;
+    const uint64_t poly_vecs = row_vecs * rows, digit_vecs = poly_vecs * batch * (P ? count : 1);
     for (uint64_t it = blockIdx.x; it < items; it += gridDim.x) {
         const uint32_t c = (uint32_t) (it % count);
         const uint64_t rest = it / count;
@@ -54,7 +57,7 @@ rns_ks_dot_kernel(const uint4 *d, const uint4 *key, uint4 *u, uint64_t batch, ui
         const uint64_t sblk = l * row_vecs + ((uint64_t) (ident ? t : src_t) << 10) + threadIdx.x;
         uint64_t pb[G];   // polynomial offsets; the last one of a ragged group stands in for the missing ones
 #pragma unroll
-        for (int p = 0; p < G; p++) pb[p] = (b0 + (p < gn ? p : gn - 1)) * poly_vecs;
+        for (int p = 0; p < G; p++) pb[p] = ((P ? (uint64_t) c * batch : 0) + b0 + (p < gn ? p : gn - 1)) * poly_vecs;
         uint32_t idx[kK_Vecs][4];   // source word of every output word, inside the staged block
 #pragma unroll
         for (int j = 0; j < kK_Vecs; j++) {
@@ -165,14 +168,14 @@ rns_ks_dot_kernel(const uint4 *d, const uint4 *key, uint4 *u, uint64_t batch, ui
     }
 }
 
-template <int G>
+template <int G, bool P>
 static int ks_dot_launch(const nttb200_rns_keyswitch *ks, const int32_t *digits, const int32_t *keys, int32_t *u,
                          size_t batch, uint32_t count, const RnsKsConsts &k, cudaStream_t st) {
     int per = 0;
-    NTTB200_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per, rns_ks_dot_kernel<G>, kK_Threads, 0));
+    NTTB200_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per, rns_ks_dot_kernel<G, P>, kK_Threads, 0));
     const uint64_t items = ((((uint64_t) batch + G - 1) / G * ks->limbs) << (ks->logn - 12)) * count;
     const uint64_t cap = (uint64_t) ks->sm_count * (per > 0 ? per : 1);
-    rns_ks_dot_kernel<G><<<(unsigned) (items < cap ? items : cap), kK_Threads, 0, st>>>(
+    rns_ks_dot_kernel<G, P><<<(unsigned) (items < cap ? items : cap), kK_Threads, 0, st>>>(
         reinterpret_cast<const uint4 *>(digits), reinterpret_cast<const uint4 *>(keys), reinterpret_cast<uint4 *>(u),
         batch, ks->limbs, ks->logn, ks->dnum, count, items, k);
     g_launches.fetch_add(1, std::memory_order_relaxed);
@@ -181,7 +184,7 @@ static int ks_dot_launch(const nttb200_rns_keyswitch *ks, const int32_t *digits,
 }
 
 static int ks_dot(const nttb200_rns_keyswitch *ks, const int32_t *digits, const int32_t *keys, int32_t *u,
-                  size_t batch, const uint32_t *galois, uint32_t count, cudaStream_t st) {
+                  size_t batch, const uint32_t *galois, uint32_t count, bool paired, cudaStream_t st) {
     RnsKsConsts k{};
     const uint32_t nmask = (1u << ks->logn) - 1;
     for (uint32_t c = 0; c < count; c++) {
@@ -192,8 +195,12 @@ static int ks_dot(const nttb200_rns_keyswitch *ks, const int32_t *digits, const 
         k.q[l] = ks->qp_fwd->pos[l].x;
         k.mu[l] = (uint64_t) ((((unsigned __int128) 1) << 64) / k.q[l]);
     }
-    return batch == 1 ? ks_dot_launch<1>(ks, digits, keys, u, batch, count, k, st)
-                      : ks_dot_launch<kK_GroupOwn>(ks, digits, keys, u, batch, count, k, st);
+    if (paired) {
+        return batch == 1 ? ks_dot_launch<1, true>(ks, digits, keys, u, batch, count, k, st)
+                          : ks_dot_launch<kK_GroupOwn, true>(ks, digits, keys, u, batch, count, k, st);
+    }
+    return batch == 1 ? ks_dot_launch<1, false>(ks, digits, keys, u, batch, count, k, st)
+                      : ks_dot_launch<kK_GroupOwn, false>(ks, digits, keys, u, batch, count, k, st);
 }
 
 // ---------------------------------------------------------------------------- host side
@@ -256,39 +263,40 @@ static int copy_rows(int32_t *dst, uint64_t dp, const int32_t *src, uint64_t sp,
 
 int launch_keyswitch(const nttb200_rns_keyswitch *ks, const int32_t *in, uint64_t in_stride, const int32_t *keys,
                      const uint32_t *galois, uint32_t count, int32_t *out, size_t batch, bool coeff_in,
-                     bool coeff_out, cudaStream_t st) {
+                     bool coeff_out, bool paired, cudaStream_t st) {
     const uint64_t n = (uint64_t) 1 << ks->logn, qw = ks->q_limbs * n, rw = ks->limbs * n;
     const uint64_t prods = (uint64_t) 2 * count * batch;   // (u0, u1) polynomials on Q P
+    const size_t polys = paired ? (size_t) count * batch : batch;   // input polynomials
     int32_t *dig = nullptr;
-    int rc = scratch_alloc_async((void **) &dig, sizeof(int32_t) * ((uint64_t) ks->dnum * batch + prods) * rw, st);
+    int rc = scratch_alloc_async((void **) &dig, sizeof(int32_t) * ((uint64_t) ks->dnum * polys + prods) * rw, st);
     if (rc != NTTB200_OK) return rc;
-    int32_t *prod = dig + (uint64_t) ks->dnum * batch * rw;
+    int32_t *prod = dig + (uint64_t) ks->dnum * polys * rw;
     // x in coefficients: the input itself, or its inverse transform in the (still unused) product buffer
     const int32_t *x = in;
     uint64_t xs = in_stride;
     if (!coeff_in) {
         const int32_t *src = in;
         if (in_stride != qw) {   // the transform reads dense rows
-            rc = copy_rows(prod, qw, in, in_stride, qw, batch, st);
+            rc = copy_rows(prod, qw, in, in_stride, qw, polys, st);
             src = prod;
         }
-        if (rc == NTTB200_OK) rc = rns_launch(ks->q_inv, 3, src, nullptr, prod, batch, st);
+        if (rc == NTTB200_OK) rc = rns_launch(ks->q_inv, 3, src, nullptr, prod, polys, st);
         x = prod;
         xs = qw;
     }
     // ModUp straight into the digit rows, then every digit to the evaluation domain on Q P
     for (uint32_t i = 0; i < ks->dnum && rc == NTTB200_OK; i++) {
         const uint32_t lo = i * ks->alpha, hi = std::min(lo + ks->alpha, ks->q_limbs);
-        int32_t *di = dig + (uint64_t) i * batch * rw;
+        int32_t *di = dig + (uint64_t) i * polys * rw;
         const int32_t *xi = x + lo * n;
-        if (i) rc = launch_rns_conv(&ks->up_lo[i - 1], xi, nullptr, xs, di, rw, batch, ConvMode::Fast, false, 0, st);
+        if (i) rc = launch_rns_conv(&ks->up_lo[i - 1], xi, nullptr, xs, di, rw, polys, ConvMode::Fast, false, 0, st);
         if (rc == NTTB200_OK) {
-            rc = launch_rns_conv(&ks->up_hi[i], xi, nullptr, xs, di + hi * n, rw, batch, ConvMode::Fast, false, 0, st);
+            rc = launch_rns_conv(&ks->up_hi[i], xi, nullptr, xs, di + hi * n, rw, polys, ConvMode::Fast, false, 0, st);
         }
-        if (rc == NTTB200_OK) rc = copy_rows(di + lo * n, rw, xi, xs, (hi - lo) * n, batch, st);
+        if (rc == NTTB200_OK) rc = copy_rows(di + lo * n, rw, xi, xs, (hi - lo) * n, polys, st);
     }
-    if (rc == NTTB200_OK) rc = rns_launch(ks->qp_fwd, 1, dig, nullptr, dig, (size_t) ks->dnum * batch, st);
-    if (rc == NTTB200_OK) rc = ks_dot(ks, dig, keys, prod, batch, galois, count, st);
+    if (rc == NTTB200_OK) rc = rns_launch(ks->qp_fwd, 1, dig, nullptr, dig, (size_t) ks->dnum * polys, st);
+    if (rc == NTTB200_OK) rc = ks_dot(ks, dig, keys, prod, batch, galois, count, paired, st);
     if (rc == NTTB200_OK) rc = rns_launch(ks->qp_inv, 3, prod, nullptr, prod, prods, st);
     if (rc == NTTB200_OK) {
         rc = launch_rns_conv(&ks->down, prod + qw, prod, rw, out, qw, prods, ConvMode::Down, true, 0, st);

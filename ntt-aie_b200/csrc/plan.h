@@ -367,8 +367,25 @@ namespace nttb200 {
 // current; the moduli checked); keyswitch_release frees them
 int keyswitch_prepare(nttb200_rns_keyswitch *ks, const nttb200_rns_plan *qp_fwd, const nttb200_rns_plan *qp_inv);
 void keyswitch_release(nttb200_rns_keyswitch *ks);
-// the caller has checked the arguments, the overlap, the 16-byte alignment and the sizes
+// the caller has checked the arguments, the overlap, the 16-byte alignment and the sizes; paired:
+// the input is count * batch polynomials (rows at in + (c * batch + b) * in_stride) and element c
+// switches only its own batch of them
 int launch_keyswitch(const nttb200_rns_keyswitch *ks, const int32_t *in, uint64_t in_stride, const int32_t *keys,
                      const uint32_t *galois, uint32_t count, int32_t *out, size_t batch, bool coeff_in,
-                     bool coeff_out, cudaStream_t st);
+                     bool coeff_out, bool paired, cudaStream_t st);
+
+// Plaintext matrix-vector products (kernels_rns_lintrans.cu): the baby-step giant-step schedule
+// of an offset set, babies j = k mod n1 >= 1 and giants i = k / n1 in ascending order.
+struct LintransSchedule {
+    std::vector<uint32_t> babies;                 // the j >= 1 that occur
+    std::vector<uint32_t> giants;                 // every i that occurs, 0 included
+    std::vector<uint32_t> offsets;                // a copy of the call's offsets
+    std::vector<std::vector<uint32_t>> terms;     // [giant] the indices into the offsets of its terms
+};
+// INVALID_ARG for a bad logn, n1, count, a null offsets, an offset >= N/2 or a duplicated one
+int lintrans_schedule(uint32_t logn, const uint32_t *offsets, uint32_t count, uint32_t n1, LintransSchedule *s);
+// the caller has checked everything, the schedule and the key count included
+int launch_lintrans(const nttb200_rns_keyswitch *ks, const int32_t *ct, const int32_t *diags,
+                    const LintransSchedule &s, uint32_t n1, const int32_t *keys, int32_t *out, size_t batch,
+                    cudaStream_t st);
 }  // namespace nttb200
